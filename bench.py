@@ -11,7 +11,7 @@ into N row bands (one per GPU), the swarm to 64*N agents, and every rank ingests
 1e7-beam share of the stream, routes the records to the band owners (NCCL all-to-all) and
 integrates what it receives.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `value` = beam-cell updates/s with the packets resident in
 HBM; `e2e` = the same metric through OccupancyGrid.update_packets() with HOST buffers (pinned
@@ -20,6 +20,10 @@ H2D copy of the batch and D2H read of the step's counters inside the timed regio
 measured HBM peak, `scatter_roofline` = updates/s vs a same-run microkernel doing nothing but
 random atomicMax(u32) on a same-size plane (SURVEY §8d); `cpu_baseline` = the reference's
 algorithm (oracle port) timed on this box's host cores on a bounded sample.
+
+`--dump-outputs DIR` (single GPU) also writes what the last timed step computed as .npy files under
+DIR (see dump_outputs()).  The inputs are seeded, so two builds run with the same arguments can
+be compared output for output.
 """
 from __future__ import annotations
 
@@ -203,6 +207,32 @@ def workload_config(n, grid_per_gpu=GRID_PER_GPU, agents_per_gpu=AGENTS_PER_GPU)
                   'L2-resident by nature of the workload'}
 
 
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_rows(height):
+    """Fixed, seeded sample of grid rows for --dump-outputs: half of them, ascending.  The whole
+    4096^2 grid in float32 (67 MB) would exceed DUMP_LIMIT_BYTES."""
+    return np.sort(np.random.default_rng(0).choice(height, height // 2, replace=False))
+
+
+def dump_outputs(out_dir, grid_sample, rows, counters):
+    """Writes what the timed path handed its caller after the last timed step:
+      grid.npy       float32 [len(rows), W]: those rows of the int8 occupancy grid (-1 / 0 / 100)
+      grid_rows.npy  float64 [len(rows)]: the row indices of grid.npy (dump_rows())
+      counters.npy   float64 [len(COUNTER_NAMES)]: the device counters of the last timed step (what
+                     counters(reset=True) returns after it), in the order of _native.COUNTER_NAMES"""
+    from occgrid_b200 import _native
+    arrays = {'grid': np.asarray(grid_sample, np.float32), 'grid_rows': np.asarray(rows, np.float64),
+              'counters': np.array([counters[k] for k in _native.COUNTER_NAMES], np.float64)}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f'--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit')
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f'{name}.npy'), a)
+
+
 # ----------------------------------------------------------------------------------------------
 #  GPU arm
 # ----------------------------------------------------------------------------------------------
@@ -271,7 +301,13 @@ def main():
                     help='N>1: which agents a rank receives (uniform = all agents, the worst case; affine = the agents of its band)')
     ap.add_argument('--exchange', default='p2p', choices=['p2p', 'nccl'],
                     help='N>1: routed records via peer-memory stores from the routing kernel (p2p) or NCCL all-to-all')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='single GPU: write the grid and counters of the last timed step as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours')
     if args.impl == 'reference':
         return run_reference(args)
 
@@ -285,6 +321,8 @@ def main():
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
     if not torch.cuda.is_available():
         raise SystemExit('bench.py needs a CUDA device (no CPU fallback)')
+    if args.dump_outputs and world > 1:
+        raise SystemExit('--dump-outputs: single-GPU runs only')
     torch.cuda.set_device(local_rank)
     dev = torch.device('cuda', local_rank)
     if world > 1:
@@ -361,12 +399,15 @@ def main():
         time.sleep(0.25)
     if world > 1:
         dist.barrier()          # nobody enters the timed region before rank 0's sampler is up
+    counters_before_last = torch.empty_like(grid._counters) if args.dump_outputs else None
     torch.cuda.synchronize()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t_wall0 = time.time()
     ev0.record()
     t_host0 = time.perf_counter()
     for i in range(K):
+        if counters_before_last is not None and i == K - 1:
+            counters_before_last.copy_(grid._counters)     # on the stream: no host synchronisation
         step(W + i)
     host_ms_per_step = (time.perf_counter() - t_host0) * 1e3 / max(K, 1)      # enqueue cost: must stay well below ms_per_step
     if n > 1:
@@ -380,6 +421,11 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
         dist.barrier()
+    if args.dump_outputs:
+        # taken before the profiling loop below integrates more batches into the same grid
+        rows = dump_rows(grid.grid_tensor.shape[0])
+        grid_sample = grid.grid_tensor[torch.from_numpy(rows).to(dev)].cpu().numpy()
+        last_counters = dict(zip(_native.COUNTER_NAMES, (grid._counters - counters_before_last).cpu().tolist()))
     counters = grid.counters(reset=True)
     upd_key = 'updates' if n == 1 else 'owned_updates'
     updates = counters[upd_key]
@@ -631,6 +677,8 @@ def main():
     result['gpu_launches'] = int(round(launches_per_step * K))
     if rank == 0:
         print(json.dumps(result))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, grid_sample, rows, last_counters)     # after every timed leg: file I/O disturbs none
     if world > 1:
         dist.destroy_process_group()
 
