@@ -12,11 +12,12 @@
 // home tile grown by R on every side.  Binning therefore needs only the robot cell — no
 // trigonometry, one record per packet, no duplicates:
 //
-//   k_home_count    thread/packet: decode (:828-843), pose correction (:851-857), robot cell
-//                   (:142) -> 48-byte pose record (packet order) + packets per home tile
-//   k_tile_plan     one CTA over the active tiles (listed by the count pass): exclusive scan of
+//   k_home_bin      thread/packet: decode (:828-843), pose correction (:851-857), robot cell
+//                   (:142) -> 48-byte pose record (packet order) + packets per home tile, and each
+//                   CTA's packet indices grouped by tile with its rank inside every tile's bin
+//   k_tile_plan     one CTA over the active tiles (listed by the bin pass): exclusive scan of
 //                   their counts -> bin offsets, (tile, chunk) work items of <= kChunkPk packets
-//   k_home_scatter  thread/packet: write the packet's index into its tile's bin
+//   k_place_runs    thread/packet: copy the grouped indices to their tile's bin
 //   k_home_raycast  persistent CTAs pull work items: zero the (64+2R)^2 smem window, expand
 //                   each record into its 4 beams (fp64 endpoints, :887-902) and walk the exact
 //                   reference Bresenham (:158-179) with atomicMax in shared memory; then flush
@@ -150,15 +151,33 @@ __device__ __forceinline__ void reserve_tile_ranges(const unsigned int* s_keys, 
         if (key[j] != kEmpty) s_vals[j * kTT + threadIdx.x] = off[j] + base[j];
 }
 
+// Packet path: the bin pass does the whole binning but the final placement.  Binning CTA b owns
+// the segment [b * kPkPerCta, (b + 1) * kPkPerCta) of the batch and of the arrays below:
+//   local_bins  its accepted packets grouped by home tile: (run << 16) | packet index in the segment
+//   runs        one per distinct tile of the segment, in local_bins order: (tile, tile_rank - local
+//               begin), where tile_rank is the CTA's position inside the tile's bin (the return
+//               value of its one atomic on tile_count) and local begin the run's first position
+//   seg_count   number of local_bins entries
+// Once k_tile_plan has the bin offsets, k_place_runs moves entry j of run r to
+// bins[tile_offset[tile] + tile_rank + (j - local begin)].  The decoded 48-byte pose record of
+// every binned packet is stored in packet order for the raycast: decoding the 42-byte wire record
+// again in the raycast instead was measured slower (DESIGN §3).
+constexpr size_t kBinSmem = (size_t)kTT * kMaxStrideT + 2 * kHash * sizeof(unsigned int) + kPkPerCta * sizeof(unsigned short);
+constexpr unsigned int kNoSlot = 0xffffu;
+
 __global__ void __launch_bounds__(kTT)
-k_home_count(Geom g, TileGeom tg, const uint8_t* __restrict__ pkts, long long n, int stride,
-             const int32_t* __restrict__ agent_idx, const double* __restrict__ drift,
-             const double* __restrict__ agent_off, int n_agents,
-             unsigned int* __restrict__ tile_count, int* __restrict__ tile_ids, PoseRec* __restrict__ recs,
-             unsigned int* __restrict__ active, TilePlanHeader* __restrict__ hdr, uint64_t* counters) {
-    __shared__ __align__(16) uint8_t s_rec[kTT * kMaxStrideT];
-    __shared__ unsigned int s_keys[kHash];
-    __shared__ unsigned int s_vals[kHash];
+k_home_bin(Geom g, TileGeom tg, const uint8_t* __restrict__ pkts, long long n, int stride,
+           const int32_t* __restrict__ agent_idx, const double* __restrict__ drift,
+           const double* __restrict__ agent_off, int n_agents,
+           unsigned int* __restrict__ tile_count, PoseRec* __restrict__ recs, unsigned int* __restrict__ local_bins, uint2* __restrict__ runs,
+           unsigned int* __restrict__ seg_count, unsigned int* __restrict__ active, TilePlanHeader* __restrict__ hdr,
+           uint64_t* counters) {
+    extern __shared__ __align__(16) uint8_t s_bin[];                                  // kBinSmem
+    uint8_t* const s_rec = s_bin;                                                     // staged records, later the local bin list
+    unsigned int* const s_keys = reinterpret_cast<unsigned int*>(s_bin + kTT * kMaxStrideT);
+    unsigned int* const s_vals = s_keys + kHash;
+    unsigned short* const s_slot = reinterpret_cast<unsigned short*>(s_vals + kHash);   // hash slot of every packet, or kNoSlot
+    __shared__ unsigned int s_wsum[kTT / 32];
     for (int i = threadIdx.x; i < kHash; i += kTT) { s_keys[i] = kEmpty; s_vals[i] = 0u; }
     unsigned long long c[OCCGRID_C_HITS + 1] = {};
     const long long cta_first = (long long)blockIdx.x * kPkPerCta;
@@ -203,7 +222,7 @@ k_home_count(Geom g, TileGeom tg, const uint8_t* __restrict__ pkts, long long n,
             double rx, ry, ryaw;
             float dist[4];
             c[OCCGRID_C_PACKETS] += 1;
-            int tile = -1;
+            unsigned int slot = kNoSlot;
             const int st = decode_packet(s_rec + threadIdx.x * stride, k, agent_idx, drift, agent_off, n_agents, &rx, &ry, &ryaw, dist);
             if (st == PKT_DROPPED) c[OCCGRID_C_DROPPED] += 1;
             else if (st == PKT_BAD_POSE) c[OCCGRID_C_BAD_POSE] += 1;
@@ -215,9 +234,10 @@ k_home_count(Geom g, TileGeom tg, const uint8_t* __restrict__ pkts, long long n,
                     const double d = (double)dist[s];
                     c[OCCGRID_C_HITS] += (OCC_MIN_DIST_M < d && d <= OCC_MAX_DIST_M) ? 1 : 0;     // :888
                 }
-                tile = home_tile(g, tg, rx, ry);
+                const int tile = home_tile(g, tg, rx, ry);
                 if (tile >= 0) {
-                    atomicAdd(&s_vals[hash_insert(s_keys, (unsigned int)tile)], 1u);
+                    slot = (unsigned int)hash_insert(s_keys, (unsigned int)tile);
+                    atomicAdd(&s_vals[slot], 1u);
                     PoseRec r;
                     r.rx = rx; r.ry = ry; r.yaw = (float)ryaw;      // ryaw came from an fp32 field: exact
                     r.d[0] = dist[0]; r.d[1] = dist[1]; r.d[2] = dist[2]; r.d[3] = dist[3];
@@ -226,13 +246,92 @@ k_home_count(Geom g, TileGeom tg, const uint8_t* __restrict__ pkts, long long n,
                     recs[k] = r;                                    // packet order: coalesced 48-byte stores
                 }
             }
-            tile_ids[k] = tile;
+            s_slot[sub * kTT + threadIdx.x] = (unsigned short)slot;
         }
     }
     __syncthreads();
-    flush_tile_counts(s_keys, s_vals, tile_count, active, hdr);
-    // the staging buffer is free now: reuse it for the counter reduction (48 KB static limit)
+    // One global atomic per distinct tile, as in flush_tile_counts; its return value is this CTA's
+    // rank inside the tile's bin.
+    unsigned int key[kHashPerThread], rank[kHashPerThread];
+#pragma unroll
+    for (int j = 0; j < kHashPerThread; ++j) {
+        const int i = j * kTT + threadIdx.x;
+        key[j] = s_keys[i];
+        rank[j] = 0u;
+        if (key[j] != kEmpty) rank[j] = atomicAdd(&tile_count[key[j]], s_vals[i]);
+    }
+    // Exclusive scan of (count | 1 << 16) over the occupied slots in (thread, j) order: the low half
+    // is the slot's first local position, the high half its run index (both < kPkPerCta).  An empty
+    // slot has count 0.
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    unsigned int mine = 0u;
+#pragma unroll
+    for (int j = 0; j < kHashPerThread; ++j) mine += key[j] != kEmpty ? s_vals[j * kTT + threadIdx.x] + 0x10000u : 0u;
+    unsigned int inc = mine;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const unsigned int u = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += u; }
+    if (lane == 31) s_wsum[warp] = inc;
+    __syncthreads();
+    unsigned int pos = inc - mine, n_local = 0u;
+#pragma unroll
+    for (int w = 0; w < kTT / 32; ++w) {
+        pos += w < warp ? s_wsum[w] : 0u;
+        n_local += s_wsum[w];
+    }
+    n_local &= 0xffffu;
+    if (threadIdx.x == 0) seg_count[blockIdx.x] = n_local;
+    const size_t seg0 = (size_t)blockIdx.x * kPkPerCta;
+    // run descriptors; each slot (owned by this thread alone) now holds its run index and its next
+    // free local position
+#pragma unroll
+    for (int j = 0; j < kHashPerThread; ++j) {
+        if (key[j] == kEmpty) continue;
+        const int i = j * kTT + threadIdx.x;
+        const unsigned int run = pos >> 16, begin = pos & 0xffffu;
+        runs[seg0 + run] = make_uint2(key[j], rank[j] - begin);
+        pos += s_vals[i] + 0x10000u;
+        s_keys[i] = run;
+        s_vals[i] = begin;
+        if (rank[j] == 0u) active[atomicAdd(&hdr->active_count, 1u)] = key[j];     // first toucher lists the tile
+    }
+    __syncthreads();
+    // the packet indices grouped by tile, assembled in the (now free) staging buffer, then stored
+    // coalesced
+    unsigned int* const s_local = reinterpret_cast<unsigned int*>(s_rec);
+    const int n_seg = (int)min((long long)kPkPerCta, n - (long long)seg0);
+    for (int j = threadIdx.x; j < n_seg; j += kTT) {
+        const unsigned int slot = s_slot[j];
+        if (slot != kNoSlot) s_local[atomicAdd(&s_vals[slot], 1u)] = (s_keys[slot] << 16) | (unsigned int)j;
+    }
+    __syncthreads();
+    for (unsigned int j = threadIdx.x; j < n_local; j += kTT) local_bins[seg0 + j] = s_local[j];
+    __syncthreads();
     block_add_counters(c, reinterpret_cast<unsigned long long*>(s_rec), counters);
+}
+
+// Thread per local_bins entry of one binning CTA's segment (see k_home_bin): no hash and no atomics,
+// and the stores of a run are contiguous.
+__global__ void __launch_bounds__(kTT)
+k_place_runs(const unsigned int* __restrict__ local_bins, const uint2* __restrict__ runs, const unsigned int* __restrict__ seg_count,
+             const unsigned int* __restrict__ tile_offset, const TilePlanHeader* __restrict__ hdr, unsigned int* __restrict__ bins) {
+    if (hdr->overflow) return;
+    const size_t seg0 = (size_t)blockIdx.x * kPkPerCta;
+    const int n_local = (int)seg_count[blockIdx.x];
+    // three dependent gathers per entry: each phase has all of the thread's loads in flight
+    unsigned int e[kSub], off[kSub];
+    uint2 d[kSub];
+#pragma unroll
+    for (int sub = 0; sub < kSub; ++sub) {
+        const int j = sub * kTT + threadIdx.x;
+        e[sub] = j < n_local ? local_bins[seg0 + j] : kEmpty;
+    }
+#pragma unroll
+    for (int sub = 0; sub < kSub; ++sub) d[sub] = e[sub] != kEmpty ? runs[seg0 + (e[sub] >> 16)] : make_uint2(0u, 0u);
+#pragma unroll
+    for (int sub = 0; sub < kSub; ++sub) off[sub] = e[sub] != kEmpty ? tile_offset[d[sub].x] : 0u;
+#pragma unroll
+    for (int sub = 0; sub < kSub; ++sub)
+        if (e[sub] != kEmpty) bins[off[sub] + d[sub].y + (unsigned int)(sub * kTT + threadIdx.x)] = (unsigned int)(seg0 + (e[sub] & 0xffffu));
 }
 
 // Segment / validity of one 2048-address chunk of a (possibly segmented) record buffer.
@@ -1113,14 +1212,16 @@ static int g_raycast_cta_cap = 0;
 void set_raycast_cta_cap(int cap) { g_raycast_cta_cap = cap < 0 ? 0 : cap; }
 
 struct TiledLayout {
-    size_t off_stamps, off_count, off_offset, off_cursor, off_active, off_hdr, off_items, off_ids, off_bins, off_recs, total;
+    size_t off_stamps, off_count, off_offset, off_cursor, off_active, off_hdr, off_items, off_ids, off_bins, off_local, off_runs,
+        off_segs, off_recs, total;
     unsigned long long max_records;
     unsigned int max_items;
 };
 
-// max_records = record ADDRESSES the bins / tile-id arrays must cover; with_recs: room for the
-// decoded records of a packet batch (input that arrives decoded brings its own buffer).
-static TiledLayout tiled_layout(const occgrid_geom* geom, int64_t max_records, bool with_recs) {
+// max_records = record ADDRESSES the bins must cover.  packets: the arrays of k_home_bin for a
+// packet batch (local bins, runs, segment counts, decoded records); else the tile ids that
+// k_home_count_poses hands to the scatter (input that arrives decoded brings its own records).
+static TiledLayout tiled_layout(const occgrid_geom* geom, int64_t max_records, bool packets) {
     TiledLayout L;
     const TileGeom tg = tile_geom(geom);
     L.max_records = (unsigned long long)max_records;
@@ -1135,9 +1236,12 @@ static TiledLayout tiled_layout(const occgrid_geom* geom, int64_t max_records, b
     L.off_active = o; o += align_up((size_t)(tg.n_tiles + 1) * 4, 256);
     L.off_hdr = o;    o += 256;
     L.off_items = o;  o += align_up((size_t)L.max_items * sizeof(uint4), 256);
-    L.off_ids = o;    o += align_up((size_t)L.max_records * sizeof(int), 256);
+    L.off_ids = o;    o += packets ? 0 : align_up((size_t)L.max_records * sizeof(int), 256);
     L.off_bins = o;   o += align_up((size_t)L.max_records * sizeof(unsigned int), 256);
-    L.off_recs = o;   o += with_recs ? align_up((size_t)L.max_records * sizeof(PoseRec), 256) : 0;
+    L.off_local = o;  o += packets ? align_up((size_t)L.max_records * sizeof(unsigned int), 256) : 0;
+    L.off_runs = o;   o += packets ? align_up((size_t)L.max_records * sizeof(uint2), 256) : 0;     // worst case: a run per packet
+    L.off_segs = o;   o += packets ? align_up((size_t)(L.max_records + kPkPerCta - 1) / kPkPerCta * sizeof(unsigned int), 256) : 0;
+    L.off_recs = o;   o += packets ? align_up((size_t)L.max_records * sizeof(PoseRec), 256) : 0;
     L.total = o;
     return L;
 }
@@ -1156,10 +1260,11 @@ size_t tiled_band_workspace_bytes(const occgrid_geom* geom, int n_segs, int64_t 
 }
 
 struct TiledPtrs {
-    unsigned int *stamps, *tile_count, *tile_offset, *tile_cursor, *active, *bins;
+    unsigned int *stamps, *tile_count, *tile_offset, *tile_cursor, *active, *bins, *local_bins, *seg_count;
     TilePlanHeader* hdr;
     uint4* items;
     int* tile_ids;
+    uint2* runs;
     PoseRec* recs;
 };
 
@@ -1175,6 +1280,9 @@ static TiledPtrs tiled_ptrs(const TiledLayout& L, void* d_ws) {
     p.items = reinterpret_cast<uint4*>(ws + L.off_items);
     p.bins = reinterpret_cast<unsigned int*>(ws + L.off_bins);
     p.tile_ids = reinterpret_cast<int*>(ws + L.off_ids);
+    p.local_bins = reinterpret_cast<unsigned int*>(ws + L.off_local);
+    p.runs = reinterpret_cast<uint2*>(ws + L.off_runs);
+    p.seg_count = reinterpret_cast<unsigned int*>(ws + L.off_segs);
     p.recs = reinterpret_cast<PoseRec*>(ws + L.off_recs);
     return p;
 }
@@ -1247,12 +1355,14 @@ int integrate_tiled(const occgrid_geom* geom, const uint8_t* d_packets, const Po
     const long long n_chunks = (n + kSegChunk - 1) / kSegChunk;
     {
         ProfileScope ps(K_TILE_COUNT, st);
-        if (d_poses)
+        if (d_poses) {
             k_home_count_poses<<<grid_chunks(n_chunks), kTT, 0, st>>>(g, tg, d_poses, nullptr, seg, n_chunks, 0, P.tile_count, P.tile_ids, P.active,
                                                                       P.hdr, d_counters);
-        else
-            k_home_count<<<blocks, kTT, 0, st>>>(g, tg, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents,
-                                                P.tile_count, P.tile_ids, P.recs, P.active, P.hdr, d_counters);
+        } else {
+            OCC_CUDA_TRY(cudaFuncSetAttribute(k_home_bin, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBinSmem));
+            k_home_bin<<<blocks, kTT, kBinSmem, st>>>(g, tg, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents,
+                                                      P.tile_count, P.recs, P.local_bins, P.runs, P.seg_count, P.active, P.hdr, d_counters);
+        }
     }
     {
         ProfileScope ps(K_TILE_SCAN, st);
@@ -1261,7 +1371,8 @@ int integrate_tiled(const occgrid_geom* geom, const uint8_t* d_packets, const Po
     }
     {
         ProfileScope ps(K_TILE_SCATTER, st);
-        k_home_scatter<<<blocks, kTT, 0, st>>>(n, P.tile_ids, P.tile_offset, P.tile_cursor, P.hdr, P.bins);
+        if (d_poses) k_home_scatter<<<blocks, kTT, 0, st>>>(n, P.tile_ids, P.tile_offset, P.tile_cursor, P.hdr, P.bins);
+        else         k_place_runs<<<blocks, kTT, 0, st>>>(P.local_bins, P.runs, P.seg_count, P.tile_offset, P.hdr, P.bins);
     }
     RouteJob none = {};
     if (d_counts) launch_raycast<true, false>(g, tg, P, recs, ordinals_in_records, reinterpret_cast<unsigned int*>(d_counts), d_counters, 1, none, st);
