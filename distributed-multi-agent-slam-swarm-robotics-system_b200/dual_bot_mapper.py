@@ -427,7 +427,7 @@ class OccupancyGrid:
 
     def log_odds(self, l_occ=0.85, l_free=-0.4, l_min=-2.0, l_max=3.5, to_host=True):
         """float32 [h, w]: clamp(hits * l_occ + misses * l_free, l_min, l_max), evaluated from the
-        integer planes (order-independent; within 1e-5 of a float64 NumPy evaluation)."""
+        integer planes (order-independent; equal to the float64 NumPy evaluation rounded to float32)."""
         with torch.cuda.device(self.device):
             h, w = self.grid_tensor.shape
             out = torch.empty((h, w), dtype=torch.float32, device=self.device)

@@ -15,15 +15,15 @@ _lib = None
 def lib():
     global _lib
     if _lib is None:
-        path = _build.LIB
-        if not os.path.exists(path) or os.environ.get('ORACLE_REBUILD'):
-            path = _build.build()
-        _lib = C.CDLL(path)
-        _lib.oracle_integrate_packets.restype = C.c_int
-        _lib.oracle_integrate_packets.argtypes = [
-            C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
-            C.c_double, C.c_double, C.c_double, C.c_int64, C.c_int64,
-            C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]
+        # build() compares modification times and returns at once when the library is current, so
+        # a library left over from older sources is rebuilt rather than loaded without new symbols
+        _lib = C.CDLL(_build.build(force=bool(os.environ.get('ORACLE_REBUILD'))))
+        for fn in (_lib.oracle_integrate_packets, _lib.oracle_accumulate_packets):
+            fn.restype = C.c_int
+            fn.argtypes = [
+                C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                C.c_double, C.c_double, C.c_double, C.c_int64, C.c_int64,
+                C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]
         _lib.oracle_update_rays.restype = C.c_int
         _lib.oracle_update_rays.argtypes = [
             C.c_void_p, C.c_void_p, C.c_int64, C.c_double, C.c_double, C.c_double,
@@ -37,11 +37,8 @@ def _ptr(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
 
-def integrate_packets(packets, grid, ox, oy, res, rec_len=42, stride=None, separation=0.0,
-                      drift=None, agent_offsets=None, agent_idx=None, window=None,
-                      size_x=None, size_y=None):
-    """packets: uint8 array [n, stride] (or flat).  grid: int8 [H, W], updated in place.
-    window=(x0, y0) places `grid` as a tile of a (size_y, size_x) global grid."""
+def _packets(fn, packets, plane, ox, oy, res, rec_len, stride, separation, drift, agent_offsets, agent_idx,
+             window, size_x, size_y):
     pk = np.ascontiguousarray(packets, dtype=np.uint8)
     if stride is None:
         stride = pk.shape[1] if pk.ndim == 2 else rec_len
@@ -55,18 +52,38 @@ def integrate_packets(packets, grid, ox, oy, res, rec_len=42, stride=None, separ
         assert drift.shape == (n, 2)
     if agent_idx is not None:
         agent_idx = np.ascontiguousarray(agent_idx, np.int32)
-    assert grid.dtype == np.int8 and grid.flags.c_contiguous
-    h, w = grid.shape
+    assert plane.flags.c_contiguous
+    h, w = plane.shape[:2]
     wx0, wy0 = window if window is not None else (0, 0)
     sx = size_x if size_x is not None else w
     sy = size_y if size_y is not None else h
     counters = np.zeros(8, np.uint64)
-    rc = lib().oracle_integrate_packets(_ptr(pk), n, stride, rec_len, _ptr(agent_idx), _ptr(drift),
-                                        _ptr(agent_offsets), n_agents, ox, oy, res, sx, sy,
-                                        wx0, wy0, w, h, _ptr(grid), _ptr(counters))
+    rc = fn(_ptr(pk), n, stride, rec_len, _ptr(agent_idx), _ptr(drift), _ptr(agent_offsets), n_agents,
+            ox, oy, res, sx, sy, wx0, wy0, w, h, _ptr(plane), _ptr(counters))
     if rc != 0:
-        raise ValueError(f'oracle_integrate_packets rc={rc}')
+        raise ValueError(f'{fn.__name__} rc={rc}')
     return dict(zip(COUNTER_NAMES, (int(c) for c in counters)))
+
+
+def integrate_packets(packets, grid, ox, oy, res, rec_len=42, stride=None, separation=0.0,
+                      drift=None, agent_offsets=None, agent_idx=None, window=None,
+                      size_x=None, size_y=None):
+    """packets: uint8 array [n, stride] (or flat).  grid: int8 [H, W], updated in place.
+    window=(x0, y0) places `grid` as a tile of a (size_y, size_x) global grid."""
+    assert grid.dtype == np.int8 and grid.ndim == 2
+    return _packets(lib().oracle_integrate_packets, packets, grid, ox, oy, res, rec_len, stride, separation,
+                    drift, agent_offsets, agent_idx, window, size_x, size_y)
+
+
+def accumulate_packets(packets, counts, ox, oy, res, rec_len=42, stride=None, separation=0.0,
+                       drift=None, agent_offsets=None, agent_idx=None, window=None,
+                       size_x=None, size_y=None):
+    """Count mode of integrate_packets: counts int32 [H, W, 2] = {miss, hit} per cell, added to in
+    place.  Same records, keywords and counters; the cells integrate_packets would store FREE
+    count one miss each, the OCCUPIED end cell of a valid hit one hit."""
+    assert counts.dtype == np.int32 and counts.ndim == 3 and counts.shape[2] == 2
+    return _packets(lib().oracle_accumulate_packets, packets, counts, ox, oy, res, rec_len, stride, separation,
+                    drift, agent_offsets, agent_idx, window, size_x, size_y)
 
 
 def update_rays(rays, hit, grid, ox, oy, res):

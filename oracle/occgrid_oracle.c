@@ -35,12 +35,22 @@ static int64_t trunc_i64(double q) {
     return (int64_t)q;
 }
 
+/* Where update_ray's stores go: the int8 grid (last writer wins, :148-156) or, when `counts` is
+ * set, int32 {miss, hit} pairs per cell (count mode: every FREE store counts one miss, every
+ * OCCUPIED store one hit).  Exactly one of the two pointers is set. */
+typedef struct { int8_t* grid; int32_t* counts; } Plane;
+
+static void store_cell(Plane out, int64_t i, int occupied) {
+    if (out.counts) out.counts[2 * i + (occupied ? 1 : 0)]++;
+    else out.grid[i] = occupied ? CELL_OCCUPIED : CELL_FREE;
+}
+
 /* OccupancyGrid.update_ray + _bresenham + in_bounds — dual_bot_mapper.py:133-179.
- * The window (win_x0, win_y0, win_w, win_h) is the part of the global grid that `grid`
+ * The window (win_x0, win_y0, win_w, win_h) is the part of the global grid that `out`
  * holds (row stride win_w): the full grid for the reference case, a spatial tile for the
  * multi-GPU tests.  Cells are generated on the unclipped global line and masked one by
  * one, exactly like the per-cell in_bounds test at :149,:155. */
-static int64_t update_ray_cells(int8_t* grid, int64_t size_x, int64_t size_y,
+static int64_t update_ray_cells(Plane out, int64_t size_x, int64_t size_y,
                                 int64_t win_x0, int64_t win_y0, int64_t win_w, int64_t win_h,
                                 int64_t x0, int64_t y0, int64_t x1, int64_t y1, int hit_valid) {
     int64_t dx = x1 > x0 ? x1 - x0 : x0 - x1;
@@ -55,7 +65,7 @@ static int64_t update_ray_cells(int8_t* grid, int64_t size_x, int64_t size_y,
         if ((!last || hit_valid) && x0 >= 0 && x0 < size_x && y0 >= 0 && y0 < size_y) {
             int64_t lx = x0 - win_x0, ly = y0 - win_y0;
             if (lx >= 0 && lx < win_w && ly >= 0 && ly < win_h)
-                grid[ly * win_w + lx] = last ? CELL_OCCUPIED : CELL_FREE;
+                store_cell(out, ly * win_w + lx, last);
         }
         if (last) break;
         int64_t e2 = 2 * err;
@@ -75,13 +85,13 @@ static int64_t update_ray_cells(int8_t* grid, int64_t size_x, int64_t size_y,
  *             the pose (:851-852; reference mode = {(0,0),(0,0),(separation,0)})
  *  drift      n x 2 doubles or NULL (:855-857)
  */
-int oracle_integrate_packets(const uint8_t* pkts, int64_t n, int stride, int rec_len,
-                             const int32_t* agent_idx, const double* drift,
-                             const double* agent_off, int n_agents,
-                             double ox, double oy, double res,
-                             int64_t size_x, int64_t size_y,
-                             int64_t win_x0, int64_t win_y0, int64_t win_w, int64_t win_h,
-                             int8_t* grid, uint64_t* counters) {
+static int packets_into(const uint8_t* pkts, int64_t n, int stride, int rec_len,
+                        const int32_t* agent_idx, const double* drift,
+                        const double* agent_off, int n_agents,
+                        double ox, double oy, double res,
+                        int64_t size_x, int64_t size_y,
+                        int64_t win_x0, int64_t win_y0, int64_t win_w, int64_t win_h,
+                        Plane out, uint64_t* counters) {
     /* :61-66 — math.pi/2, math.pi, -math.pi/2 as doubles (hex literals: exact) */
     static const double ANG[4] = { 0.0, 0x1.921fb54442d18p+0, 0x1.921fb54442d18p+1,
                                    -0x1.921fb54442d18p+0 };
@@ -113,11 +123,37 @@ int oracle_integrate_packets(const uint8_t* pkts, int64_t n, int stride, int rec
             int64_t y1 = trunc_i64((wy - oy) / res);
             counters[C_BEAMS]++;
             counters[C_HITS] += (uint64_t)hit_valid;
-            counters[C_UPDATES] += (uint64_t)update_ray_cells(grid, size_x, size_y, win_x0, win_y0,
+            counters[C_UPDATES] += (uint64_t)update_ray_cells(out, size_x, size_y, win_x0, win_y0,
                                                               win_w, win_h, x0, y0, x1, y1, hit_valid);
         }
     }
     return 0;
+}
+
+/* The loop body into the int8 grid `grid` [win_h][win_w]. */
+int oracle_integrate_packets(const uint8_t* pkts, int64_t n, int stride, int rec_len,
+                             const int32_t* agent_idx, const double* drift,
+                             const double* agent_off, int n_agents,
+                             double ox, double oy, double res,
+                             int64_t size_x, int64_t size_y,
+                             int64_t win_x0, int64_t win_y0, int64_t win_w, int64_t win_h,
+                             int8_t* grid, uint64_t* counters) {
+    const Plane out = { grid, NULL };
+    return packets_into(pkts, n, stride, rec_len, agent_idx, drift, agent_off, n_agents, ox, oy, res,
+                        size_x, size_y, win_x0, win_y0, win_w, win_h, out, counters);
+}
+
+/* Count mode: the same loop body, adding into `counts` [win_h][win_w][2] = {miss, hit}. */
+int oracle_accumulate_packets(const uint8_t* pkts, int64_t n, int stride, int rec_len,
+                              const int32_t* agent_idx, const double* drift,
+                              const double* agent_off, int n_agents,
+                              double ox, double oy, double res,
+                              int64_t size_x, int64_t size_y,
+                              int64_t win_x0, int64_t win_y0, int64_t win_w, int64_t win_h,
+                              int32_t* counts, uint64_t* counters) {
+    const Plane out = { NULL, counts };
+    return packets_into(pkts, n, stride, rec_len, agent_idx, drift, agent_off, n_agents, ox, oy, res,
+                        size_x, size_y, win_x0, win_y0, win_w, win_h, out, counters);
 }
 
 /* OccupancyGrid.update_ray on explicit world-space rays (the per-ray API, :136-156). */
@@ -131,7 +167,8 @@ int oracle_update_rays(const double* rays /* n x 4: x0 y0 x1 y1 */, const uint8_
         int64_t y1 = trunc_i64((rays[4 * k + 3] - oy) / res);
         counters[C_BEAMS]++;
         counters[C_HITS] += hit[k] != 0;
-        counters[C_UPDATES] += (uint64_t)update_ray_cells(grid, size_x, size_y, 0, 0, size_x, size_y,
+        const Plane out = { grid, NULL };
+        counters[C_UPDATES] += (uint64_t)update_ray_cells(out, size_x, size_y, 0, 0, size_x, size_y,
                                                           x0, y0, x1, y1, hit[k] != 0);
     }
     return 0;
