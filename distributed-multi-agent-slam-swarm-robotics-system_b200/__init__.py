@@ -3,7 +3,7 @@
 Import as ``occgrid_b200`` (the repository root carries an alias package, because this
 directory's mandated name is not a Python identifier):
 
-    from occgrid_b200.dual_bot_mapper import OccupancyGrid
+    from occgrid_b200.dual_bot_mapper import OccupancyGrid, AgentGrids
     from occgrid_b200.map_merger import MapMerger
 """
 from . import _native  # noqa: F401

@@ -101,6 +101,10 @@ def lib():
     L.occgrid_workspace_reset.argtypes = [vp, sz, vp]
     L.occgrid_integrate_packets.restype = i32
     L.occgrid_integrate_packets.argtypes = [gp, vp, i64, i32, i32, vp, vp, vp, i32, vp, vp, sz, vp, i32, vp]
+    L.occgrid_agent_maps_workspace_bytes.restype = sz
+    L.occgrid_agent_maps_workspace_bytes.argtypes = [gp, i32, i64, i32]
+    L.occgrid_integrate_packets_agent_maps.restype = i32
+    L.occgrid_integrate_packets_agent_maps.argtypes = [gp, vp, i64, i32, i32, vp, vp, vp, i32, vp, vp, sz, vp, i32, vp]
     L.occgrid_update_rays.restype = i32
     L.occgrid_update_rays.argtypes = [gp, vp, vp, i64, vp, vp, sz, vp, i32, vp]
     L.occgrid_scatter_probe.restype = i32

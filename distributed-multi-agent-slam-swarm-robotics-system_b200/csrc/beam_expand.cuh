@@ -126,13 +126,15 @@ OCC_HD void expand_beam(const Geom& g, double rx, double ry, double ryaw, int x0
 enum { PKT_OK = 0, PKT_DROPPED = 1, PKT_BAD_POSE = 2 };
 
 // Decode + filter + pose correction for one record (:828-857).  `p` points at the record
-// (any alignment).  Returns PKT_*; on PKT_OK fills the corrected pose and the 4 ranges.
+// (any alignment).  Returns PKT_*; on PKT_OK fills the corrected pose and the 4 ranges, and
+// `agent_out` (when given) with the accepted agent id 1..n_agents.
 OCC_HD int decode_packet(const uint8_t* p, long long k, const int32_t* agent_idx, const double* drift,
                          const double* agent_off, int n_agents,
-                         double* rx, double* ry, double* ryaw, float dist[4]) {
+                         double* rx, double* ry, double* ryaw, float dist[4], int* agent_out = nullptr) {
     if (!(p[0] == 'Q' && p[1] == 'S' && p[2] == 'R' && p[3] == 'L')) return PKT_DROPPED;   // :840
     long long agent = agent_idx ? (long long)agent_idx[k] : (long long)p[4];
     if (agent < 1 || agent > n_agents) return PKT_DROPPED;                                  // :842
+    if (agent_out) *agent_out = (int)agent;
     double x = (double)load_f32_unaligned(p + 5);
     double y = (double)load_f32_unaligned(p + 9);
     double yaw = (double)load_f32_unaligned(p + 13);

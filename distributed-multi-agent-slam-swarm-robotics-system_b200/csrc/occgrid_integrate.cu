@@ -153,12 +153,14 @@ __device__ __forceinline__ bool start_in_window(const Geom& g, const Beam& b) {
     return b.valid && b.x0 >= g.win_x0 && b.x0 < g.win_x0 + g.win_w && b.y0 >= g.win_y0 && b.y0 < g.win_y0 + g.win_h;
 }
 
-template <bool kCounts>
+// kMaps: one stamp plane per agent (occgrid_integrate_packets_agent_maps); a record of agent a
+// draws into plane a - 1, `map_cells` words after plane a - 2.
+template <bool kCounts, bool kMaps = false>
 __global__ void __launch_bounds__(kThreads)
 k_integrate_global(Geom g, const uint8_t* __restrict__ pkts, long long n, int stride,
                    const int32_t* __restrict__ agent_idx, const double* __restrict__ drift,
                    const double* __restrict__ agent_off, int n_agents,
-                   unsigned int* __restrict__ stamps, uint64_t* counters) {
+                   unsigned int* __restrict__ stamps, uint64_t* counters, size_t map_cells = 0) {
     __shared__ __align__(16) uint8_t s_rec[kThreads * kMaxStride];
     __shared__ unsigned long long s_acc[(OCCGRID_C_OWNED_UPDATES + 1) * 32];
     const long long first = (long long)blockIdx.x * kThreads;
@@ -171,13 +173,15 @@ k_integrate_global(Geom g, const uint8_t* __restrict__ pkts, long long n, int st
         const long long k = first + threadIdx.x;
         double rx, ry, ryaw;
         float dist[4];
+        int agent = 1;
         c[OCCGRID_C_PACKETS] = 1;
         const int st = decode_packet(s_rec + threadIdx.x * stride, k, agent_idx, drift, agent_off, n_agents,
-                                     &rx, &ry, &ryaw, dist);
+                                     &rx, &ry, &ryaw, dist, kMaps ? &agent : nullptr);
         if (st == PKT_DROPPED) c[OCCGRID_C_DROPPED] = 1;
         else if (st == PKT_BAD_POSE) c[OCCGRID_C_BAD_POSE] = 1;
         else {
             c[OCCGRID_C_ACCEPTED] = 1;
+            if (kMaps) stamps += (size_t)(agent - 1) * map_cells;
             Beam b[4];
             expand_packet(g, rx, ry, ryaw, dist, LibSinCos(), b);
             bool later_writes_first = false;
@@ -300,8 +304,9 @@ int device_sm_count() {
 }
 static int sm_count() { return device_sm_count(); }
 
-static int launch_resolve(const occgrid_geom* geom, unsigned int* stamps, int8_t* grid, cudaStream_t st) {
-    const size_t n_cells = (size_t)geom->win_w * geom->win_h;
+// n_maps > 1: the planes and grids of an agent-map stack are contiguous, so one pass streams them all.
+static int launch_resolve(const occgrid_geom* geom, unsigned int* stamps, int8_t* grid, cudaStream_t st, int n_maps = 1) {
+    const size_t n_cells = (size_t)geom->win_w * geom->win_h * (size_t)n_maps;
     const int vec_ok = ((reinterpret_cast<uintptr_t>(stamps) & 15) == 0 && (reinterpret_cast<uintptr_t>(grid) & 3) == 0) ? 1 : 0;
     size_t want = (n_cells / 4 + kThreads - 1) / kThreads;
     if (want < 1) want = 1;
@@ -335,6 +340,32 @@ int integrate_packets_global(const occgrid_geom* geom, const uint8_t* d_packets,
     }
     OCC_CUDA_TRY(cudaGetLastError());
     return launch_resolve(geom, stamps, d_grid, st);
+}
+
+// Agent-map stack: n_agents stamp planes, each the size of the (whole-grid) window.
+size_t global_agent_maps_workspace_bytes(const occgrid_geom* geom, int n_agents) {
+    return align_up((size_t)geom->win_w * geom->win_h * (size_t)n_agents * sizeof(unsigned int), 256);
+}
+
+int integrate_packets_global_agent_maps(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride,
+                                        const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
+                                        int n_agents, int8_t* d_grids, void* d_ws, size_t ws_bytes, uint64_t* d_counters,
+                                        cudaStream_t st) {
+    const size_t need = global_agent_maps_workspace_bytes(geom, n_agents);
+    if (ws_bytes < need) {
+        set_last_error("workspace %zu B < %zu B needed by GLOBAL_ATOMIC for %d agent maps", ws_bytes, need, n_agents);
+        return OCCGRID_E_WORKSPACE;
+    }
+    unsigned int* stamps = reinterpret_cast<unsigned int*>(d_ws);
+    const long long blocks = (n + kThreads - 1) / kThreads;
+    {
+        ProfileScope ps(K_INTEGRATE_GLOBAL, st);
+        k_integrate_global<false, true><<<(unsigned int)blocks, kThreads, 0, st>>>(to_geom(geom), d_packets, n, stride, d_agent_idx,
+                                                                                  d_drift, d_agent_off, n_agents, stamps, d_counters,
+                                                                                  (size_t)geom->win_w * geom->win_h);
+    }
+    OCC_CUDA_TRY(cudaGetLastError());
+    return launch_resolve(geom, stamps, d_grids, st, n_agents);
 }
 
 // L = clamp(hits * l_occ + misses * l_free, l_min, l_max), derived from the integer planes so
@@ -432,6 +463,30 @@ int accumulate_packets_tiled(const occgrid_geom* geom, const uint8_t* d_packets,
 void set_raycast_cta_cap(int cap);
 int integrate_poses_tiled(const occgrid_geom* geom, const void* d_poses, int64_t n, int ordinals_in_records, int8_t* d_grid,
                           void* d_ws, size_t ws_bytes, uint64_t* d_counters, cudaStream_t st);
+size_t tiled_agent_maps_workspace_bytes(const occgrid_geom* geom, int n_agents, int64_t max_packets);
+bool tiled_agent_maps_supported(const occgrid_geom* geom, int n_agents);
+int integrate_packets_tiled_agent_maps(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride,
+                                       const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
+                                       int n_agents, int8_t* d_grids, void* d_ws, size_t ws_bytes, uint64_t* d_counters,
+                                       cudaStream_t st);
+
+// Geometry of an agent-map stack: a valid geometry whose window is the whole grid, n_agents >= 1,
+// and a stack (of 4-byte stamps: the larger of the two) whose size fits size_t.
+static int validate_agent_maps(const occgrid_geom* geom, int n_agents) {
+    int rc = validate_geom(geom);
+    if (rc != OCCGRID_OK) return rc;
+    if (geom->win_x0 != 0 || geom->win_y0 != 0 || geom->win_w != geom->size_x || geom->win_h != geom->size_y) {
+        set_last_error("agent maps: the window must be the whole grid");
+        return OCCGRID_E_ARG;
+    }
+    if (n_agents < 1) { set_last_error("agent maps: n_agents=%d, need >= 1", n_agents); return OCCGRID_E_ARG; }
+    const size_t cells = (size_t)geom->size_x * (size_t)geom->size_y;
+    if (cells > SIZE_MAX / sizeof(unsigned int) / (size_t)n_agents) {
+        set_last_error("agent maps: %d maps of %d x %d cells overflow size_t", n_agents, geom->size_x, geom->size_y);
+        return OCCGRID_E_ARG;
+    }
+    return OCCGRID_OK;
+}
 }
 
 extern "C" {
@@ -489,6 +544,58 @@ int occgrid_integrate_packets(const occgrid_geom* geom, const uint8_t* d_packets
         if (!tiled_supported(geom)) { set_last_error("TILED strategy does not support this geometry"); return OCCGRID_E_RANGE; }
         return integrate_packets_tiled(geom, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents, d_grid,
                                        d_workspace, workspace_bytes, d_counters, st);
+    }
+    set_last_error("unknown strategy %d", strategy);
+    return OCCGRID_E_ARG;
+}
+
+static int pick_agent_maps_strategy(const occgrid_geom* geom, int n_agents, int strategy) {
+    if (strategy == OCCGRID_STRATEGY_AUTO)
+        return tiled_agent_maps_supported(geom, n_agents) ? OCCGRID_STRATEGY_TILED : OCCGRID_STRATEGY_GLOBAL_ATOMIC;
+    return strategy;
+}
+
+size_t occgrid_agent_maps_workspace_bytes(const occgrid_geom* geom, int n_agents, int64_t max_packets, int strategy) {
+    if (validate_agent_maps(geom, n_agents) != OCCGRID_OK) return 0;
+    if (max_packets < 0) { set_last_error("max_packets < 0"); return 0; }
+    const int s = pick_agent_maps_strategy(geom, n_agents, strategy);
+    if (s == OCCGRID_STRATEGY_GLOBAL_ATOMIC) return global_agent_maps_workspace_bytes(geom, n_agents);
+    if (s == OCCGRID_STRATEGY_TILED) {
+        if (!tiled_agent_maps_supported(geom, n_agents)) { set_last_error("TILED strategy does not support this geometry and agent count"); return 0; }
+        return tiled_agent_maps_workspace_bytes(geom, n_agents, max_packets);
+    }
+    set_last_error("unknown strategy %d", strategy);
+    return 0;
+}
+
+int occgrid_integrate_packets_agent_maps(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride, int rec_len,
+                                         const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
+                                         int n_agents, int8_t* d_grids, void* d_workspace, size_t workspace_bytes,
+                                         uint64_t* d_counters, int strategy, void* stream) {
+    int rc = validate_agent_maps(geom, n_agents);
+    if (rc != OCCGRID_OK) return rc;
+    if (n < 0 || n > (1ll << 29) - 1) { set_last_error("n=%lld outside 0..2^29-1 records per call", (long long)n); return OCCGRID_E_ARG; }
+    if (rec_len != OCCGRID_PACKET_SIZE && rec_len != OCCGRID_PACKET_SIZE_V1) {
+        set_last_error("rec_len must be 42 or 41, got %d", rec_len);
+        return OCCGRID_E_ARG;
+    }
+    if (stride < rec_len || stride > kMaxStride) { set_last_error("stride %d outside %d..%d", stride, rec_len, kMaxStride); return OCCGRID_E_ARG; }
+    if (!d_agent_off) { set_last_error("need an agent offset table"); return OCCGRID_E_ARG; }
+    if (!d_grids || !d_workspace) { set_last_error("grids/workspace is NULL"); return OCCGRID_E_ARG; }
+    if (n == 0) return OCCGRID_OK;
+    if (!d_packets) { set_last_error("packets is NULL"); return OCCGRID_E_ARG; }
+    const int s = pick_agent_maps_strategy(geom, n_agents, strategy);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (s == OCCGRID_STRATEGY_GLOBAL_ATOMIC)
+        return integrate_packets_global_agent_maps(geom, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents, d_grids,
+                                                   d_workspace, workspace_bytes, d_counters, st);
+    if (s == OCCGRID_STRATEGY_TILED) {
+        if (!tiled_agent_maps_supported(geom, n_agents)) {
+            set_last_error("TILED strategy does not support this geometry and agent count");
+            return OCCGRID_E_RANGE;
+        }
+        return integrate_packets_tiled_agent_maps(geom, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents, d_grids,
+                                                  d_workspace, workspace_bytes, d_counters, st);
     }
     set_last_error("unknown strategy %d", strategy);
     return OCCGRID_E_ARG;

@@ -162,9 +162,13 @@ __device__ __forceinline__ void reserve_tile_ranges(const unsigned int* s_keys, 
 // bins[tile_offset[tile] + tile_rank + (j - local begin)].  The decoded 48-byte pose record of
 // every binned packet is stored in packet order for the raycast: decoding the 42-byte wire record
 // again in the raycast instead was measured slower (DESIGN §3).
+//
+// kMaps (occgrid_integrate_packets_agent_maps): the map is folded into the tile KEY, (agent - 1) *
+// n_tiles + home tile.  Everything below and the plan and placement passes work on keys unchanged.
 constexpr size_t kBinSmem = (size_t)kTT * kMaxStrideT + 2 * kHash * sizeof(unsigned int) + kPkPerCta * sizeof(unsigned short);
 constexpr unsigned int kNoSlot = 0xffffu;
 
+template <bool kMaps = false>
 __global__ void __launch_bounds__(kTT)
 k_home_bin(Geom g, TileGeom tg, const uint8_t* __restrict__ pkts, long long n, int stride,
            const int32_t* __restrict__ agent_idx, const double* __restrict__ drift,
@@ -223,7 +227,9 @@ k_home_bin(Geom g, TileGeom tg, const uint8_t* __restrict__ pkts, long long n, i
             float dist[4];
             c[OCCGRID_C_PACKETS] += 1;
             unsigned int slot = kNoSlot;
-            const int st = decode_packet(s_rec + threadIdx.x * stride, k, agent_idx, drift, agent_off, n_agents, &rx, &ry, &ryaw, dist);
+            int agent = 1;
+            const int st = decode_packet(s_rec + threadIdx.x * stride, k, agent_idx, drift, agent_off, n_agents, &rx, &ry, &ryaw, dist,
+                                         kMaps ? &agent : nullptr);
             if (st == PKT_DROPPED) c[OCCGRID_C_DROPPED] += 1;
             else if (st == PKT_BAD_POSE) c[OCCGRID_C_BAD_POSE] += 1;
             else {
@@ -234,7 +240,8 @@ k_home_bin(Geom g, TileGeom tg, const uint8_t* __restrict__ pkts, long long n, i
                     const double d = (double)dist[s];
                     c[OCCGRID_C_HITS] += (OCC_MIN_DIST_M < d && d <= OCC_MAX_DIST_M) ? 1 : 0;     // :888
                 }
-                const int tile = home_tile(g, tg, rx, ry);
+                int tile = home_tile(g, tg, rx, ry);
+                if (kMaps && tile >= 0) tile += (agent - 1) * tg.n_tiles;
                 if (tile >= 0) {
                     slot = (unsigned int)hash_insert(s_keys, (unsigned int)tile);
                     atomicAdd(&s_vals[slot], 1u);
@@ -1019,7 +1026,8 @@ __device__ __forceinline__ unsigned int route_items_before(unsigned int i, unsig
 
 // Three CTAs per SM (80 registers): measured 0.204 ms against 0.248 (two CTAs, <= 128 registers)
 // and 0.256 (four CTAs, 64 registers with spills) on BASELINE configs[1].
-template <bool kCounts, bool kRoute>
+// kMaps: item.x is a key (map * n_tiles + tile, see k_home_bin); the map selects the stamp plane.
+template <bool kCounts, bool kRoute, bool kMaps = false>
 __global__ void __launch_bounds__(kTT, 3)
 k_home_raycast(Geom g, TileGeom tg, const uint4* __restrict__ items, TilePlanHeader* __restrict__ hdr,
                const unsigned int* __restrict__ bins, const PoseRec* __restrict__ recs, int ordinals_in_records,
@@ -1069,7 +1077,10 @@ k_home_raycast(Geom g, TileGeom tg, const uint4* __restrict__ items, TilePlanHea
             __syncthreads();
         }
         const uint4 item = items[it];
-        const int ttx = item.x % tg.tiles_x, tty = item.x / tg.tiles_x;
+        const unsigned int map = kMaps ? item.x / (unsigned int)tg.n_tiles : 0u;
+        const unsigned int tile = item.x - map * (unsigned int)tg.n_tiles;
+        unsigned int* __restrict__ const plane = kMaps ? stamps + (size_t)map * ((size_t)g.win_w * g.win_h) : stamps;
+        const int ttx = tile % tg.tiles_x, tty = tile / tg.tiles_x;
         // global cell of window-local (0, 0)
         const int wx0 = g.win_x0 - tg.pad + (ttx << kTileShift) - tg.reach;
         const int wy0 = g.win_y0 - tg.pad + (tty << kTileShift) - tg.reach;
@@ -1125,14 +1136,14 @@ k_home_raycast(Geom g, TileGeom tg, const uint4* __restrict__ items, TilePlanHea
             for (int ly = warp; ly < side; ly += kTT / 32) {                   // one warp per window row
                 unsigned int* row = s_win + ly * pitch;
                 const bool row_in = ly >= ly_lo && ly < ly_hi;
-                unsigned int* out = stamps + (size_t)(wy0 + ly - g.win_y0) * g.win_w + (wx0 - g.win_x0);
+                unsigned int* out = plane + (size_t)(wy0 + ly - g.win_y0) * g.win_w + (wx0 - g.win_x0);
                 for (int lx = lane; lx < side; lx += 32) {
                     const unsigned int v = row[lx];
                     if (!v) continue;
                     if (!kRoute) row[lx] = 0u;
                     if (!(row_in && lx >= lx_lo && lx < lx_hi)) continue;
                     if (kCounts)     // {miss, hit} int32 pair of the cell: one 64-bit add (the halves cannot carry into each other)
-                        atomicAdd(reinterpret_cast<unsigned long long*>(stamps) + ((size_t)(wy0 + ly - g.win_y0) * g.win_w + (wx0 - g.win_x0) + lx),
+                        atomicAdd(reinterpret_cast<unsigned long long*>(plane) + ((size_t)(wy0 + ly - g.win_y0) * g.win_w + (wx0 - g.win_x0) + lx),
                                   ((unsigned long long)(v >> 16) << 32) | (unsigned long long)(v & 0xffffu));
                     else
                         atomicMax(out + lx, v);
@@ -1170,6 +1181,8 @@ k_home_raycast(Geom g, TileGeom tg, const uint4* __restrict__ items, TilePlanHea
 
 constexpr int kResolveSplit = 8;      // CTAs per active window (row slices) — few tiles are active, keep all SMs busy
 
+// kMaps: the active list holds keys (see k_home_bin); the map selects the stamp plane and the grid.
+template <bool kMaps = false>
 __global__ void __launch_bounds__(kTT)
 k_home_resolve(Geom g, TileGeom tg, const unsigned int* __restrict__ active, TilePlanHeader* __restrict__ hdr,
                unsigned int* __restrict__ stamps, int8_t* __restrict__ grid) {
@@ -1183,7 +1196,12 @@ k_home_resolve(Geom g, TileGeom tg, const unsigned int* __restrict__ active, Til
         __syncthreads();
         const unsigned int it = s_item;
         if (it >= n_work) break;
-        const unsigned int t = active[it / kResolveSplit];
+        const unsigned int key = active[it / kResolveSplit];
+        const unsigned int map = kMaps ? key / (unsigned int)tg.n_tiles : 0u;
+        const unsigned int t = key - map * (unsigned int)tg.n_tiles;
+        const size_t map_off = kMaps ? (size_t)map * ((size_t)g.win_w * g.win_h) : 0;
+        unsigned int* __restrict__ const plane = stamps + map_off;
+        int8_t* __restrict__ const map_grid = grid + map_off;
         const int part = (int)(it % kResolveSplit);
         const int ttx = t % tg.tiles_x, tty = t / tg.tiles_x;
         const int wx0 = -tg.pad + (ttx << kTileShift) - tg.reach;      // window-relative
@@ -1194,10 +1212,10 @@ k_home_resolve(Geom g, TileGeom tg, const unsigned int* __restrict__ active, Til
         for (int ly = ly_lo + part * (kTT / 32) + warp; ly < ly_hi; ly += kResolveSplit * (kTT / 32)) {   // one warp per row
             const size_t row = (size_t)(wy0 + ly) * g.win_w + wx0;
             for (int lx = lx_lo + lane; lx < lx_hi; lx += 32) {
-                const unsigned int s = stamps[row + lx];
+                const unsigned int s = plane[row + lx];
                 if (s) {
-                    grid[row + lx] = (s & 1u) ? OCCGRID_CELL_OCCUPIED : OCCGRID_CELL_FREE;
-                    stamps[row + lx] = 0u;
+                    map_grid[row + lx] = (s & 1u) ? OCCGRID_CELL_OCCUPIED : OCCGRID_CELL_FREE;
+                    plane[row + lx] = 0u;
                 }
             }
         }
@@ -1221,19 +1239,22 @@ struct TiledLayout {
 // max_records = record ADDRESSES the bins must cover.  packets: the arrays of k_home_bin for a
 // packet batch (local bins, runs, segment counts, decoded records); else the tile ids that
 // k_home_count_poses hands to the scatter (input that arrives decoded brings its own records).
-static TiledLayout tiled_layout(const occgrid_geom* geom, int64_t max_records, bool packets) {
+// n_maps > 1 (agent maps, packets only): one stamp plane per map and per-key tile arrays, key =
+// map * n_tiles + tile.
+static TiledLayout tiled_layout(const occgrid_geom* geom, int64_t max_records, bool packets, int n_maps = 1) {
     TiledLayout L;
     const TileGeom tg = tile_geom(geom);
+    const size_t n_keys = (size_t)n_maps * tg.n_tiles;
     L.max_records = (unsigned long long)max_records;
-    unsigned long long items = L.max_records / kChunkMin + (unsigned long long)tg.n_tiles + 1;
+    unsigned long long items = L.max_records / kChunkMin + (unsigned long long)n_keys + 1;
     if (items > L.max_records + 1) items = L.max_records + 1;
     L.max_items = (unsigned int)items;
     size_t o = 0;
-    L.off_stamps = o; o += align_up((size_t)geom->win_w * geom->win_h * 4, 256);
-    L.off_count = o;  o += align_up((size_t)(tg.n_tiles + 1) * 4, 256);
-    L.off_offset = o; o += align_up((size_t)(tg.n_tiles + 1) * 4, 256);
-    L.off_cursor = o; o += align_up((size_t)(tg.n_tiles + 1) * 4, 256);
-    L.off_active = o; o += align_up((size_t)(tg.n_tiles + 1) * 4, 256);
+    L.off_stamps = o; o += align_up((size_t)geom->win_w * geom->win_h * 4 * (size_t)n_maps, 256);
+    L.off_count = o;  o += align_up((n_keys + 1) * 4, 256);
+    L.off_offset = o; o += align_up((n_keys + 1) * 4, 256);
+    L.off_cursor = o; o += align_up((n_keys + 1) * 4, 256);
+    L.off_active = o; o += align_up((n_keys + 1) * 4, 256);
     L.off_hdr = o;    o += 256;
     L.off_items = o;  o += align_up((size_t)L.max_items * sizeof(uint4), 256);
     L.off_ids = o;    o += packets ? 0 : align_up((size_t)L.max_records * sizeof(int), 256);
@@ -1253,6 +1274,15 @@ bool tiled_supported(const occgrid_geom* geom) {
 
 size_t tiled_workspace_bytes(const occgrid_geom* geom, int64_t max_packets) {
     return tiled_layout(geom, max_packets < 1 ? 1 : max_packets, true).total;
+}
+
+// Keys (map * n_tiles + tile) stay below 2^24, as tiles do on one grid.
+bool tiled_agent_maps_supported(const occgrid_geom* geom, int n_agents) {
+    return tiled_supported(geom) && (long long)n_agents * tile_geom(geom).n_tiles <= (1ll << 24);
+}
+
+size_t tiled_agent_maps_workspace_bytes(const occgrid_geom* geom, int n_agents, int64_t max_packets) {
+    return tiled_layout(geom, max_packets < 1 ? 1 : max_packets, true, n_agents).total;
 }
 
 size_t tiled_band_workspace_bytes(const occgrid_geom* geom, int n_segs, int64_t seg_cap) {
@@ -1298,23 +1328,23 @@ static size_t raycast_smem(const TileGeom& tg, bool route) {
     return b;
 }
 
-template <bool kCounts, bool kRoute>
+template <bool kCounts, bool kRoute, bool kMaps = false>
 static int launch_raycast(const Geom& g, const TileGeom& tg, const TiledPtrs& P, const PoseRec* recs, int ordinals_in_records,
                           unsigned int* plane, uint64_t* d_counters, int have_items, const RouteJob& job, cudaStream_t st) {
     const size_t smem = raycast_smem(tg, kRoute);
     static thread_local size_t configured = 0;
     if (smem > configured) {
-        OCC_CUDA_TRY(cudaFuncSetAttribute(k_home_raycast<kCounts, kRoute>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        OCC_CUDA_TRY(cudaFuncSetAttribute(k_home_raycast<kCounts, kRoute, kMaps>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         configured = smem;
     }
     int ctas_per_sm = 1;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, k_home_raycast<kCounts, kRoute>, kTT, smem) != cudaSuccess || ctas_per_sm < 1)
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, k_home_raycast<kCounts, kRoute, kMaps>, kTT, smem) != cudaSuccess || ctas_per_sm < 1)
         ctas_per_sm = 1;
     if (g_raycast_cta_cap > 0 && ctas_per_sm > g_raycast_cta_cap) ctas_per_sm = g_raycast_cta_cap;
     ProfileScope ps(K_TILE_RAYCAST, st);
-    k_home_raycast<kCounts, kRoute><<<device_sm_count() * ctas_per_sm, kTT, smem, st>>>(g, tg, P.items, P.hdr, P.bins, recs,
-                                                                                        ordinals_in_records, plane, d_counters,
-                                                                                        have_items, job);
+    k_home_raycast<kCounts, kRoute, kMaps><<<device_sm_count() * ctas_per_sm, kTT, smem, st>>>(g, tg, P.items, P.hdr, P.bins, recs,
+                                                                                               ordinals_in_records, plane, d_counters,
+                                                                                               have_items, job);
     return OCCGRID_OK;
 }
 
@@ -1335,12 +1365,13 @@ static int grid_chunks(long long n_chunks) {
 }
 
 // `d_poses` != NULL: input is n PoseRec (already decoded and corrected), `d_packets` etc. unused.
+// `maps` (packets into the grid only): d_grid is a stack of n_agents grids, agent a's at a - 1.
 int integrate_tiled(const occgrid_geom* geom, const uint8_t* d_packets, const PoseRec* d_poses, int ordinals_in_records,
                     int64_t n, int stride,
                     const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
                     int n_agents, int8_t* d_grid, int32_t* d_counts, void* d_ws, size_t ws_bytes, uint64_t* d_counters,
-                    cudaStream_t st) {
-    const TiledLayout L = tiled_layout(geom, n, d_poses == nullptr);
+                    cudaStream_t st, bool maps = false) {
+    const TiledLayout L = tiled_layout(geom, n, d_poses == nullptr, maps ? n_agents : 1);
     if (ws_bytes < L.total) {
         set_last_error("workspace %zu B < %zu B needed by TILED for %lld records", ws_bytes, L.total, (long long)n);
         return OCCGRID_E_WORKSPACE;
@@ -1358,10 +1389,14 @@ int integrate_tiled(const occgrid_geom* geom, const uint8_t* d_packets, const Po
         if (d_poses) {
             k_home_count_poses<<<grid_chunks(n_chunks), kTT, 0, st>>>(g, tg, d_poses, nullptr, seg, n_chunks, 0, P.tile_count, P.tile_ids, P.active,
                                                                       P.hdr, d_counters);
+        } else if (maps) {
+            OCC_CUDA_TRY(cudaFuncSetAttribute(k_home_bin<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBinSmem));
+            k_home_bin<true><<<blocks, kTT, kBinSmem, st>>>(g, tg, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents,
+                                                            P.tile_count, P.recs, P.local_bins, P.runs, P.seg_count, P.active, P.hdr, d_counters);
         } else {
-            OCC_CUDA_TRY(cudaFuncSetAttribute(k_home_bin, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBinSmem));
-            k_home_bin<<<blocks, kTT, kBinSmem, st>>>(g, tg, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents,
-                                                      P.tile_count, P.recs, P.local_bins, P.runs, P.seg_count, P.active, P.hdr, d_counters);
+            OCC_CUDA_TRY(cudaFuncSetAttribute(k_home_bin<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBinSmem));
+            k_home_bin<false><<<blocks, kTT, kBinSmem, st>>>(g, tg, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents,
+                                                             P.tile_count, P.recs, P.local_bins, P.runs, P.seg_count, P.active, P.hdr, d_counters);
         }
     }
     {
@@ -1375,11 +1410,13 @@ int integrate_tiled(const occgrid_geom* geom, const uint8_t* d_packets, const Po
         else         k_place_runs<<<blocks, kTT, 0, st>>>(P.local_bins, P.runs, P.seg_count, P.tile_offset, P.hdr, P.bins);
     }
     RouteJob none = {};
-    if (d_counts) launch_raycast<true, false>(g, tg, P, recs, ordinals_in_records, reinterpret_cast<unsigned int*>(d_counts), d_counters, 1, none, st);
-    else          launch_raycast<false, false>(g, tg, P, recs, ordinals_in_records, P.stamps, d_counters, 1, none, st);
+    if (d_counts)  launch_raycast<true, false>(g, tg, P, recs, ordinals_in_records, reinterpret_cast<unsigned int*>(d_counts), d_counters, 1, none, st);
+    else if (maps) launch_raycast<false, false, true>(g, tg, P, recs, ordinals_in_records, P.stamps, d_counters, 1, none, st);
+    else           launch_raycast<false, false>(g, tg, P, recs, ordinals_in_records, P.stamps, d_counters, 1, none, st);
     if (!d_counts) {
         ProfileScope ps(K_TILE_RESOLVE, st);
-        k_home_resolve<<<device_sm_count() * 8, kTT, 0, st>>>(g, tg, P.active, P.hdr, P.stamps, d_grid);
+        if (maps) k_home_resolve<true><<<device_sm_count() * 8, kTT, 0, st>>>(g, tg, P.active, P.hdr, P.stamps, d_grid);
+        else      k_home_resolve<false><<<device_sm_count() * 8, kTT, 0, st>>>(g, tg, P.active, P.hdr, P.stamps, d_grid);
     }
     OCC_CUDA_TRY(cudaGetLastError());
     return OCCGRID_OK;
@@ -1441,7 +1478,7 @@ int tiled_raycast_route(const occgrid_geom* geom, const PoseRec* d_recs, int hav
     if (after_fused) OCC_CUDA_TRY(cudaEventRecord(after_fused, st));      // the routed batch is out: publishing may overlap the resolve
     if (have_items) {
         ProfileScope ps(K_TILE_RESOLVE, st);
-        k_home_resolve<<<device_sm_count() * 8, kTT, 0, st>>>(g, tg, P.active, P.hdr, P.stamps, d_grid);
+        k_home_resolve<false><<<device_sm_count() * 8, kTT, 0, st>>>(g, tg, P.active, P.hdr, P.stamps, d_grid);
     }
     OCC_CUDA_TRY(cudaGetLastError());
     return OCCGRID_OK;
@@ -1453,6 +1490,14 @@ int integrate_packets_tiled(const occgrid_geom* geom, const uint8_t* d_packets, 
                             cudaStream_t st) {
     return integrate_tiled(geom, d_packets, nullptr, 0, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents, d_grid, nullptr, d_ws,
                            ws_bytes, d_counters, st);
+}
+
+int integrate_packets_tiled_agent_maps(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride,
+                                       const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
+                                       int n_agents, int8_t* d_grids, void* d_ws, size_t ws_bytes, uint64_t* d_counters,
+                                       cudaStream_t st) {
+    return integrate_tiled(geom, d_packets, nullptr, 0, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents, d_grids, nullptr, d_ws,
+                           ws_bytes, d_counters, st, true);
 }
 
 int accumulate_packets_tiled(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride,

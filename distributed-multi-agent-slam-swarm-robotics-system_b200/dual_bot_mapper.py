@@ -135,12 +135,16 @@ class OccupancyGrid:
         if self._ws is not None and n_packets <= self._ws_capacity:
             return
         cap = max(n_packets, 1)
-        nbytes = self._lib.occgrid_workspace_bytes(self._geom, cap, self._strategy)
-        if nbytes == 0:
-            raise OccGridError('occgrid_workspace_bytes: ' + _native.last_error())
+        nbytes = self._workspace_nbytes(cap)
         with torch.cuda.device(self.device):
             self._ws = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
         self._ws_capacity = cap
+
+    def _workspace_nbytes(self, cap):
+        nbytes = self._lib.occgrid_workspace_bytes(self._geom, cap, self._strategy)
+        if nbytes == 0:
+            raise OccGridError('occgrid_workspace_bytes: ' + _native.last_error())
+        return nbytes
 
     def _ray_workspace(self):
         if self._ws_ray is None:
@@ -386,12 +390,16 @@ class OccupancyGrid:
                     self._counters.data_ptr(), self._strategy, self._stream())
                 _native.check(rc, 'occgrid_accumulate_packets')
                 return
-            rc = self._lib.occgrid_integrate_packets(
-                self._geom, pk.data_ptr(), n, stride, rec_len, a_ptr, d_ptr, tab.data_ptr(), tab.shape[0] - 1,
-                self.grid_tensor.data_ptr(), self._ws.data_ptr(), self._ws.numel(),
-                self._counters.data_ptr(), self._strategy, self._stream())
-            _native.check(rc, 'occgrid_integrate_packets')
+            self._launch_packets(pk, rec_len, a_ptr, d_ptr, tab)
         self._host_cache = None
+
+    def _launch_packets(self, pk, rec_len, a_ptr, d_ptr, tab):
+        n, stride = pk.shape
+        rc = self._lib.occgrid_integrate_packets(
+            self._geom, pk.data_ptr(), n, stride, rec_len, a_ptr, d_ptr, tab.data_ptr(), tab.shape[0] - 1,
+            self.grid_tensor.data_ptr(), self._ws.data_ptr(), self._ws.numel(),
+            self._counters.data_ptr(), self._strategy, self._stream())
+        _native.check(rc, 'occgrid_integrate_packets')
 
     # ---- extension: hit/miss counts and log-odds (no reference counterpart) -------------------
     _accumulating = False
@@ -591,6 +599,108 @@ class OccupancyGrid:
     def clear(self):
         self.grid_tensor.fill_(CELL_UNKNOWN)
         self._host_cache = None
+
+
+def _single_map_only(name):
+    def method(self, *args, **kwargs):
+        raise OccGridError(f'AgentGrids.{name}: single-map operation; run it on an OccupancyGrid built from grid(agent_id)')
+    method.__name__ = name
+    return method
+
+
+class AgentGrids(OccupancyGrid):
+    """EXTENSION: one occupancy grid per agent, integrated from ONE packet stream on the device.
+
+    The reference's multi-agent architecture maps every robot in its own frame (``/agent_{id}/map``)
+    and lets ``map_merger.py`` register and fuse the maps.  ``update_packets`` takes the same input
+    as ``OccupancyGrid.update_packets`` (and streams large host batches the same way); grid a - 1 of
+    the stack ends equal to ``OccupancyGrid.update_packets`` run over only the records of agent a.
+
+      grids_tensor  int8 [n_agents, size, size] on the device, agent a at index a - 1
+      origins       float64 [n_agents, 2], every row (origin_x, origin_y); ``res`` the resolution
+
+    The stack is what ``MapMerger.merge(maps.grids_tensor, maps.origins, maps.res, transforms)``
+    takes, without a copy.  All maps share one geometry.  ``agent_offsets`` must have n_agents + 1
+    rows; the default is zero except row 2 = (separation, 0) (:851-852), so with separation = 0
+    every agent maps in its own odometry frame.  Single-map operations (rays, pose records, counts,
+    frontiers, rendering) raise ``OccGridError``.
+    """
+
+    def __init__(self, n_agents=2, size=GRID_SIZE, resolution=GRID_RESOLUTION,
+                 origin_x=GRID_ORIGIN_X, origin_y=GRID_ORIGIN_Y, *,
+                 device='cuda', strategy='auto', max_batch=1 << 16):
+        self.n_agents = int(n_agents)
+        if self.n_agents < 1:
+            raise ValueError('n_agents must be >= 1')
+        super().__init__(size, resolution, origin_x, origin_y, device=device, strategy=strategy, lazy_workspace=True)
+        del self.grid_tensor
+        with torch.cuda.device(self.device):
+            self.grids_tensor = torch.full((self.n_agents, self.size, self.size), CELL_UNKNOWN, dtype=torch.int8,
+                                           device=self.device)
+        self.origins = np.tile(np.array([[self.ox, self.oy]], np.float64), (self.n_agents, 1))
+        self._ensure_workspace(int(max_batch))
+
+    def _workspace_nbytes(self, cap):
+        nbytes = self._lib.occgrid_agent_maps_workspace_bytes(self._geom, self.n_agents, cap, self._strategy)
+        if nbytes == 0:
+            raise OccGridError('occgrid_agent_maps_workspace_bytes: ' + _native.last_error())
+        return nbytes
+
+    def _agent_table(self, separation, agent_offsets):
+        if agent_offsets is None:
+            agent_offsets = np.zeros((self.n_agents + 1, 2), np.float64)
+            if self.n_agents >= 2:
+                agent_offsets[2, 0] = float(separation)
+        tab = super()._agent_table(separation, agent_offsets)
+        if tab.shape[0] != self.n_agents + 1:
+            raise ValueError(f'agent_offsets has {tab.shape[0]} rows, need n_agents + 1 = {self.n_agents + 1}')
+        return tab
+
+    def _launch_packets(self, pk, rec_len, a_ptr, d_ptr, tab):
+        n, stride = pk.shape
+        rc = self._lib.occgrid_integrate_packets_agent_maps(
+            self._geom, pk.data_ptr(), n, stride, rec_len, a_ptr, d_ptr, tab.data_ptr(), self.n_agents,
+            self.grids_tensor.data_ptr(), self._ws.data_ptr(), self._ws.numel(),
+            self._counters.data_ptr(), self._strategy, self._stream())
+        _native.check(rc, 'occgrid_integrate_packets_agent_maps')
+
+    def grid(self, agent_id):
+        """Host copy of agent ``agent_id``'s map, ``np.int8 [gy, gx]``, cached until the next update."""
+        a = int(agent_id)
+        if not 1 <= a <= self.n_agents:
+            raise ValueError(f'agent_id {a} outside 1..{self.n_agents}')
+        if self._host_cache is None:
+            self._host_cache = {}
+        if a not in self._host_cache:
+            self._host_cache[a] = self.grids_tensor[a - 1].cpu().numpy()
+        return self._host_cache[a]
+
+    @property
+    def grids(self):
+        """Host copy of the stack, ``np.int8 [n_agents, size, size]``, cached until the next update."""
+        if self._host_cache is None:
+            self._host_cache = {}
+        if 'all' not in self._host_cache:
+            self._host_cache['all'] = self.grids_tensor.cpu().numpy()
+        return self._host_cache['all']
+
+    def clear(self):
+        self.grids_tensor.fill_(CELL_UNKNOWN)
+        self._host_cache = None
+
+    update_ray = _single_map_only('update_ray')
+    update_rays = _single_map_only('update_rays')
+    update_poses = _single_map_only('update_poses')
+    accumulate_packets = _single_map_only('accumulate_packets')
+    log_odds = _single_map_only('log_odds')
+    reset_counts = _single_map_only('reset_counts')
+    counts_tensor = property(_single_map_only('counts_tensor'))
+    hit_counts = property(_single_map_only('hit_counts'))
+    miss_counts = property(_single_map_only('miss_counts'))
+    get_frontiers = _single_map_only('get_frontiers')
+    cluster_frontiers = _single_map_only('cluster_frontiers')
+    frontier_centroids = _single_map_only('frontier_centroids')
+    render_overlay = _single_map_only('render_overlay')
 
 
 class PoseNode:

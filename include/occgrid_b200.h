@@ -131,6 +131,29 @@ int occgrid_integrate_packets(const occgrid_geom* geom,
                               uint64_t* d_counters, int strategy, void* stream);
 
 /*
+ * Per-agent maps (EXTENSION): the same batch integrated into a stack of n_agents grids, one per
+ * agent, the input map_merger.py's MapMerger fuses (/agent_{id}/map).  Grid a - 1 of the stack
+ * ends equal to occgrid_integrate_packets run over only the records whose agent (wire byte, or
+ * d_agent_idx[k]) is a, in buffer order: decode, filter, offsets, drift, beams, per-cell clipping
+ * and last-writer-wins are unchanged, and records of different agents never interact.  The
+ * counters equal those of occgrid_integrate_packets on the same batch, geometry and strategy.
+ *
+ *   geom     shared by every map; the window must be the whole grid
+ *   d_grids  int8 [n_agents][size_y][size_x], agent a at index a - 1, updated in place
+ *   other arguments as occgrid_integrate_packets
+ * AUTO picks TILED when the geometry supports it and n_agents * (tiles of the grid) <= 2^24, else
+ * GLOBAL_ATOMIC.  The workspace holds n_agents stamp planes (0 bytes on error).
+ */
+size_t occgrid_agent_maps_workspace_bytes(const occgrid_geom* geom, int n_agents, int64_t max_packets, int strategy);
+int occgrid_integrate_packets_agent_maps(const occgrid_geom* geom,
+                                         const uint8_t* d_packets, int64_t n, int stride, int rec_len,
+                                         const int32_t* d_agent_idx, const double* d_drift,
+                                         const double* d_agent_off, int n_agents,
+                                         int8_t* d_grids,
+                                         void* d_workspace, size_t workspace_bytes,
+                                         uint64_t* d_counters, int strategy, void* stream);
+
+/*
  * Batched OccupancyGrid.update_ray (dual_bot_mapper.py:136-156) on explicit world-space rays:
  * d_rays = double[n][4] (robot_x, robot_y, hit_x, hit_y), d_hit = uint8[n] (hit_valid),
  * applied in index order with last-writer-wins.
