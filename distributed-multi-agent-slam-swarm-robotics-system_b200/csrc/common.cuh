@@ -63,6 +63,61 @@ struct ProfileScope {
 
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// ---- packet batches -------------------------------------------------------------------------------
+constexpr int kMaxRecStride = 64;            // bytes per packet record slot staged in shared memory
+
+// One batch of wire records as the packet entry points receive it (include/occgrid_b200.h).
+struct PacketBatch {
+    const uint8_t* pkts; int64_t n; int stride;
+    const int32_t* agent_idx; const double* drift; const double* agent_off; int n_agents;
+};
+
+// What a packet batch is integrated into: one int8 grid, a stack of n_agents grids (agent a's at
+// a - 1), or the int32 {miss, hit} count planes of one grid.
+enum class Output { kGrid, kAgentMaps, kCounts };
+
+// The record checks every packet entry point shares: n in 0..2^29-1, rec_len 42 or 41, stride in
+// rec_len..kMaxRecStride, n_agents >= 1 with an agent offset table, packets non-NULL when n > 0.
+// `who` prefixes the error message.
+int check_packet_batch(const PacketBatch& b, int rec_len, const char* who);
+
+// Cooperative copy of a CTA's records into shared memory with 16-byte loads.
+__device__ __forceinline__ void stage_records(const uint8_t* __restrict__ src, size_t bytes, uint8_t* smem) {
+    const size_t nvec = ((reinterpret_cast<uintptr_t>(src) & 15) == 0) ? bytes / 16 : 0;
+    const uint4* s4 = reinterpret_cast<const uint4*>(src);
+    uint4* d4 = reinterpret_cast<uint4*>(smem);
+    for (size_t i = threadIdx.x; i < nvec; i += blockDim.x) d4[i] = __ldg(s4 + i);
+    for (size_t i = nvec * 16 + threadIdx.x; i < bytes; i += blockDim.x) smem[i] = __ldg(src + i);
+}
+
+// ---- tiles of the TILED strategy (occgrid_tiled.cu) ------------------------------------------------
+constexpr int kTile = 64;            // home-tile side in cells
+constexpr int kTileShift = 6;
+
+// Cells a beam can reach from the robot cell: R = ceil(MAX_DIST_M / res) + 2 (:57, :900).
+__host__ __device__ __forceinline__ int reach_cells(double res) { return (int)ceil(OCC_MAX_DIST_M / res) + 2; }
+
+struct TileGeom {
+    int reach;            // R
+    int pad;              // cells added around the window so that every home tile is >= 0
+    int tiles_x, tiles_y, n_tiles;
+    int win_side;         // smem window side = kTile + 2R
+    int pitch;            // smem row pitch (odd)
+};
+
+inline TileGeom tile_geom(double res, int win_w, int win_h) {
+    TileGeom t;
+    t.reach = reach_cells(res);
+    t.pad = ((t.reach + kTile - 1) / kTile) * kTile;
+    t.tiles_x = (win_w + 2 * t.pad + kTile - 1) >> kTileShift;
+    t.tiles_y = (win_h + 2 * t.pad + kTile - 1) >> kTileShift;
+    t.n_tiles = t.tiles_x * t.tiles_y;
+    t.win_side = kTile + 2 * t.reach;
+    t.pitch = t.win_side | 1;
+    return t;
+}
+inline TileGeom tile_geom(const occgrid_geom* g) { return tile_geom(g->res, g->win_w, g->win_h); }
+
 // ---- band exchange (multi-GPU row bands, SURVEY §8e) -----------------------------------------
 // Records of a batch arrive in per-source segments of a receive slot: segment s occupies record
 // addresses [s * seg_cap, s * seg_cap + count[s]).  count[] lives on the device (written by the
@@ -99,6 +154,14 @@ struct RouteJob {
     unsigned int n_route_items;              // work items of kRouteItemPk * kRouteSubs packets
 };
 
+// TILED entry points.  n_maps: grids the call writes (n_agents for Output::kAgentMaps, else 1);
+// their tile keys, map * n_tiles + tile, must stay below 2^24.
+bool tiled_supported(const occgrid_geom* geom, int n_maps);
+size_t tiled_workspace_bytes(const occgrid_geom* geom, int n_maps, int64_t max_packets);
+// Integrates a packet batch, or (d_poses != NULL) batch.n decoded pose records, into d_out.
+int integrate_tiled(const occgrid_geom* geom, const PacketBatch& batch, const PoseRec* d_poses, int ordinals_in_records, Output kind,
+                    void* d_out, void* d_ws, size_t ws_bytes, uint64_t* d_counters, cudaStream_t st);
+void set_raycast_cta_cap(int cap);
 size_t tiled_band_workspace_bytes(const occgrid_geom* geom, int n_segs, int64_t seg_cap);
 int tiled_prepare_poses(const occgrid_geom* geom, const PoseRec* d_recs, const int* d_tiles, const SegInfo& seg, int tiles_in_records,
                         void* d_ws, size_t ws_bytes, uint64_t* d_counters, cudaStream_t st);

@@ -106,7 +106,10 @@ int occgrid_band_raycast_route(const occgrid_geom* band_geom, const void* d_recv
     if (occgrid_band_workspace_bytes(band_geom, n_segs, seg_capacity) == 0) return OCCGRID_E_ARG;
     RouteJob J = {};
     if (job && job->n > 0) {
-        if (!job->d_packets || !job->d_agent_off || job->n_agents < 1 || !job->d_peer_recs || !job->d_peer_tiles || !job->d_resv || !job->d_status) {
+        const PacketBatch batch = {job->d_packets, job->n, job->stride, job->d_agent_idx, job->d_drift, job->d_agent_off, job->n_agents};
+        rc = check_packet_batch(batch, job->rec_len, "band_raycast_route: ");
+        if (rc != OCCGRID_OK) return rc;
+        if (!job->d_peer_recs || !job->d_peer_tiles || !job->d_resv || !job->d_status) {
             set_last_error("band_raycast_route: NULL pointer in the route job");
             return OCCGRID_E_ARG;
         }
@@ -114,11 +117,10 @@ int occgrid_band_raycast_route(const occgrid_geom* band_geom, const void* d_recv
             set_last_error("band_raycast_route: n_bands must be 1..32 and src_rank one of them");
             return OCCGRID_E_ARG;
         }
-        if (job->rec_len != OCCGRID_PACKET_SIZE && job->rec_len != OCCGRID_PACKET_SIZE_V1) { set_last_error("band_raycast_route: rec_len must be 42 or 41"); return OCCGRID_E_ARG; }
-        if (job->stride < job->rec_len || job->stride > 64) { set_last_error("band_raycast_route: bad stride %d", job->stride); return OCCGRID_E_ARG; }
         if ((uint64_t)job->ordinal_base + (uint64_t)job->n > (1ull << 29) - 1) { set_last_error("band_raycast_route: ordinals must stay below 2^29-1"); return OCCGRID_E_ARG; }
         if (job->seg_capacity != seg_capacity) { set_last_error("band_raycast_route: the job's segment capacity differs from the slot's"); return OCCGRID_E_ARG; }
-        const int reach = (int)ceil(OCC_MAX_DIST_M / job->res) + 2;
+        const TileGeom tg = tile_geom(job->res, job->size_x, 0);      // bands are full-width rows: only reach, pad and tiles_x are used
+        const int reach = tg.reach;
         for (int b = 0; b < job->n_bands; ++b)
             if (job->band_y0[b + 1] - job->band_y0[b] < 2 * reach + 1 && job->n_bands > 1) {
                 set_last_error("band_raycast_route: band %d is thinner than 2 * reach + 1 = %d rows (a packet may reach at most two bands)", b, 2 * reach + 1);
@@ -128,9 +130,7 @@ int occgrid_band_raycast_route(const occgrid_geom* band_geom, const void* d_recv
         J.agent_idx = job->d_agent_idx; J.drift = job->d_drift; J.agent_off = job->d_agent_off; J.n_agents = job->n_agents;
         J.ordinal_base = job->ordinal_base;
         J.ox = job->ox; J.oy = job->oy; J.res = job->res; J.inv_res = 1.0 / job->res; J.size_x = job->size_x;
-        J.reach = reach;
-        J.pad = ((reach + 63) / 64) * 64;                              // tile_geom(): kTile = 64
-        J.tiles_x = (job->size_x + 2 * J.pad + 63) >> 6;
+        J.reach = tg.reach; J.pad = tg.pad; J.tiles_x = tg.tiles_x;
         J.n_bands = job->n_bands; J.src_rank = job->src_rank;
         for (int b = 0; b <= kMaxBands; ++b) J.band_y0[b] = job->band_y0[b <= job->n_bands ? b : job->n_bands];
         J.peer_recs = reinterpret_cast<PoseRec* const*>(job->d_peer_recs);

@@ -84,7 +84,6 @@ int validate_geom(const occgrid_geom* g) {
 // ------------------------------------------------------------------------------------------
 
 constexpr int kThreads = 256;          // threads (= packets) per CTA
-constexpr int kMaxStride = 64;         // bytes per record slot staged in shared memory
 
 // Walk one beam (exact reference Bresenham, :158-179) and raise the stamp of every cell the
 // sequential update_ray (:148-156) would have stored to: all cells but the last -> FREE,
@@ -140,15 +139,6 @@ __device__ __forceinline__ void count_beam_global(const Geom& g, int* __restrict
         atomicAdd(&counts[2 * ((size_t)(y - g.win_y0) * g.win_w + (x - g.win_x0)) + 1], 1);
 }
 
-// Cooperative copy of this CTA's records into shared memory with 16-byte loads.
-__device__ __forceinline__ void stage_records(const uint8_t* __restrict__ src, size_t bytes, uint8_t* smem) {
-    const size_t nvec = ((reinterpret_cast<uintptr_t>(src) & 15) == 0) ? bytes / 16 : 0;
-    const uint4* s4 = reinterpret_cast<const uint4*>(src);
-    uint4* d4 = reinterpret_cast<uint4*>(smem);
-    for (size_t i = threadIdx.x; i < nvec; i += blockDim.x) d4[i] = __ldg(s4 + i);
-    for (size_t i = nvec * 16 + threadIdx.x; i < bytes; i += blockDim.x) smem[i] = __ldg(src + i);
-}
-
 __device__ __forceinline__ bool start_in_window(const Geom& g, const Beam& b) {
     return b.valid && b.x0 >= g.win_x0 && b.x0 < g.win_x0 + g.win_w && b.y0 >= g.win_y0 && b.y0 < g.win_y0 + g.win_h;
 }
@@ -161,7 +151,7 @@ k_integrate_global(Geom g, const uint8_t* __restrict__ pkts, long long n, int st
                    const int32_t* __restrict__ agent_idx, const double* __restrict__ drift,
                    const double* __restrict__ agent_off, int n_agents,
                    unsigned int* __restrict__ stamps, uint64_t* counters, size_t map_cells = 0) {
-    __shared__ __align__(16) uint8_t s_rec[kThreads * kMaxStride];
+    __shared__ __align__(16) uint8_t s_rec[kThreads * kMaxRecStride];
     __shared__ unsigned long long s_acc[(OCCGRID_C_OWNED_UPDATES + 1) * 32];
     const long long first = (long long)blockIdx.x * kThreads;
     const int count = (int)min((long long)kThreads, n - first);
@@ -302,7 +292,6 @@ int device_sm_count() {
     }
     return by_device[dev];
 }
-static int sm_count() { return device_sm_count(); }
 
 // n_maps > 1: the planes and grids of an agent-map stack are contiguous, so one pass streams them all.
 static int launch_resolve(const occgrid_geom* geom, unsigned int* stamps, int8_t* grid, cudaStream_t st, int n_maps = 1) {
@@ -310,7 +299,7 @@ static int launch_resolve(const occgrid_geom* geom, unsigned int* stamps, int8_t
     const int vec_ok = ((reinterpret_cast<uintptr_t>(stamps) & 15) == 0 && (reinterpret_cast<uintptr_t>(grid) & 3) == 0) ? 1 : 0;
     size_t want = (n_cells / 4 + kThreads - 1) / kThreads;
     if (want < 1) want = 1;
-    const size_t cap = (size_t)sm_count() * 8;
+    const size_t cap = (size_t)device_sm_count() * 8;
     const int blocks = (int)(want < cap ? want : cap);
     ProfileScope ps(K_RESOLVE, st);
     k_resolve<<<blocks, kThreads, 0, st>>>(stamps, grid, n_cells, vec_ok);
@@ -318,54 +307,38 @@ static int launch_resolve(const occgrid_geom* geom, unsigned int* stamps, int8_t
     return OCCGRID_OK;
 }
 
-size_t global_workspace_bytes(const occgrid_geom* geom) {
-    return align_up((size_t)geom->win_w * geom->win_h * sizeof(unsigned int), 256);
+// One stamp plane per map, each the size of the window (agent maps: the whole grid).
+static size_t global_workspace_bytes(const occgrid_geom* geom, int n_maps) {
+    return align_up((size_t)geom->win_w * geom->win_h * (size_t)n_maps * sizeof(unsigned int), 256);
 }
 
-int integrate_packets_global(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride,
-                             const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
-                             int n_agents, int8_t* d_grid, void* d_ws, size_t ws_bytes, uint64_t* d_counters,
-                             cudaStream_t st) {
-    if (ws_bytes < global_workspace_bytes(geom)) {
-        set_last_error("workspace %zu B < %zu B needed by GLOBAL_ATOMIC", ws_bytes, global_workspace_bytes(geom));
+// Count planes take the beams' adds directly: no stamp plane, no workspace, no resolve.
+static int integrate_packets_global(const occgrid_geom* geom, const PacketBatch& b, Output kind, void* d_out, void* d_ws,
+                                    size_t ws_bytes, uint64_t* d_counters, cudaStream_t st) {
+    const int n_maps = kind == Output::kAgentMaps ? b.n_agents : 1;
+    const size_t need = global_workspace_bytes(geom, n_maps);
+    if (kind != Output::kCounts && ws_bytes < need) {
+        set_last_error("workspace %zu B < %zu B needed by GLOBAL_ATOMIC for %d map(s)", ws_bytes, need, n_maps);
         return OCCGRID_E_WORKSPACE;
     }
-    unsigned int* stamps = reinterpret_cast<unsigned int*>(d_ws);
+    unsigned int* stamps = reinterpret_cast<unsigned int*>(kind == Output::kCounts ? d_out : d_ws);
     const Geom g = to_geom(geom);
-    const long long blocks = (n + kThreads - 1) / kThreads;
+    const unsigned int blocks = (unsigned int)((b.n + kThreads - 1) / kThreads);
     {
         ProfileScope ps(K_INTEGRATE_GLOBAL, st);
-        k_integrate_global<false><<<(unsigned int)blocks, kThreads, 0, st>>>(g, d_packets, n, stride, d_agent_idx, d_drift,
-                                                                            d_agent_off, n_agents, stamps, d_counters);
+        if (kind == Output::kCounts)
+            k_integrate_global<true><<<blocks, kThreads, 0, st>>>(g, b.pkts, b.n, b.stride, b.agent_idx, b.drift, b.agent_off,
+                                                                  b.n_agents, stamps, d_counters);
+        else if (kind == Output::kAgentMaps)
+            k_integrate_global<false, true><<<blocks, kThreads, 0, st>>>(g, b.pkts, b.n, b.stride, b.agent_idx, b.drift, b.agent_off,
+                                                                         b.n_agents, stamps, d_counters, (size_t)geom->win_w * geom->win_h);
+        else
+            k_integrate_global<false><<<blocks, kThreads, 0, st>>>(g, b.pkts, b.n, b.stride, b.agent_idx, b.drift, b.agent_off,
+                                                                   b.n_agents, stamps, d_counters);
     }
     OCC_CUDA_TRY(cudaGetLastError());
-    return launch_resolve(geom, stamps, d_grid, st);
-}
-
-// Agent-map stack: n_agents stamp planes, each the size of the (whole-grid) window.
-size_t global_agent_maps_workspace_bytes(const occgrid_geom* geom, int n_agents) {
-    return align_up((size_t)geom->win_w * geom->win_h * (size_t)n_agents * sizeof(unsigned int), 256);
-}
-
-int integrate_packets_global_agent_maps(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride,
-                                        const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
-                                        int n_agents, int8_t* d_grids, void* d_ws, size_t ws_bytes, uint64_t* d_counters,
-                                        cudaStream_t st) {
-    const size_t need = global_agent_maps_workspace_bytes(geom, n_agents);
-    if (ws_bytes < need) {
-        set_last_error("workspace %zu B < %zu B needed by GLOBAL_ATOMIC for %d agent maps", ws_bytes, need, n_agents);
-        return OCCGRID_E_WORKSPACE;
-    }
-    unsigned int* stamps = reinterpret_cast<unsigned int*>(d_ws);
-    const long long blocks = (n + kThreads - 1) / kThreads;
-    {
-        ProfileScope ps(K_INTEGRATE_GLOBAL, st);
-        k_integrate_global<false, true><<<(unsigned int)blocks, kThreads, 0, st>>>(to_geom(geom), d_packets, n, stride, d_agent_idx,
-                                                                                  d_drift, d_agent_off, n_agents, stamps, d_counters,
-                                                                                  (size_t)geom->win_w * geom->win_h);
-    }
-    OCC_CUDA_TRY(cudaGetLastError());
-    return launch_resolve(geom, stamps, d_grids, st, n_agents);
+    if (kind == Output::kCounts) return OCCGRID_OK;
+    return launch_resolve(geom, stamps, reinterpret_cast<int8_t*>(d_out), st, n_maps);
 }
 
 // L = clamp(hits * l_occ + misses * l_free, l_min, l_max), derived from the integer planes so
@@ -450,25 +423,24 @@ k_probe_smem(unsigned int* out, unsigned int cells, int iters, unsigned int seed
 using namespace occ;
 
 namespace occ {
-size_t tiled_workspace_bytes(const occgrid_geom* geom, int64_t max_packets);
-int integrate_packets_tiled(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride,
-                            const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
-                            int n_agents, int8_t* d_grid, void* d_ws, size_t ws_bytes, uint64_t* d_counters,
-                            cudaStream_t st);
-bool tiled_supported(const occgrid_geom* geom);
-int accumulate_packets_tiled(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride,
-                             const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
-                             int n_agents, int32_t* d_counts, void* d_ws, size_t ws_bytes, uint64_t* d_counters,
-                             cudaStream_t st);
-void set_raycast_cta_cap(int cap);
-int integrate_poses_tiled(const occgrid_geom* geom, const void* d_poses, int64_t n, int ordinals_in_records, int8_t* d_grid,
-                          void* d_ws, size_t ws_bytes, uint64_t* d_counters, cudaStream_t st);
-size_t tiled_agent_maps_workspace_bytes(const occgrid_geom* geom, int n_agents, int64_t max_packets);
-bool tiled_agent_maps_supported(const occgrid_geom* geom, int n_agents);
-int integrate_packets_tiled_agent_maps(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride,
-                                       const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
-                                       int n_agents, int8_t* d_grids, void* d_ws, size_t ws_bytes, uint64_t* d_counters,
-                                       cudaStream_t st);
+
+int check_packet_batch(const PacketBatch& b, int rec_len, const char* who) {
+    if (b.n < 0 || b.n > (1ll << 29) - 1) {
+        set_last_error("%sn=%lld outside 0..2^29-1 records per call", who, (long long)b.n);
+        return OCCGRID_E_ARG;
+    }
+    if (rec_len != OCCGRID_PACKET_SIZE && rec_len != OCCGRID_PACKET_SIZE_V1) {
+        set_last_error("%srec_len must be 42 or 41, got %d", who, rec_len);
+        return OCCGRID_E_ARG;
+    }
+    if (b.stride < rec_len || b.stride > kMaxRecStride) {
+        set_last_error("%sstride %d outside %d..%d", who, b.stride, rec_len, kMaxRecStride);
+        return OCCGRID_E_ARG;
+    }
+    if (b.n_agents < 1 || !b.agent_off) { set_last_error("%sneed n_agents >= 1 and an agent offset table", who); return OCCGRID_E_ARG; }
+    if (b.n > 0 && !b.pkts) { set_last_error("%spackets is NULL", who); return OCCGRID_E_ARG; }
+    return OCCGRID_OK;
+}
 
 // Geometry of an agent-map stack: a valid geometry whose window is the whole grid, n_agents >= 1,
 // and a stack (of 4-byte stamps: the larger of the two) whose size fits size_t.
@@ -487,6 +459,41 @@ static int validate_agent_maps(const occgrid_geom* geom, int n_agents) {
     }
     return OCCGRID_OK;
 }
+
+// AUTO takes TILED wherever it supports the geometry and the number of maps.  An explicit TILED
+// that does not is E_RANGE; an unknown strategy is E_ARG.
+static int pick_strategy(const occgrid_geom* geom, int n_maps, int strategy, int* picked) {
+    if (strategy == OCCGRID_STRATEGY_AUTO) {
+        strategy = tiled_supported(geom, n_maps) ? OCCGRID_STRATEGY_TILED : OCCGRID_STRATEGY_GLOBAL_ATOMIC;
+    } else if (strategy == OCCGRID_STRATEGY_TILED && !tiled_supported(geom, n_maps)) {
+        set_last_error("TILED strategy does not support this geometry%s", n_maps > 1 ? " and agent count" : "");
+        return OCCGRID_E_RANGE;
+    } else if (strategy != OCCGRID_STRATEGY_TILED && strategy != OCCGRID_STRATEGY_GLOBAL_ATOMIC) {
+        set_last_error("unknown strategy %d", strategy);
+        return OCCGRID_E_ARG;
+    }
+    *picked = strategy;
+    return OCCGRID_OK;
+}
+
+static size_t workspace_bytes(const occgrid_geom* geom, int n_maps, int64_t max_packets, int strategy) {
+    if (max_packets < 0) { set_last_error("max_packets < 0"); return 0; }
+    int s;
+    if (pick_strategy(geom, n_maps, strategy, &s) != OCCGRID_OK) return 0;
+    return s == OCCGRID_STRATEGY_TILED ? tiled_workspace_bytes(geom, n_maps, max_packets) : global_workspace_bytes(geom, n_maps);
+}
+
+// The packet entry points once the batch and their output have been checked.
+static int integrate_packets(const occgrid_geom* geom, const PacketBatch& b, Output kind, void* d_out, void* d_ws, size_t ws_bytes,
+                             uint64_t* d_counters, int strategy, void* stream) {
+    if (b.n == 0) return OCCGRID_OK;
+    int s;
+    const int rc = pick_strategy(geom, kind == Output::kAgentMaps ? b.n_agents : 1, strategy, &s);
+    if (rc != OCCGRID_OK) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (s == OCCGRID_STRATEGY_TILED) return integrate_tiled(geom, b, nullptr, 0, kind, d_out, d_ws, ws_bytes, d_counters, st);
+    return integrate_packets_global(geom, b, kind, d_out, d_ws, ws_bytes, d_counters, st);
+}
 }
 
 extern "C" {
@@ -495,22 +502,14 @@ int occgrid_abi_version(void) { return OCCGRID_ABI_VERSION; }
 
 const char* occgrid_last_error(void) { return g_last_error.c_str(); }
 
-static int pick_strategy(const occgrid_geom* geom, int strategy) {
-    if (strategy == OCCGRID_STRATEGY_AUTO) return tiled_supported(geom) ? OCCGRID_STRATEGY_TILED : OCCGRID_STRATEGY_GLOBAL_ATOMIC;
-    return strategy;
-}
-
 size_t occgrid_workspace_bytes(const occgrid_geom* geom, int64_t max_packets, int strategy) {
     if (validate_geom(geom) != OCCGRID_OK) return 0;
-    if (max_packets < 0) { set_last_error("max_packets < 0"); return 0; }
-    const int s = pick_strategy(geom, strategy);
-    if (s == OCCGRID_STRATEGY_GLOBAL_ATOMIC) return global_workspace_bytes(geom);
-    if (s == OCCGRID_STRATEGY_TILED) {
-        if (!tiled_supported(geom)) { set_last_error("TILED strategy does not support this geometry"); return 0; }
-        return tiled_workspace_bytes(geom, max_packets);
-    }
-    set_last_error("unknown strategy %d", strategy);
-    return 0;
+    return workspace_bytes(geom, 1, max_packets, strategy);
+}
+
+size_t occgrid_agent_maps_workspace_bytes(const occgrid_geom* geom, int n_agents, int64_t max_packets, int strategy) {
+    if (validate_agent_maps(geom, n_agents) != OCCGRID_OK) return 0;
+    return workspace_bytes(geom, n_agents, max_packets, strategy);
 }
 
 int occgrid_workspace_reset(void* d_workspace, size_t workspace_bytes, void* stream) {
@@ -523,117 +522,36 @@ int occgrid_integrate_packets(const occgrid_geom* geom, const uint8_t* d_packets
                               const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
                               int n_agents, int8_t* d_grid, void* d_workspace, size_t workspace_bytes,
                               uint64_t* d_counters, int strategy, void* stream) {
+    const PacketBatch b = {d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents};
     int rc = validate_geom(geom);
+    if (rc == OCCGRID_OK) rc = check_packet_batch(b, rec_len, "");
     if (rc != OCCGRID_OK) return rc;
-    if (n < 0 || n > (1ll << 29) - 1) { set_last_error("n=%lld outside 0..2^29-1 records per call", (long long)n); return OCCGRID_E_ARG; }
-    if (rec_len != OCCGRID_PACKET_SIZE && rec_len != OCCGRID_PACKET_SIZE_V1) {
-        set_last_error("rec_len must be 42 or 41, got %d", rec_len);
-        return OCCGRID_E_ARG;
-    }
-    if (stride < rec_len || stride > kMaxStride) { set_last_error("stride %d outside %d..%d", stride, rec_len, kMaxStride); return OCCGRID_E_ARG; }
-    if (n_agents < 1 || !d_agent_off) { set_last_error("need n_agents >= 1 and an agent offset table"); return OCCGRID_E_ARG; }
     if (!d_grid || !d_workspace) { set_last_error("grid/workspace is NULL"); return OCCGRID_E_ARG; }
-    if (n == 0) return OCCGRID_OK;
-    if (!d_packets) { set_last_error("packets is NULL"); return OCCGRID_E_ARG; }
-    const int s = pick_strategy(geom, strategy);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (s == OCCGRID_STRATEGY_GLOBAL_ATOMIC)
-        return integrate_packets_global(geom, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents, d_grid,
-                                        d_workspace, workspace_bytes, d_counters, st);
-    if (s == OCCGRID_STRATEGY_TILED) {
-        if (!tiled_supported(geom)) { set_last_error("TILED strategy does not support this geometry"); return OCCGRID_E_RANGE; }
-        return integrate_packets_tiled(geom, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents, d_grid,
-                                       d_workspace, workspace_bytes, d_counters, st);
-    }
-    set_last_error("unknown strategy %d", strategy);
-    return OCCGRID_E_ARG;
-}
-
-static int pick_agent_maps_strategy(const occgrid_geom* geom, int n_agents, int strategy) {
-    if (strategy == OCCGRID_STRATEGY_AUTO)
-        return tiled_agent_maps_supported(geom, n_agents) ? OCCGRID_STRATEGY_TILED : OCCGRID_STRATEGY_GLOBAL_ATOMIC;
-    return strategy;
-}
-
-size_t occgrid_agent_maps_workspace_bytes(const occgrid_geom* geom, int n_agents, int64_t max_packets, int strategy) {
-    if (validate_agent_maps(geom, n_agents) != OCCGRID_OK) return 0;
-    if (max_packets < 0) { set_last_error("max_packets < 0"); return 0; }
-    const int s = pick_agent_maps_strategy(geom, n_agents, strategy);
-    if (s == OCCGRID_STRATEGY_GLOBAL_ATOMIC) return global_agent_maps_workspace_bytes(geom, n_agents);
-    if (s == OCCGRID_STRATEGY_TILED) {
-        if (!tiled_agent_maps_supported(geom, n_agents)) { set_last_error("TILED strategy does not support this geometry and agent count"); return 0; }
-        return tiled_agent_maps_workspace_bytes(geom, n_agents, max_packets);
-    }
-    set_last_error("unknown strategy %d", strategy);
-    return 0;
+    return integrate_packets(geom, b, Output::kGrid, d_grid, d_workspace, workspace_bytes, d_counters, strategy, stream);
 }
 
 int occgrid_integrate_packets_agent_maps(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride, int rec_len,
                                          const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
                                          int n_agents, int8_t* d_grids, void* d_workspace, size_t workspace_bytes,
                                          uint64_t* d_counters, int strategy, void* stream) {
+    const PacketBatch b = {d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents};
     int rc = validate_agent_maps(geom, n_agents);
+    if (rc == OCCGRID_OK) rc = check_packet_batch(b, rec_len, "");
     if (rc != OCCGRID_OK) return rc;
-    if (n < 0 || n > (1ll << 29) - 1) { set_last_error("n=%lld outside 0..2^29-1 records per call", (long long)n); return OCCGRID_E_ARG; }
-    if (rec_len != OCCGRID_PACKET_SIZE && rec_len != OCCGRID_PACKET_SIZE_V1) {
-        set_last_error("rec_len must be 42 or 41, got %d", rec_len);
-        return OCCGRID_E_ARG;
-    }
-    if (stride < rec_len || stride > kMaxStride) { set_last_error("stride %d outside %d..%d", stride, rec_len, kMaxStride); return OCCGRID_E_ARG; }
-    if (!d_agent_off) { set_last_error("need an agent offset table"); return OCCGRID_E_ARG; }
     if (!d_grids || !d_workspace) { set_last_error("grids/workspace is NULL"); return OCCGRID_E_ARG; }
-    if (n == 0) return OCCGRID_OK;
-    if (!d_packets) { set_last_error("packets is NULL"); return OCCGRID_E_ARG; }
-    const int s = pick_agent_maps_strategy(geom, n_agents, strategy);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (s == OCCGRID_STRATEGY_GLOBAL_ATOMIC)
-        return integrate_packets_global_agent_maps(geom, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents, d_grids,
-                                                   d_workspace, workspace_bytes, d_counters, st);
-    if (s == OCCGRID_STRATEGY_TILED) {
-        if (!tiled_agent_maps_supported(geom, n_agents)) {
-            set_last_error("TILED strategy does not support this geometry and agent count");
-            return OCCGRID_E_RANGE;
-        }
-        return integrate_packets_tiled_agent_maps(geom, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents, d_grids,
-                                                  d_workspace, workspace_bytes, d_counters, st);
-    }
-    set_last_error("unknown strategy %d", strategy);
-    return OCCGRID_E_ARG;
+    return integrate_packets(geom, b, Output::kAgentMaps, d_grids, d_workspace, workspace_bytes, d_counters, strategy, stream);
 }
 
 int occgrid_accumulate_packets(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride, int rec_len,
                                const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
                                int n_agents, int32_t* d_counts, void* d_workspace, size_t workspace_bytes,
                                uint64_t* d_counters, int strategy, void* stream) {
+    const PacketBatch b = {d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents};
     int rc = validate_geom(geom);
+    if (rc == OCCGRID_OK) rc = check_packet_batch(b, rec_len, "");
     if (rc != OCCGRID_OK) return rc;
-    if (n < 0 || n > (1ll << 29) - 1) { set_last_error("n=%lld outside 0..2^29-1 records per call", (long long)n); return OCCGRID_E_ARG; }
-    if (rec_len != OCCGRID_PACKET_SIZE && rec_len != OCCGRID_PACKET_SIZE_V1) {
-        set_last_error("rec_len must be 42 or 41, got %d", rec_len);
-        return OCCGRID_E_ARG;
-    }
-    if (stride < rec_len || stride > kMaxStride) { set_last_error("stride %d outside %d..%d", stride, rec_len, kMaxStride); return OCCGRID_E_ARG; }
-    if (n_agents < 1 || !d_agent_off) { set_last_error("need n_agents >= 1 and an agent offset table"); return OCCGRID_E_ARG; }
     if (!d_counts || (reinterpret_cast<uintptr_t>(d_counts) & 7) || !d_workspace) { set_last_error("counts (8-byte aligned) / workspace is NULL"); return OCCGRID_E_ARG; }
-    if (n == 0) return OCCGRID_OK;
-    if (!d_packets) { set_last_error("packets is NULL"); return OCCGRID_E_ARG; }
-    const int s = pick_strategy(geom, strategy);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (s == OCCGRID_STRATEGY_TILED) {
-        if (!tiled_supported(geom)) { set_last_error("TILED strategy does not support this geometry"); return OCCGRID_E_RANGE; }
-        return accumulate_packets_tiled(geom, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents, d_counts,
-                                        d_workspace, workspace_bytes, d_counters, st);
-    }
-    if (s != OCCGRID_STRATEGY_GLOBAL_ATOMIC) { set_last_error("unknown strategy %d", strategy); return OCCGRID_E_ARG; }
-    const long long blocks = (n + kThreads - 1) / kThreads;
-    {
-        ProfileScope ps(K_INTEGRATE_GLOBAL, st);
-        k_integrate_global<true><<<(unsigned int)blocks, kThreads, 0, st>>>(to_geom(geom), d_packets, n, stride, d_agent_idx, d_drift,
-                                                                           d_agent_off, n_agents, reinterpret_cast<unsigned int*>(d_counts),
-                                                                           d_counters);
-    }
-    OCC_CUDA_TRY(cudaGetLastError());
-    return OCCGRID_OK;
+    return integrate_packets(geom, b, Output::kCounts, d_counts, d_workspace, workspace_bytes, d_counters, strategy, stream);
 }
 
 int occgrid_counts_to_logodds(const int32_t* d_counts, int64_t n_cells, double l_occ, double l_free, double l_min, double l_max,
@@ -658,15 +576,18 @@ int occgrid_integrate_poses(const occgrid_geom* geom, const void* d_pose_recs, i
     if (!d_grid || !d_workspace) { set_last_error("grid/workspace is NULL"); return OCCGRID_E_ARG; }
     if (n == 0) return OCCGRID_OK;
     if (!d_pose_recs || (reinterpret_cast<uintptr_t>(d_pose_recs) & 15)) { set_last_error("pose records must be non-NULL and 16-byte aligned"); return OCCGRID_E_ARG; }
-    const int s = pick_strategy(geom, strategy);
+    int s;
+    rc = pick_strategy(geom, 1, strategy, &s);
+    if (rc != OCCGRID_OK) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     if (s == OCCGRID_STRATEGY_TILED) {
-        if (!tiled_supported(geom)) { set_last_error("TILED strategy does not support this geometry"); return OCCGRID_E_RANGE; }
-        return integrate_poses_tiled(geom, d_pose_recs, n, ordinals_in_records, d_grid, d_workspace, workspace_bytes, d_counters, st);
+        PacketBatch b = {};
+        b.n = n;
+        return integrate_tiled(geom, b, reinterpret_cast<const PoseRec*>(d_pose_recs), ordinals_in_records, Output::kGrid, d_grid,
+                               d_workspace, workspace_bytes, d_counters, st);
     }
-    if (s != OCCGRID_STRATEGY_GLOBAL_ATOMIC) { set_last_error("unknown strategy %d", strategy); return OCCGRID_E_ARG; }
-    if (workspace_bytes < global_workspace_bytes(geom)) {
-        set_last_error("workspace %zu B < %zu B needed by GLOBAL_ATOMIC", workspace_bytes, global_workspace_bytes(geom));
+    if (workspace_bytes < global_workspace_bytes(geom, 1)) {
+        set_last_error("workspace %zu B < %zu B needed by GLOBAL_ATOMIC", workspace_bytes, global_workspace_bytes(geom, 1));
         return OCCGRID_E_WORKSPACE;
     }
     unsigned int* stamps = reinterpret_cast<unsigned int*>(d_workspace);
@@ -691,8 +612,8 @@ int occgrid_update_rays(const occgrid_geom* geom, const double* d_rays, const ui
     if (n == 0) return OCCGRID_OK;
     if (!d_rays || !d_hit) { set_last_error("rays/hit is NULL"); return OCCGRID_E_ARG; }
     if (reinterpret_cast<uintptr_t>(d_rays) & 15) { set_last_error("rays must be 16-byte aligned"); return OCCGRID_E_ARG; }
-    if (workspace_bytes < global_workspace_bytes(geom)) {
-        set_last_error("workspace %zu B < %zu B needed by update_rays", workspace_bytes, global_workspace_bytes(geom));
+    if (workspace_bytes < global_workspace_bytes(geom, 1)) {
+        set_last_error("workspace %zu B < %zu B needed by update_rays", workspace_bytes, global_workspace_bytes(geom, 1));
         return OCCGRID_E_WORKSPACE;
     }
     unsigned int* stamps = reinterpret_cast<unsigned int*>(d_workspace);

@@ -24,15 +24,13 @@
 namespace occ {
 
 constexpr int kRT = 256;
-constexpr int kRouteMaxBands = 32;
-constexpr int kRouteMaxStride = 64;
 
 struct RouteParams {
     double oy, res;
     int size_y;
     int reach;                       // cells
     int n_bands;
-    int band_y0[kRouteMaxBands + 1]; // row boundaries, band b = [band_y0[b], band_y0[b+1])
+    int band_y0[kMaxBands + 1];      // row boundaries, band b = [band_y0[b], band_y0[b+1])
 };
 
 // Bands whose rows intersect [gy - reach, gy + reach]; 0 for packets that are dropped, have a
@@ -58,26 +56,18 @@ __device__ __forceinline__ unsigned int band_mask(const RouteParams& P, const ui
     return m;
 }
 
-__device__ __forceinline__ void stage(const uint8_t* __restrict__ src, size_t bytes, uint8_t* smem) {
-    const size_t nvec = ((reinterpret_cast<uintptr_t>(src) & 15) == 0) ? bytes / 16 : 0;
-    const uint4* s4 = reinterpret_cast<const uint4*>(src);
-    uint4* d4 = reinterpret_cast<uint4*>(smem);
-    for (size_t i = threadIdx.x; i < nvec; i += blockDim.x) d4[i] = __ldg(s4 + i);
-    for (size_t i = nvec * 16 + threadIdx.x; i < bytes; i += blockDim.x) smem[i] = __ldg(src + i);
-}
-
 __global__ void __launch_bounds__(kRT)
 k_route_count(RouteParams P, const uint8_t* __restrict__ pkts, long long n, int stride,
               const int32_t* __restrict__ agent_idx, const double* __restrict__ drift,
               const double* __restrict__ agent_off, int n_agents,
               unsigned int* __restrict__ hist /* [n_bands][n_blocks] */, int n_blocks, uint64_t* counters) {
-    __shared__ __align__(16) uint8_t s_rec[kRT * kRouteMaxStride];
-    __shared__ unsigned int s_hist[kRouteMaxBands];
+    __shared__ __align__(16) uint8_t s_rec[kRT * kMaxRecStride];
+    __shared__ unsigned int s_hist[kMaxBands];
     __shared__ unsigned long long s_acc[4 * 32];
     const long long first = (long long)blockIdx.x * kRT;
     const int count = (int)min((long long)kRT, n - first);
-    if (threadIdx.x < kRouteMaxBands) s_hist[threadIdx.x] = 0;
-    stage(pkts + (size_t)first * stride, (size_t)count * stride, s_rec);
+    if (threadIdx.x < kMaxBands) s_hist[threadIdx.x] = 0;
+    stage_records(pkts + (size_t)first * stride, (size_t)count * stride, s_rec);
     __syncthreads();
     unsigned int m = 0;
     int st = -1;
@@ -143,12 +133,12 @@ k_route_scatter(RouteParams P, const uint8_t* __restrict__ pkts, long long n, in
                 const double* __restrict__ agent_off, int n_agents,
                 const unsigned int* __restrict__ hist, int n_blocks, const int* __restrict__ status,
                 PoseRec* __restrict__ send) {
-    __shared__ __align__(16) uint8_t s_rec[kRT * kRouteMaxStride];
+    __shared__ __align__(16) uint8_t s_rec[kRT * kMaxRecStride];
     __shared__ unsigned int s_woff[kRT / 32];
     if (*status & 1) return;                                   // send buffer too small: nothing is written
     const long long first = (long long)blockIdx.x * kRT;
     const int count = (int)min((long long)kRT, n - first);
-    stage(pkts + (size_t)first * stride, (size_t)count * stride, s_rec);
+    stage_records(pkts + (size_t)first * stride, (size_t)count * stride, s_rec);
     __syncthreads();
     unsigned int m = 0;
     int st;
@@ -190,21 +180,20 @@ int occgrid_route_packets(const occgrid_geom* geom, int n_bands, const int32_t* 
                           void* d_ws, size_t ws_bytes, void* stream) {
     int rc = validate_geom(geom);
     if (rc != OCCGRID_OK) return rc;
-    if (n_bands < 1 || n_bands > kRouteMaxBands || !band_y0_host) { set_last_error("route: n_bands must be 1..32"); return OCCGRID_E_ARG; }
-    if (n < 0 || n > (1ll << 29) - 1) { set_last_error("route: n outside 0..2^29-1"); return OCCGRID_E_ARG; }
-    if (rec_len != OCCGRID_PACKET_SIZE && rec_len != OCCGRID_PACKET_SIZE_V1) { set_last_error("route: rec_len must be 42 or 41"); return OCCGRID_E_ARG; }
-    if (stride < rec_len || stride > kRouteMaxStride) { set_last_error("route: bad stride %d", stride); return OCCGRID_E_ARG; }
-    if (!d_send || !d_band_counts || !d_status || !d_ws || !d_agent_off || n_agents < 1) { set_last_error("route: NULL argument"); return OCCGRID_E_ARG; }
+    if (n_bands < 1 || n_bands > kMaxBands || !band_y0_host) { set_last_error("route: n_bands must be 1..32"); return OCCGRID_E_ARG; }
+    rc = check_packet_batch(PacketBatch{d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents}, rec_len, "route: ");
+    if (rc != OCCGRID_OK) return rc;
+    if (!d_send || !d_band_counts || !d_status || !d_ws) { set_last_error("route: NULL argument"); return OCCGRID_E_ARG; }
     if (reinterpret_cast<uintptr_t>(d_send) & 15) { set_last_error("route: send buffer must be 16-byte aligned"); return OCCGRID_E_ARG; }
     if (send_capacity >= (1ll << 32)) { set_last_error("route: send capacity must be < 2^32 records"); return OCCGRID_E_ARG; }
     if (ws_bytes < occgrid_route_workspace_bytes(n, n_bands)) { set_last_error("route: workspace too small"); return OCCGRID_E_WORKSPACE; }
     cudaStream_t st = (cudaStream_t)stream;
     RouteParams P;
     P.oy = geom->oy; P.res = geom->res; P.size_y = geom->size_y;
-    P.reach = (int)ceil(OCC_MAX_DIST_M / geom->res) + 2;
+    P.reach = reach_cells(geom->res);
     P.n_bands = n_bands;
     for (int b = 0; b <= n_bands; ++b) P.band_y0[b] = band_y0_host[b];
-    for (int b = n_bands + 1; b <= kRouteMaxBands; ++b) P.band_y0[b] = band_y0_host[n_bands];
+    for (int b = n_bands + 1; b <= kMaxBands; ++b) P.band_y0[b] = band_y0_host[n_bands];
     const int blocks = (int)((n + kRT - 1) / kRT);
     unsigned int* hist = reinterpret_cast<unsigned int*>(reinterpret_cast<char*>(d_ws) + 256);
     if (n == 0) {

@@ -26,14 +26,10 @@
 //
 // Windows of neighbouring tiles overlap; the global atomicMax merges them, and chunks of one
 // tile likewise, so the result is independent of how work was cut.
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace occ {
 
-constexpr int kTile = 64;            // home-tile side in cells
-constexpr int kTileShift = 6;
 constexpr int kTT = 256;             // threads per CTA
 // Packets per work item: chosen per batch by k_tile_plan so that the persistent raycast CTAs get
 // ~kItemsPerCta items each: a small batch cut into 2 048-packet items would leave most CTAs without
@@ -43,7 +39,6 @@ constexpr int kChunkPk = 2048;       // largest work item
 constexpr int kChunkMin = 256;       // smallest: one packet per thread
 constexpr int kItemsPerCta = 3;       // raycast of configs[1]: 3 -> 0.202 ms, 5 -> 0.220, 8 -> 0.235, 12 -> 0.263; cutting only the
                                       // last quarter of the queue 4x / 8x finer: 0.201 / 0.215 against 0.198
-constexpr int kMaxStrideT = 64;
 constexpr int kMaxWindowBytes = 100 * 1024;   // smem window budget (two CTAs per SM at least)
 
 struct TilePlanHeader {
@@ -51,37 +46,6 @@ struct TilePlanHeader {
     unsigned int active_count;   // tiles appended to the active list by the count pass of the current call
     unsigned int pad;
 };
-
-struct TileGeom {
-    int reach;            // R
-    int pad;              // cells added around the window so that every home tile is >= 0
-    int tiles_x, tiles_y, n_tiles;
-    int win_side;         // smem window side = kTile + 2R
-    int pitch;            // smem row pitch (odd)
-};
-
-static inline int reach_cells(double res) { return (int)ceil(OCC_MAX_DIST_M / res) + 2; }
-__device__ __forceinline__ int reach_cells_dev(double res) { return (int)ceil(OCC_MAX_DIST_M / res) + 2; }
-
-static inline TileGeom tile_geom(const occgrid_geom* g) {
-    TileGeom t;
-    t.reach = reach_cells(g->res);
-    t.pad = ((t.reach + kTile - 1) / kTile) * kTile;
-    t.tiles_x = (g->win_w + 2 * t.pad + kTile - 1) >> kTileShift;
-    t.tiles_y = (g->win_h + 2 * t.pad + kTile - 1) >> kTileShift;
-    t.n_tiles = t.tiles_x * t.tiles_y;
-    t.win_side = kTile + 2 * t.reach;
-    t.pitch = t.win_side | 1;
-    return t;
-}
-
-__device__ __forceinline__ void stage_records_t(const uint8_t* __restrict__ src, size_t bytes, uint8_t* smem) {
-    const size_t nvec = ((reinterpret_cast<uintptr_t>(src) & 15) == 0) ? bytes / 16 : 0;
-    const uint4* s4 = reinterpret_cast<const uint4*>(src);
-    uint4* d4 = reinterpret_cast<uint4*>(smem);
-    for (size_t i = threadIdx.x; i < nvec; i += blockDim.x) d4[i] = __ldg(s4 + i);
-    for (size_t i = nvec * 16 + threadIdx.x; i < bytes; i += blockDim.x) smem[i] = __ldg(src + i);
-}
 
 // Home tile of a corrected pose, or -1 when no beam of the packet can reach the window.
 __device__ __forceinline__ int home_tile(const Geom& g, const TileGeom& tg, double rx, double ry) {
@@ -165,7 +129,7 @@ __device__ __forceinline__ void reserve_tile_ranges(const unsigned int* s_keys, 
 //
 // kMaps (occgrid_integrate_packets_agent_maps): the map is folded into the tile KEY, (agent - 1) *
 // n_tiles + home tile.  Everything below and the plan and placement passes work on keys unchanged.
-constexpr size_t kBinSmem = (size_t)kTT * kMaxStrideT + 2 * kHash * sizeof(unsigned int) + kPkPerCta * sizeof(unsigned short);
+constexpr size_t kBinSmem = (size_t)kTT * kMaxRecStride + 2 * kHash * sizeof(unsigned int) + kPkPerCta * sizeof(unsigned short);
 constexpr unsigned int kNoSlot = 0xffffu;
 
 template <bool kMaps = false>
@@ -178,7 +142,7 @@ k_home_bin(Geom g, TileGeom tg, const uint8_t* __restrict__ pkts, long long n, i
            uint64_t* counters) {
     extern __shared__ __align__(16) uint8_t s_bin[];                                  // kBinSmem
     uint8_t* const s_rec = s_bin;                                                     // staged records, later the local bin list
-    unsigned int* const s_keys = reinterpret_cast<unsigned int*>(s_bin + kTT * kMaxStrideT);
+    unsigned int* const s_keys = reinterpret_cast<unsigned int*>(s_bin + kTT * kMaxRecStride);
     unsigned int* const s_vals = s_keys + kHash;
     unsigned short* const s_slot = reinterpret_cast<unsigned short*>(s_vals + kHash);   // hash slot of every packet, or kNoSlot
     __shared__ unsigned int s_wsum[kTT / 32];
@@ -187,7 +151,7 @@ k_home_bin(Geom g, TileGeom tg, const uint8_t* __restrict__ pkts, long long n, i
     const long long cta_first = (long long)blockIdx.x * kPkPerCta;
     // Software-pipelined staging: the 16-byte loads of sub-batch s+1 are in flight while
     // sub-batch s is decoded out of shared memory.
-    constexpr int kVec = (kTT * kMaxStrideT / 16 + kTT - 1) / kTT;      // uint4 per thread per sub-batch (<= 4)
+    constexpr int kVec = (kTT * kMaxRecStride / 16 + kTT - 1) / kTT;      // uint4 per thread per sub-batch (<= 4)
     uint4 pre[kVec];
     auto prefetch = [&](int sub) {
         const long long first = cta_first + (long long)sub * kTT;
@@ -218,7 +182,7 @@ k_home_bin(Geom g, TileGeom tg, const uint8_t* __restrict__ pkts, long long n, i
             for (size_t i = (bytes / 16) * 16 + threadIdx.x; i < bytes; i += kTT) s_rec[i] = __ldg(pkts + (size_t)first * stride + i);
             if (sub + 1 < kSub) prefetch(sub + 1);
         } else {
-            stage_records_t(pkts + (size_t)first * stride, (size_t)count * stride, s_rec);
+            stage_records(pkts + (size_t)first * stride, (size_t)count * stride, s_rec);
         }
         __syncthreads();
         if ((int)threadIdx.x < count) {
@@ -352,7 +316,7 @@ __device__ __forceinline__ int chunk_valid(const SegInfo& seg, long long chunk, 
     return cnt > j0 ? (int)min((unsigned int)kSegChunk, cnt - j0) : 0;
 }
 
-// Same as k_home_count for input that is already decoded (routed pose records, binned in place).
+// The count pass for input that is already decoded (routed pose records, binned in place).
 // The buffer is a set of per-source segments whose fill counts live on the device; persistent
 // CTAs stride over 2048-address chunks and skip the empty ones.  `tiles_in_records`: the router
 // already computed the home tile for THIS window (rec.tile), nothing is re-derived here.
@@ -417,46 +381,6 @@ k_home_count_poses(Geom g, TileGeom tg, const PoseRec* __restrict__ recs, const 
     }
     block_add_counters(c, s_acc, counters);
 }
-
-__global__ void __launch_bounds__(kTT)
-k_home_scatter(long long n, const int* __restrict__ tile_ids, const unsigned int* __restrict__ tile_offset,
-               unsigned int* __restrict__ tile_cursor, const TilePlanHeader* __restrict__ hdr,
-               unsigned int* __restrict__ bins) {
-    __shared__ unsigned int s_keys[kHash];
-    __shared__ unsigned int s_vals[kHash];
-    if (hdr->overflow) return;
-    for (int i = threadIdx.x; i < kHash; i += kTT) { s_keys[i] = kEmpty; s_vals[i] = 0u; }
-    __syncthreads();
-    const long long cta_first = (long long)blockIdx.x * kPkPerCta;
-    unsigned int where[kSub];          // (hash slot << 16) | rank within this CTA's share of the tile
-    int tl[kSub];
-#pragma unroll
-    for (int sub = 0; sub < kSub; ++sub) {
-        const long long k = cta_first + (long long)sub * kTT + threadIdx.x;
-        tl[sub] = k < n ? tile_ids[k] : -1;
-    }
-#pragma unroll
-    for (int sub = 0; sub < kSub; ++sub) {
-        const long long k = cta_first + (long long)sub * kTT + threadIdx.x;
-        where[sub] = kEmpty;
-        if (k < n) {
-            const int tile = tl[sub];
-            if (tile >= 0) {
-                const int h = hash_insert(s_keys, (unsigned int)tile);
-                where[sub] = ((unsigned int)h << 16) | atomicAdd(&s_vals[h], 1u);
-            }
-        }
-    }
-    __syncthreads();
-    reserve_tile_ranges(s_keys, s_vals, tile_offset, tile_cursor);          // one reservation per distinct tile
-    __syncthreads();
-#pragma unroll
-    for (int sub = 0; sub < kSub; ++sub) {
-        const long long k = cta_first + (long long)sub * kTT + threadIdx.x;
-        if (where[sub] != kEmpty) bins[s_vals[where[sub] >> 16] + (where[sub] & 0xffffu)] = (unsigned int)k;
-    }
-}
-
 
 // Scatter for segmented record buffers: bins hold record ADDRESSES (segment * seg_cap + index).
 __global__ void __launch_bounds__(kTT)
@@ -935,7 +859,7 @@ __device__ __noinline__ RouteStats route_item(const RouteJob& J, unsigned int it
             // would pay one DRAM latency per iteration)
             const uint8_t* src = J.pkts + (size_t)first * J.stride;
             const size_t bytes = (size_t)count * J.stride;
-            constexpr int kVec = kRouteItemPk * kMaxStrideT / 16 / kTT;         // <= 8 chunks of 16 bytes per thread
+            constexpr int kVec = kRouteItemPk * kMaxRecStride / 16 / kTT;         // <= 8 chunks of 16 bytes per thread
             if ((reinterpret_cast<uintptr_t>(src) & 15) == 0) {
                 const uint4* s4 = reinterpret_cast<const uint4*>(src);
                 uint4* d4 = reinterpret_cast<uint4*>(s_buf);
@@ -953,7 +877,7 @@ __device__ __noinline__ RouteStats route_item(const RouteJob& J, unsigned int it
                 }
                 for (size_t i = nvec * 16 + threadIdx.x; i < bytes; i += kTT) reinterpret_cast<uint8_t*>(s_buf)[i] = __ldg(src + i);
             } else {
-                stage_records_t(src, bytes, reinterpret_cast<uint8_t*>(s_buf));
+                stage_records(src, bytes, reinterpret_cast<uint8_t*>(s_buf));
             }
         }
         {   // pull the NEXT sub-batch towards L2 while this one is decoded, sorted and copied out
@@ -1267,22 +1191,13 @@ static TiledLayout tiled_layout(const occgrid_geom* geom, int64_t max_records, b
     return L;
 }
 
-bool tiled_supported(const occgrid_geom* geom) {
+bool tiled_supported(const occgrid_geom* geom, int n_maps) {
     const TileGeom tg = tile_geom(geom);
-    return (size_t)tg.win_side * tg.pitch * 4 <= (size_t)kMaxWindowBytes && tg.n_tiles <= (1 << 24);
+    return (size_t)tg.win_side * tg.pitch * 4 <= (size_t)kMaxWindowBytes && (long long)n_maps * tg.n_tiles <= (1ll << 24);
 }
 
-size_t tiled_workspace_bytes(const occgrid_geom* geom, int64_t max_packets) {
-    return tiled_layout(geom, max_packets < 1 ? 1 : max_packets, true).total;
-}
-
-// Keys (map * n_tiles + tile) stay below 2^24, as tiles do on one grid.
-bool tiled_agent_maps_supported(const occgrid_geom* geom, int n_agents) {
-    return tiled_supported(geom) && (long long)n_agents * tile_geom(geom).n_tiles <= (1ll << 24);
-}
-
-size_t tiled_agent_maps_workspace_bytes(const occgrid_geom* geom, int n_agents, int64_t max_packets) {
-    return tiled_layout(geom, max_packets < 1 ? 1 : max_packets, true, n_agents).total;
+size_t tiled_workspace_bytes(const occgrid_geom* geom, int n_maps, int64_t max_packets) {
+    return tiled_layout(geom, max_packets < 1 ? 1 : max_packets, true, n_maps).total;
 }
 
 size_t tiled_band_workspace_bytes(const occgrid_geom* geom, int n_segs, int64_t seg_cap) {
@@ -1322,7 +1237,7 @@ static TiledPtrs tiled_ptrs(const TiledLayout& L, void* d_ws) {
 static size_t raycast_smem(const TileGeom& tg, bool route) {
     size_t b = (size_t)tg.win_side * tg.pitch * 4;
     const size_t r = (size_t)kRouteItemPk * 2 * sizeof(PoseRec);   // every packet may go to two bands
-    const size_t raw = (size_t)kRouteItemPk * kMaxStrideT;
+    const size_t raw = (size_t)kRouteItemPk * kMaxRecStride;
     if (route) b = b > r ? b : r;
     if (route) b = b > raw ? b : raw;
     return b;
@@ -1349,14 +1264,7 @@ static int launch_raycast(const Geom& g, const TileGeom& tg, const TiledPtrs& P,
 }
 
 // Work items the plan aims for: kItemsPerCta per persistent raycast CTA (three CTAs per SM).
-static unsigned int plan_target_items() {
-    static unsigned int forced = 0xffffffffu;          // OCC_PLAN_ITEMS_PER_CTA: tuning hook
-    if (forced == 0xffffffffu) {
-        const char* e = getenv("OCC_PLAN_ITEMS_PER_CTA");
-        forced = e ? (unsigned int)atoi(e) : 0u;
-    }
-    return (unsigned int)device_sm_count() * 3u * (forced ? forced : (unsigned int)kItemsPerCta);
-}
+static unsigned int plan_target_items() { return (unsigned int)device_sm_count() * 3u * (unsigned int)kItemsPerCta; }
 
 static int grid_chunks(long long n_chunks) {
     long long b = n_chunks < 1 ? 1 : n_chunks;
@@ -1364,14 +1272,13 @@ static int grid_chunks(long long n_chunks) {
     return (int)(b < cap ? b : cap);
 }
 
-// `d_poses` != NULL: input is n PoseRec (already decoded and corrected), `d_packets` etc. unused.
-// `maps` (packets into the grid only): d_grid is a stack of n_agents grids, agent a's at a - 1.
-int integrate_tiled(const occgrid_geom* geom, const uint8_t* d_packets, const PoseRec* d_poses, int ordinals_in_records,
-                    int64_t n, int stride,
-                    const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
-                    int n_agents, int8_t* d_grid, int32_t* d_counts, void* d_ws, size_t ws_bytes, uint64_t* d_counters,
-                    cudaStream_t st, bool maps = false) {
-    const TiledLayout L = tiled_layout(geom, n, d_poses == nullptr, maps ? n_agents : 1);
+// Pose records are binned like a band's receive slot of one segment: count, plan and scatter run
+// over 2048-record chunks of it.
+int integrate_tiled(const occgrid_geom* geom, const PacketBatch& batch, const PoseRec* d_poses, int ordinals_in_records, Output kind,
+                    void* d_out, void* d_ws, size_t ws_bytes, uint64_t* d_counters, cudaStream_t st) {
+    const int64_t n = batch.n;
+    const bool maps = kind == Output::kAgentMaps;
+    const TiledLayout L = tiled_layout(geom, n, d_poses == nullptr, maps ? batch.n_agents : 1);
     if (ws_bytes < L.total) {
         set_last_error("workspace %zu B < %zu B needed by TILED for %lld records", ws_bytes, L.total, (long long)n);
         return OCCGRID_E_WORKSPACE;
@@ -1389,14 +1296,11 @@ int integrate_tiled(const occgrid_geom* geom, const uint8_t* d_packets, const Po
         if (d_poses) {
             k_home_count_poses<<<grid_chunks(n_chunks), kTT, 0, st>>>(g, tg, d_poses, nullptr, seg, n_chunks, 0, P.tile_count, P.tile_ids, P.active,
                                                                       P.hdr, d_counters);
-        } else if (maps) {
-            OCC_CUDA_TRY(cudaFuncSetAttribute(k_home_bin<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBinSmem));
-            k_home_bin<true><<<blocks, kTT, kBinSmem, st>>>(g, tg, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents,
-                                                            P.tile_count, P.recs, P.local_bins, P.runs, P.seg_count, P.active, P.hdr, d_counters);
         } else {
-            OCC_CUDA_TRY(cudaFuncSetAttribute(k_home_bin<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBinSmem));
-            k_home_bin<false><<<blocks, kTT, kBinSmem, st>>>(g, tg, d_packets, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents,
-                                                             P.tile_count, P.recs, P.local_bins, P.runs, P.seg_count, P.active, P.hdr, d_counters);
+            const auto bin = maps ? k_home_bin<true> : k_home_bin<false>;
+            OCC_CUDA_TRY(cudaFuncSetAttribute(bin, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBinSmem));
+            bin<<<blocks, kTT, kBinSmem, st>>>(g, tg, batch.pkts, n, batch.stride, batch.agent_idx, batch.drift, batch.agent_off, batch.n_agents,
+                                               P.tile_count, P.recs, P.local_bins, P.runs, P.seg_count, P.active, P.hdr, d_counters);
         }
     }
     {
@@ -1406,17 +1310,18 @@ int integrate_tiled(const occgrid_geom* geom, const uint8_t* d_packets, const Po
     }
     {
         ProfileScope ps(K_TILE_SCATTER, st);
-        if (d_poses) k_home_scatter<<<blocks, kTT, 0, st>>>(n, P.tile_ids, P.tile_offset, P.tile_cursor, P.hdr, P.bins);
+        if (d_poses) k_home_scatter_segs<<<grid_chunks(n_chunks), kTT, 0, st>>>(seg, n_chunks, P.tile_ids, P.tile_offset, P.tile_cursor, P.hdr, P.bins);
         else         k_place_runs<<<blocks, kTT, 0, st>>>(P.local_bins, P.runs, P.seg_count, P.tile_offset, P.hdr, P.bins);
     }
     RouteJob none = {};
-    if (d_counts)  launch_raycast<true, false>(g, tg, P, recs, ordinals_in_records, reinterpret_cast<unsigned int*>(d_counts), d_counters, 1, none, st);
-    else if (maps) launch_raycast<false, false, true>(g, tg, P, recs, ordinals_in_records, P.stamps, d_counters, 1, none, st);
-    else           launch_raycast<false, false>(g, tg, P, recs, ordinals_in_records, P.stamps, d_counters, 1, none, st);
-    if (!d_counts) {
+    unsigned int* const plane = kind == Output::kCounts ? reinterpret_cast<unsigned int*>(d_out) : P.stamps;
+    if (kind == Output::kCounts) launch_raycast<true, false>(g, tg, P, recs, ordinals_in_records, plane, d_counters, 1, none, st);
+    else if (maps)               launch_raycast<false, false, true>(g, tg, P, recs, ordinals_in_records, plane, d_counters, 1, none, st);
+    else                         launch_raycast<false, false>(g, tg, P, recs, ordinals_in_records, plane, d_counters, 1, none, st);
+    if (kind != Output::kCounts) {
         ProfileScope ps(K_TILE_RESOLVE, st);
-        if (maps) k_home_resolve<true><<<device_sm_count() * 8, kTT, 0, st>>>(g, tg, P.active, P.hdr, P.stamps, d_grid);
-        else      k_home_resolve<false><<<device_sm_count() * 8, kTT, 0, st>>>(g, tg, P.active, P.hdr, P.stamps, d_grid);
+        const auto resolve = maps ? k_home_resolve<true> : k_home_resolve<false>;
+        resolve<<<device_sm_count() * 8, kTT, 0, st>>>(g, tg, P.active, P.hdr, P.stamps, reinterpret_cast<int8_t*>(d_out));
     }
     OCC_CUDA_TRY(cudaGetLastError());
     return OCCGRID_OK;
@@ -1468,10 +1373,9 @@ int tiled_raycast_route(const occgrid_geom* geom, const PoseRec* d_recs, int hav
         // nothing prepared (first step of a stream): the header still has to carry a clean queue
         OCC_CUDA_TRY(cudaMemsetAsync(P.hdr, 0, sizeof(TilePlanHeader), st));
     }
-    static const bool force_route_variant = getenv("OCC_ROUTE_VARIANT_ALWAYS") != nullptr;      // diagnostic: template overhead alone
-    if (job) launch_raycast<false, true>(g, tg, P, d_recs, 1, P.stamps, d_counters, have_items, *job, st);
-    else if (force_route_variant) { RouteJob none = {}; launch_raycast<false, true>(g, tg, P, d_recs, 1, P.stamps, d_counters, have_items, none, st); }
-    else {
+    if (job) {
+        launch_raycast<false, true>(g, tg, P, d_recs, 1, P.stamps, d_counters, have_items, *job, st);
+    } else {
         RouteJob none = {};
         launch_raycast<false, false>(g, tg, P, d_recs, 1, P.stamps, d_counters, have_items, none, st);
     }
@@ -1482,37 +1386,6 @@ int tiled_raycast_route(const occgrid_geom* geom, const PoseRec* d_recs, int hav
     }
     OCC_CUDA_TRY(cudaGetLastError());
     return OCCGRID_OK;
-}
-
-int integrate_packets_tiled(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride,
-                            const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
-                            int n_agents, int8_t* d_grid, void* d_ws, size_t ws_bytes, uint64_t* d_counters,
-                            cudaStream_t st) {
-    return integrate_tiled(geom, d_packets, nullptr, 0, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents, d_grid, nullptr, d_ws,
-                           ws_bytes, d_counters, st);
-}
-
-int integrate_packets_tiled_agent_maps(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride,
-                                       const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
-                                       int n_agents, int8_t* d_grids, void* d_ws, size_t ws_bytes, uint64_t* d_counters,
-                                       cudaStream_t st) {
-    return integrate_tiled(geom, d_packets, nullptr, 0, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents, d_grids, nullptr, d_ws,
-                           ws_bytes, d_counters, st, true);
-}
-
-int accumulate_packets_tiled(const occgrid_geom* geom, const uint8_t* d_packets, int64_t n, int stride,
-                             const int32_t* d_agent_idx, const double* d_drift, const double* d_agent_off,
-                             int n_agents, int32_t* d_counts, void* d_ws, size_t ws_bytes, uint64_t* d_counters,
-                             cudaStream_t st) {
-    return integrate_tiled(geom, d_packets, nullptr, 0, n, stride, d_agent_idx, d_drift, d_agent_off, n_agents, nullptr, d_counts, d_ws,
-                           ws_bytes, d_counters, st);
-}
-
-int integrate_poses_tiled(const occgrid_geom* geom, const void* d_poses, int64_t n, int ordinals_in_records, int8_t* d_grid,
-                          void* d_ws, size_t ws_bytes, uint64_t* d_counters, cudaStream_t st) {
-    return integrate_tiled(geom, nullptr, reinterpret_cast<const PoseRec*>(d_poses), ordinals_in_records, n, 0, nullptr, nullptr,
-                           nullptr, 0,
-                           d_grid, nullptr, d_ws, ws_bytes, d_counters, st);
 }
 
 }  // namespace occ

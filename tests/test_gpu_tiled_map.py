@@ -115,6 +115,32 @@ def test_fused_swarm_map_full_size_config2():
     assert cn['owned_updates'] == c['updates'] and cn['beams'] == c['beams'] == 4 * n
 
 
+def test_routed_poses_full_size_config2_tiled():
+    """update_poses under TILED on the whole BASELINE config 2 batch (2.5e6 packets into 4096^2),
+    routed to one band: the pose-record count and scatter passes walk 1 221 chunks of 2 048 records,
+    more than their 8 CTAs per SM take in one pass, and the map equals the C oracle."""
+    if not torch.cuda.is_available():
+        pytest.skip('no CUDA device')
+    from occgrid_b200 import simulation_tools as st
+    from occgrid_b200.distributed import BandLayout, CudaBandOps
+    from oracle import c_oracle
+    size, origin, n = 4096, (-102.4, -102.4), 2_500_000
+    sess = st.generate_session(n_agents=64, n_packets=n, grid_size=size, origin=origin, seed=42)
+    ops = CudaBandOps(BandLayout(size, 1), 0, size, 0.05, origin[0], origin[1], 'cuda', 'tiled', n)
+    pk = ops.stage(sess['packets'])
+    idx = torch.from_numpy(sess['agent_idx'].copy()).cuda()
+    send, counts = ops.route(pk, idx, None, torch.from_numpy(sess['agent_offsets']).cuda())
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    assert 8 * sms * 2048 < counts[0] <= n                # some persistent CTAs take a second chunk
+    ops.integrate(send)
+    got = ops.band_tensor().cpu().numpy()
+    want = np.full((size, size), -1, np.int8)
+    c = c_oracle.integrate_packets(sess['packets'], want, origin[0], origin[1], 0.05, agent_offsets=sess['agent_offsets'],
+                                   agent_idx=sess['agent_idx'])
+    assert np.array_equal(got, want)
+    assert ops.grid.counters()['owned_updates'] == c['updates']
+
+
 def _emulated_band_steps(world, size, origin, max_batch):
     """`world` logical ranks on ONE GPU: plain receive buffers linked by pointer (peer-mapped over
     NVLink in production), publish without the wait (the steps are issued one rank after another on
