@@ -14,7 +14,7 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, 'csrc')
 LIB_PATH = os.path.join(PKG_DIR, 'liboccgrid_b200.so')
 SOURCES = ['occgrid_integrate.cu', 'occgrid_tiled.cu', 'occgrid_route.cu', 'occgrid_band.cu', 'mapmerge.cu', 'frontier.cu', 'icp.cu', 'render.cu', 'slam_chain.cpp']
-HEADERS = ['common.cuh', 'beam_expand.cuh', 'sincos_dd.cuh', os.path.join('..', '..', 'include', 'occgrid_b200.h')]
+HEADERS = ['common.cuh', 'beam_expand.cuh', 'block_ops.cuh', 'sincos_dd.cuh', os.path.join('..', '..', 'include', 'occgrid_b200.h')]
 
 STRATEGY = {'auto': -1, 'global_atomic': 0, 'tiled': 1}
 COUNTER_NAMES = ('packets', 'accepted', 'dropped', 'bad_pose', 'beams', 'hits', 'updates', 'slowpath',

@@ -7,6 +7,7 @@
 
 #include "../../include/occgrid_b200.h"
 #include "beam_expand.cuh"
+#include "block_ops.cuh"
 
 namespace occ {
 

@@ -68,27 +68,6 @@ __device__ __forceinline__ unsigned int frontier_mask16(const int8_t* __restrict
     return mask;
 }
 
-__device__ __forceinline__ unsigned int block_scan_excl(unsigned int v, unsigned int* s_warp /* 33 */, unsigned int* total) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    unsigned int inc = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { unsigned int t = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += t; }
-    if (lane == 31) s_warp[warp] = inc;
-    __syncthreads();
-    if (warp == 0) {
-        unsigned int wv = (lane < (int)(blockDim.x >> 5)) ? s_warp[lane] : 0u, winc = wv;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { unsigned int t = __shfl_up_sync(0xffffffffu, winc, o); if (lane >= o) winc += t; }
-        s_warp[lane] = winc - wv;
-        if (lane == 31) s_warp[32] = winc;
-    }
-    __syncthreads();
-    const unsigned int r = s_warp[warp] + inc - v;
-    *total = s_warp[32];
-    __syncthreads();
-    return r;
-}
-
 // The grid is read ONCE: the count pass keeps the 16 frontier bits of every thread's cells, the
 // write pass expands those bits into (x, y) tuples without touching the grid again.
 __global__ void __launch_bounds__(kFT)
@@ -100,7 +79,7 @@ k_frontier_count(const int8_t* __restrict__ g, int w, int h, unsigned int* __res
     const unsigned int m = base < n ? frontier_mask16(g, w, h, base, n) : 0u;
     masks[(size_t)blockIdx.x * kFT + threadIdx.x] = (unsigned short)m;
     unsigned int total;
-    block_scan_excl(__popc(m), s_warp, &total);
+    block_exclusive_scan(__popc(m), s_warp, &total);
     if (threadIdx.x == 0) block_counts[blockIdx.x] = total;
 }
 
@@ -111,28 +90,9 @@ constexpr int kReserveItems = 16;
 __global__ void __launch_bounds__(1024)
 k_frontier_reserve(unsigned int* __restrict__ block_counts, int n_blocks, long long capacity,
                    long long* __restrict__ d_count, int* __restrict__ status) {
-    __shared__ unsigned int s_warp[33];
-    __shared__ unsigned int s_carry;
-    if (threadIdx.x == 0) s_carry = 0;
-    __syncthreads();
-    for (int start = 0; start < n_blocks; start += 1024 * kReserveItems) {
-        const int i0 = start + (int)threadIdx.x * kReserveItems;
-        unsigned int v[kReserveItems], sum = 0;
-#pragma unroll
-        for (int j = 0; j < kReserveItems; ++j) { v[j] = (i0 + j < n_blocks) ? block_counts[i0 + j] : 0u; sum += v[j]; }
-        unsigned int total;
-        unsigned int run = s_carry + block_scan_excl(sum, s_warp, &total);
-#pragma unroll
-        for (int j = 0; j < kReserveItems; ++j) {
-            if (i0 + j < n_blocks) block_counts[i0 + j] = run;
-            run += v[j];
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) s_carry += total;
-        __syncthreads();
-    }
+    const unsigned long long sum = cta_scan_in_place<kReserveItems>(block_counts, n_blocks, 0ull);
     if (threadIdx.x == 0) {
-        long long total = s_carry;
+        long long total = (long long)sum;
         if (total > capacity) { atomicOr(status, 1); total = 0; }
         *d_count = total;
     }
@@ -146,7 +106,7 @@ k_frontier_write(const unsigned short* __restrict__ masks, int w, int h, const u
     const long long base = ((long long)blockIdx.x * kFT + threadIdx.x) * kFCells;
     unsigned int m = masks[(size_t)blockIdx.x * kFT + threadIdx.x];
     unsigned int total;
-    long long dst = block_offsets[blockIdx.x] + block_scan_excl(__popc(m), s_warp, &total);
+    long long dst = block_offsets[blockIdx.x] + block_exclusive_scan(__popc(m), s_warp, &total);
     while (m) {
         const int i = __ffs(m) - 1;
         m &= m - 1;
@@ -252,7 +212,7 @@ k_cluster_emit(const long long* __restrict__ d_count, const int* __restrict__ la
             if (i < n && label[i] == (int)i && csize[i] >= (unsigned int)min_cluster) keep |= 1u << j;              // :228
         }
         unsigned int total;
-        unsigned int pos = s_carry + block_scan_excl(__popc(keep), s_warp, &total);
+        unsigned int pos = s_carry + block_exclusive_scan(__popc(keep), s_warp, &total);
         while (keep) {
             const long long i = i0 + (__ffs(keep) - 1);
             keep &= keep - 1;

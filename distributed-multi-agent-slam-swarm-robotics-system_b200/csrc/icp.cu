@@ -57,33 +57,12 @@ k_icp_count(const double* __restrict__ tx, const double* __restrict__ ty, long l
         atomicAdd(&cnt[(size_t)icp_cell_of(ty[i], min_y, cell, h) * w + icp_cell_of(tx[i], min_x, cell, w)], 1u);
 }
 
-// One CTA: start[c] = exclusive sum of cnt; cursor[c] = start[c] (consumed by the fill pass).
+// start[c] = exclusive sum of cnt; cursor[c] = start[c] (consumed by the fill pass).
 // Exclusive scan of the per-cell counts in three launches (block sums -> scan of the block sums ->
 // rescan with the carry): every block of 16 384 cells runs on its own CTA, so the index of a
 // 640 k-cell map is built in tens of microseconds instead of one CTA looping for a millisecond.
 constexpr int kScanItemsIcp = 16;
 constexpr int kScanBlockIcp = 1024 * kScanItemsIcp;
-
-__device__ __forceinline__ unsigned int icp_block_scan(unsigned int sum, unsigned int* s_warp /* 33 */, unsigned int* total) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    unsigned int inc = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { const unsigned int t = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += t; }
-    if (lane == 31) s_warp[warp] = inc;
-    __syncthreads();
-    if (warp == 0) {
-        unsigned int wv = s_warp[lane], winc = wv;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const unsigned int t = __shfl_up_sync(0xffffffffu, winc, o); if (lane >= o) winc += t; }
-        s_warp[lane] = winc - wv;
-        if (lane == 31) s_warp[32] = winc;
-    }
-    __syncthreads();
-    const unsigned int ex = s_warp[warp] + inc - sum;
-    *total = s_warp[32];
-    __syncthreads();
-    return ex;
-}
 
 __global__ void __launch_bounds__(1024)
 k_icp_scan_sums(const unsigned int* __restrict__ cnt, long long cells, unsigned int* __restrict__ block_sums) {
@@ -93,27 +72,14 @@ k_icp_scan_sums(const unsigned int* __restrict__ cnt, long long cells, unsigned 
 #pragma unroll
     for (int j = 0; j < kScanItemsIcp; ++j) sum += (i0 + j < cells) ? cnt[i0 + j] : 0u;
     unsigned int total;
-    icp_block_scan(sum, s_warp, &total);
+    block_exclusive_scan(sum, s_warp, &total);
     if (threadIdx.x == 0) block_sums[blockIdx.x] = total;
 }
 
 __global__ void __launch_bounds__(1024)
 k_icp_scan_top(unsigned int* __restrict__ block_sums, int n_blocks, unsigned int* __restrict__ start, long long cells) {
-    __shared__ unsigned int s_warp[33];
-    __shared__ unsigned int s_carry;
-    if (threadIdx.x == 0) s_carry = 0;
-    __syncthreads();
-    for (int base = 0; base < n_blocks; base += 1024) {
-        const int i = base + threadIdx.x;
-        const unsigned int v = i < n_blocks ? block_sums[i] : 0u;
-        unsigned int total;
-        const unsigned int ex = icp_block_scan(v, s_warp, &total);
-        if (i < n_blocks) block_sums[i] = s_carry + ex;
-        __syncthreads();
-        if (threadIdx.x == 0) s_carry += total;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) start[cells] = s_carry;
+    const unsigned long long total = cta_scan_in_place<1>(block_sums, n_blocks, 0ull);
+    if (threadIdx.x == 0) start[cells] = (unsigned int)total;
 }
 
 __global__ void __launch_bounds__(1024)
@@ -125,7 +91,7 @@ k_icp_scan_apply(const unsigned int* __restrict__ cnt, long long cells, const un
 #pragma unroll
     for (int j = 0; j < kScanItemsIcp; ++j) { v[j] = (i0 + j < cells) ? cnt[i0 + j] : 0u; sum += v[j]; }
     unsigned int total;
-    unsigned int run = block_sums[blockIdx.x] + icp_block_scan(sum, s_warp, &total);
+    unsigned int run = block_sums[blockIdx.x] + block_exclusive_scan(sum, s_warp, &total);
 #pragma unroll
     for (int j = 0; j < kScanItemsIcp; ++j) {
         if (i0 + j < cells) { start[i0 + j] = run; cursor[i0 + j] = run; }
@@ -221,43 +187,8 @@ struct IcpLoop {
     double* partial2;                              // [n_vb][2] = {sum dot, sum cross} of the demeaned pairs
     int n_vb, max_iteration;
     IcpState* state;
-    unsigned int* bar;                             // [0] arrivals (monotonic), [1] abort flag
+    unsigned int* bar;                             // [0, 4) grid_barrier words, [4] abort flag; zeroed before each launch
 };
-
-constexpr unsigned long long kIcpBarrierTimeoutNs = 2000000000ull;
-
-__device__ __forceinline__ unsigned long long icp_global_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-
-// Cooperative launch keeps every CTA resident; the time-out only turns a would-be hang (a lost
-// CTA) into an error the host can report.
-__device__ __forceinline__ bool icp_grid_barrier(unsigned int* bar, unsigned int& target) {
-    __shared__ int s_ok;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        target += gridDim.x;
-        int ok = 1;
-        __threadfence();
-        atomicAdd(bar, 1u);
-        const unsigned long long t0 = icp_global_ns();
-        unsigned int spins = 0;
-        while (*reinterpret_cast<volatile unsigned int*>(bar) < target) {
-            if (((++spins) & 1023u) == 0u &&
-                (reinterpret_cast<volatile unsigned int*>(bar)[1] || icp_global_ns() - t0 > kIcpBarrierTimeoutNs)) {
-                atomicExch(bar + 1, 1u);
-                ok = 0;
-                break;
-            }
-        }
-        __threadfence();
-        s_ok = ok;
-    }
-    __syncthreads();
-    return s_ok != 0;
-}
 
 // Folds the association partials in a fixed order, scores the registration and decides whether
 // the loop has converged (Registration.cpp: |d fitness| < rel_f && |d rmse| < rel_r).
@@ -354,7 +285,9 @@ __device__ __forceinline__ void icp_cov_phase(const IcpLoop& p, const IcpState* 
     }
 }
 
-__global__ void __launch_bounds__(kIT)
+// Three CTAs per SM: without the bound ptxas may cut the kernel to 64 registers and spill in the
+// neighbour search.
+__global__ void __launch_bounds__(kIT, 3)
 k_icp_loop(const IcpLoop p) {
     __shared__ IcpState L;
     if (threadIdx.x == 0) {
@@ -365,16 +298,17 @@ k_icp_loop(const IcpLoop p) {
     }
     __syncthreads();
     unsigned int target = 0;
+    int* abort_flag = reinterpret_cast<int*>(p.bar + 4);
     bool alive = true;
     icp_assoc_phase(p, &L, false);
-    alive = icp_grid_barrier(p.bar, target);
+    alive = grid_barrier(p.bar, target, abort_flag);
     if (alive) icp_fold_eval(p, &L, 1);
     for (int it = 0; alive && it < p.max_iteration && !L.done; ++it) {
         icp_cov_phase(p, &L);
-        if (!(alive = icp_grid_barrier(p.bar, target))) break;
+        if (!(alive = grid_barrier(p.bar, target, abort_flag))) break;
         icp_fold_solve(p, &L);
         icp_assoc_phase(p, &L, true);
-        if (!(alive = icp_grid_barrier(p.bar, target))) break;
+        if (!(alive = grid_barrier(p.bar, target, abort_flag))) break;
         icp_fold_eval(p, &L, 0);
     }
     if (blockIdx.x == 0 && threadIdx.x == 0) {

@@ -31,66 +31,6 @@ enum { ST_POINT_OVERFLOW = 1, ST_LATTICE_OVERFLOW = 2, ST_CHAIN_ABORTED = 4 };
 
 struct Xform { double m[16]; int identity; };
 
-// ---- block-level exclusive scan of one unsigned value per thread --------------------------
-__device__ __forceinline__ unsigned int block_exclusive_scan(unsigned int v, unsigned int* s_warp /* >= 32 */,
-                                                             unsigned int* total) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    unsigned int inc = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        unsigned int t = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += t;
-    }
-    if (lane == 31) s_warp[warp] = inc;
-    __syncthreads();
-    if (warp == 0) {
-        unsigned int w = (lane < (int)(blockDim.x >> 5)) ? s_warp[lane] : 0u;
-        unsigned int winc = w;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            unsigned int t = __shfl_up_sync(0xffffffffu, winc, o);
-            if (lane >= o) winc += t;
-        }
-        s_warp[lane] = winc - w;          // exclusive warp offsets
-        if (lane == 31) s_warp[32] = winc;   // block total
-    }
-    __syncthreads();
-    unsigned int res = s_warp[warp] + inc - v;
-    *total = s_warp[32];
-    __syncthreads();
-    return res;
-}
-
-// Same for 64-bit values (sums of per-agent point counts).  s_warp64 >= 33 entries.
-__device__ __forceinline__ unsigned long long block_exclusive_scan64(unsigned long long v, unsigned long long* s_warp64,
-                                                                     unsigned long long* total) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    unsigned long long inc = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        unsigned long long t = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += t;
-    }
-    if (lane == 31) s_warp64[warp] = inc;
-    __syncthreads();
-    if (warp == 0) {
-        unsigned long long w = (lane < (int)(blockDim.x >> 5)) ? s_warp64[lane] : 0ull;
-        unsigned long long winc = w;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            unsigned long long t = __shfl_up_sync(0xffffffffu, winc, o);
-            if (lane >= o) winc += t;
-        }
-        s_warp64[lane] = winc - w;
-        if (lane == 31) s_warp64[32] = winc;
-    }
-    __syncthreads();
-    const unsigned long long res = s_warp64[warp] + inc - v;
-    *total = s_warp64[32];
-    __syncthreads();
-    return res;
-}
-
 // ---- a10: occupied-cell extraction (data > 50, map_merger.py:72) --------------------------
 
 __device__ __forceinline__ unsigned int occupied_mask16(const int8_t* __restrict__ grid, long long base, long long n) {
@@ -147,23 +87,10 @@ __global__ void __launch_bounds__(1024)
 k_extract_reserve(unsigned int* __restrict__ block_counts, int n_blocks, long long* __restrict__ d_count,
                   long long capacity, long long* __restrict__ ws_base, int* __restrict__ status,
                   long long* __restrict__ d_last_appended) {
-    __shared__ unsigned int s_warp[33];
-    __shared__ unsigned int s_carry;
-    if (threadIdx.x == 0) s_carry = 0;
-    __syncthreads();
-    for (int start = 0; start < n_blocks; start += blockDim.x) {
-        const int i = start + threadIdx.x;
-        const unsigned int v = i < n_blocks ? block_counts[i] : 0u;
-        unsigned int total;
-        const unsigned int ex = block_exclusive_scan(v, s_warp, &total);
-        if (i < n_blocks) block_counts[i] = s_carry + ex;
-        __syncthreads();
-        if (threadIdx.x == 0) s_carry += total;
-        __syncthreads();
-    }
+    const unsigned long long sum = cta_scan_in_place<1>(block_counts, n_blocks, 0ull);
     if (threadIdx.x == 0) {
         const long long base = *d_count;
-        long long total = s_carry;
+        long long total = (long long)sum;
         if (base + total > capacity) { atomicOr(status, ST_POINT_OVERFLOW); total = 0; }
         ws_base[0] = base;
         ws_base[1] = total;
@@ -205,8 +132,35 @@ k_extract_write(const int8_t* __restrict__ grid, long long n_cells, int width, d
     }
 }
 
-__device__ __forceinline__ double warp_min(double v);
-__device__ __forceinline__ double warp_max(double v);
+// ---- block-level min/max of (x, y) -----------------------------------------------------------
+__device__ __forceinline__ double warp_min(double v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = fmin(v, __shfl_xor_sync(0xffffffffu, v, o));
+    return v;
+}
+__device__ __forceinline__ double warp_max(double v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
+    return v;
+}
+
+// Every thread calls with its own values; thread 0 then calls use(min x, min y, max x, max y) of
+// the whole block (any block size up to 1024).  Warps fold in a fixed fmin / fmax order, so the
+// bounds do not depend on timing, down to the sign of zero.
+template <class F>
+__device__ __forceinline__ void block_min_max(double mnx, double mny, double mxx, double mxy, F&& use) {
+    __shared__ double s_b[4][32];
+    mnx = warp_min(mnx); mny = warp_min(mny); mxx = warp_max(mxx); mxy = warp_max(mxy);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (lane == 0) { s_b[0][warp] = mnx; s_b[1][warp] = mny; s_b[2][warp] = mxx; s_b[3][warp] = mxy; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int w = 1; w < (int)(blockDim.x >> 5); ++w) {
+            mnx = fmin(mnx, s_b[0][w]); mny = fmin(mny, s_b[1][w]); mxx = fmax(mxx, s_b[2][w]); mxy = fmax(mxy, s_b[3][w]);
+        }
+        use(mnx, mny, mxx, mxy);
+    }
+}
 
 // ---- bounds carried on the device between callbacks ----------------------------------------
 // doubles mapped to uint64 keys that sort like the doubles, so min/max become integer atomics;
@@ -223,20 +177,12 @@ __device__ __forceinline__ double dec_double(unsigned long long k) {
 // Block-level min/max of (x, y) over the calling threads' values, then 4 atomics per CTA.
 __device__ __forceinline__ void block_bounds_atomic(double mnx, double mny, double mxx, double mxy,
                                                     unsigned long long* __restrict__ benc) {
-    __shared__ double s_b[4][32];                  // any block size up to 1024
-    mnx = warp_min(mnx); mny = warp_min(mny); mxx = warp_max(mxx); mxy = warp_max(mxy);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (lane == 0) { s_b[0][warp] = mnx; s_b[1][warp] = mny; s_b[2][warp] = mxx; s_b[3][warp] = mxy; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        for (int w = 1; w < (int)(blockDim.x >> 5); ++w) {
-            mnx = fmin(mnx, s_b[0][w]); mny = fmin(mny, s_b[1][w]); mxx = fmax(mxx, s_b[2][w]); mxy = fmax(mxy, s_b[3][w]);
+    block_min_max(mnx, mny, mxx, mxy, [&](double x0, double y0, double x1, double y1) {
+        if (x0 <= x1) {
+            atomicMin(&benc[0], enc_double(x0)); atomicMin(&benc[1], enc_double(y0));
+            atomicMax(&benc[2], enc_double(x1)); atomicMax(&benc[3], enc_double(y1));
         }
-        if (mnx <= mxx) {
-            atomicMin(&benc[0], enc_double(mnx)); atomicMin(&benc[1], enc_double(mny));
-            atomicMax(&benc[2], enc_double(mxx)); atomicMax(&benc[3], enc_double(mxy));
-        }
-    }
+    });
 }
 
 __global__ void k_benc_reset(unsigned long long* __restrict__ benc) {
@@ -366,22 +312,8 @@ k_batch_count_tma(const int8_t* const* __restrict__ grids, long long n_cells, in
 // One CTA per agent: exclusive scan of its block counts (in place) and its total.
 __global__ void __launch_bounds__(1024)
 k_batch_scan(unsigned int* __restrict__ block_counts, int blocks_per_grid, long long* __restrict__ agent_total) {
-    __shared__ unsigned int s_warp[33];
-    __shared__ unsigned int s_carry;
-    unsigned int* bc = block_counts + (size_t)blockIdx.x * blocks_per_grid;
-    if (threadIdx.x == 0) s_carry = 0;
-    __syncthreads();
-    for (int start = 0; start < blocks_per_grid; start += blockDim.x) {
-        const int i = start + threadIdx.x;
-        const unsigned int v = i < blocks_per_grid ? bc[i] : 0u;
-        unsigned int total;
-        const unsigned int ex = block_exclusive_scan(v, s_warp, &total);
-        if (i < blocks_per_grid) bc[i] = s_carry + ex;
-        __syncthreads();
-        if (threadIdx.x == 0) s_carry += total;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) agent_total[blockIdx.x] = s_carry;
+    const unsigned long long total = cta_scan_in_place<1>(block_counts + (size_t)blockIdx.x * blocks_per_grid, blocks_per_grid, 0ull);
+    if (threadIdx.x == 0) agent_total[blockIdx.x] = (long long)total;
 }
 
 // agent_offset[a] = sum of totals of the agents before a that take part in the merge (one CTA).
@@ -396,7 +328,7 @@ k_batch_offsets(const long long* __restrict__ agent_total, const BatchXform* __r
         const int a = start + threadIdx.x;
         const unsigned long long v = (a < n_agents && T[a].use) ? (unsigned long long)agent_total[a] : 0ull;
         unsigned long long total;
-        const unsigned long long ex = block_exclusive_scan64(v, s_warp, &total);
+        const unsigned long long ex = block_exclusive_scan(v, s_warp, &total);
         if (a < n_agents) agent_offset[a] = s_carry + (long long)ex;
         __syncthreads();
         if (threadIdx.x == 0) s_carry += (long long)total;
@@ -476,21 +408,9 @@ __global__ void k_bump_count(const long long* __restrict__ agent_offset, int a, 
 
 // ---- bounds (GetMinBound/GetMaxBound; publish_global_map :95-98) ---------------------------
 
-__device__ __forceinline__ double warp_min(double v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmin(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
-__device__ __forceinline__ double warp_max(double v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
-
 __global__ void __launch_bounds__(kMT)
 k_bounds_partial(const double* __restrict__ px, const double* __restrict__ py, const long long* __restrict__ d_count,
                  double* __restrict__ partial /* gridDim.x * 4 */) {
-    __shared__ double s[4][kMT / 32];
     const long long n = *d_count;
     double mnx = INFINITY, mny = INFINITY, mxx = -INFINITY, mxy = -INFINITY;
     for (long long i = (long long)blockIdx.x * kMT + threadIdx.x; i < n; i += (long long)gridDim.x * kMT) {
@@ -498,37 +418,22 @@ k_bounds_partial(const double* __restrict__ px, const double* __restrict__ py, c
         mnx = fmin(mnx, x); mxx = fmax(mxx, x);
         mny = fmin(mny, y); mxy = fmax(mxy, y);
     }
-    mnx = warp_min(mnx); mny = warp_min(mny); mxx = warp_max(mxx); mxy = warp_max(mxy);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (lane == 0) { s[0][warp] = mnx; s[1][warp] = mny; s[2][warp] = mxx; s[3][warp] = mxy; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        for (int w = 1; w < kMT / 32; ++w) {
-            mnx = fmin(mnx, s[0][w]); mny = fmin(mny, s[1][w]); mxx = fmax(mxx, s[2][w]); mxy = fmax(mxy, s[3][w]);
-        }
-        partial[blockIdx.x * 4 + 0] = mnx; partial[blockIdx.x * 4 + 1] = mny;
-        partial[blockIdx.x * 4 + 2] = mxx; partial[blockIdx.x * 4 + 3] = mxy;
-    }
+    block_min_max(mnx, mny, mxx, mxy, [&](double x0, double y0, double x1, double y1) {
+        partial[blockIdx.x * 4 + 0] = x0; partial[blockIdx.x * 4 + 1] = y0;
+        partial[blockIdx.x * 4 + 2] = x1; partial[blockIdx.x * 4 + 3] = y1;
+    });
 }
 
 __global__ void __launch_bounds__(kMT)
 k_bounds_final(const double* __restrict__ partial, int n_partial, double* __restrict__ bounds) {
-    __shared__ double s[4][kMT / 32];
     double mnx = INFINITY, mny = INFINITY, mxx = -INFINITY, mxy = -INFINITY;
     for (int i = threadIdx.x; i < n_partial; i += kMT) {
         mnx = fmin(mnx, partial[i * 4 + 0]); mny = fmin(mny, partial[i * 4 + 1]);
         mxx = fmax(mxx, partial[i * 4 + 2]); mxy = fmax(mxy, partial[i * 4 + 3]);
     }
-    mnx = warp_min(mnx); mny = warp_min(mny); mxx = warp_max(mxx); mxy = warp_max(mxy);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (lane == 0) { s[0][warp] = mnx; s[1][warp] = mny; s[2][warp] = mxx; s[3][warp] = mxy; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        for (int w = 1; w < kMT / 32; ++w) {
-            mnx = fmin(mnx, s[0][w]); mny = fmin(mny, s[1][w]); mxx = fmax(mxx, s[2][w]); mxy = fmax(mxy, s[3][w]);
-        }
-        bounds[0] = mnx; bounds[1] = mny; bounds[2] = mxx; bounds[3] = mxy;
-    }
+    block_min_max(mnx, mny, mxx, mxy, [&](double x0, double y0, double x1, double y1) {
+        bounds[0] = x0; bounds[1] = y0; bounds[2] = x1; bounds[3] = y1;
+    });
 }
 
 // ---- a11: VoxelDownSample -------------------------------------------------------------------
@@ -870,59 +775,6 @@ struct ChainRun {
     unsigned int* bar;                                         // {arrivals, exits, release, verdict}; all zero between launches
     int bc_stride;
 };
-
-// Grid-wide barrier over co-resident CTAs (cooperative launch).  bar[0] counts arrivals, bar[2] is
-// the release word, bar[3] the verdict the LAST arriver computed (`last_arriver()` runs in exactly
-// one thread of the grid, after every CTA's pre-barrier writes are visible and before anybody is
-// released) — a decision every CTA must agree on is therefore single-sourced: nobody re-derives it
-// from header fields a faster CTA may already be overwriting in the next phase.
-// A CTA that waits longer than kBarrierTimeoutNs gives up (returns false, sets *abort_flag): a
-// missing CTA can then no longer hang the device.
-constexpr unsigned long long kBarrierTimeoutNs = 2000000000ull;
-
-__device__ __forceinline__ unsigned long long global_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-
-template <class F>
-__device__ __forceinline__ bool grid_barrier(unsigned int* bar, unsigned int& target, int* abort_flag, int* verdict, F&& last_arriver) {
-    __shared__ int s_ok, s_verdict;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        target += gridDim.x;
-        int ok = 1;
-        __threadfence();
-        if (atomicAdd(bar, 1u) == target - 1u) {               // last arriver: decide, publish, release
-            __threadfence();
-            reinterpret_cast<volatile unsigned int*>(bar)[3] = (unsigned int)last_arriver();
-            __threadfence();
-            reinterpret_cast<volatile unsigned int*>(bar)[2] = target;
-        } else {
-            const unsigned long long t0 = global_ns();
-            unsigned int spins = 0;
-            while (reinterpret_cast<volatile unsigned int*>(bar)[2] < target) {
-                if (((++spins) & 1023u) == 0u &&
-                    (*reinterpret_cast<volatile int*>(abort_flag) || global_ns() - t0 > kBarrierTimeoutNs)) {
-                    atomicExch(abort_flag, 1);
-                    ok = 0;
-                    break;
-                }
-            }
-        }
-        __threadfence();
-        s_ok = ok;
-        s_verdict = (int)reinterpret_cast<volatile unsigned int*>(bar)[3];
-    }
-    __syncthreads();
-    if (verdict) *verdict = s_verdict;
-    return s_ok != 0;
-}
-
-__device__ __forceinline__ bool grid_barrier(unsigned int* bar, unsigned int& target, int* abort_flag) {
-    return grid_barrier(bar, target, abort_flag, nullptr, [] { return 0; });
-}
 
 __device__ __forceinline__ void chain_link(const ChainRun& p, long long b, long long n, double mbx, double mby) {
     for (long long j = (long long)blockIdx.x * kMT + threadIdx.x; j < n; j += (long long)gridDim.x * kMT) {

@@ -24,12 +24,6 @@ namespace occ {
 
 constexpr unsigned long long kBandBarrierTimeoutNs = 10000000000ull;      // 10 s: a peer died; give up instead of hanging
 
-__device__ __forceinline__ unsigned long long band_global_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-
 __device__ __forceinline__ void st_release_sys(unsigned int* p, unsigned int v) {
     asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
@@ -55,10 +49,10 @@ __global__ void k_band_publish(int n_bands, int rank, unsigned int* __restrict__
     __threadfence_system();
     st_release_sys(peer_flags[b] + rank, epoch);
     if (!wait) return;
-    const unsigned long long t0 = band_global_ns();
+    const unsigned long long t0 = global_ns();
     unsigned int spins = 0;
     while ((int)(ld_acquire_sys(my_flags + b) - epoch) < 0) {
-        if (((++spins) & 255u) == 0u && band_global_ns() - t0 > kBandBarrierTimeoutNs) { atomicOr(status, 4); return; }
+        if (((++spins) & 255u) == 0u && global_ns() - t0 > kBandBarrierTimeoutNs) { atomicOr(status, 4); return; }
     }
 }
 

@@ -89,42 +89,13 @@ k_route_count(RouteParams P, const uint8_t* __restrict__ pkts, long long n, int 
 __global__ void __launch_bounds__(1024)
 k_route_scan(unsigned int* __restrict__ hist, int n_bands, int n_blocks, long long* __restrict__ band_counts,
              long long capacity, int* __restrict__ status) {
-    __shared__ unsigned int s_warp[33];
-    __shared__ unsigned long long s_carry;
-    __shared__ unsigned long long s_band_start;
-    if (threadIdx.x == 0) s_carry = 0;
-    __syncthreads();
-    for (int b = 0; b < n_bands; ++b) {
-        if (threadIdx.x == 0) s_band_start = s_carry;
-        __syncthreads();
-        for (int start = 0; start < n_blocks; start += blockDim.x) {
-            const int i = start + threadIdx.x;
-            const unsigned int v = i < n_blocks ? hist[(size_t)b * n_blocks + i] : 0u;
-            // block-wide exclusive scan
-            const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-            unsigned int inc = v;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) { unsigned int t = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += t; }
-            if (lane == 31) s_warp[warp] = inc;
-            __syncthreads();
-            if (warp == 0) {
-                unsigned int w = s_warp[lane], winc = w;
-#pragma unroll
-                for (int o = 1; o < 32; o <<= 1) { unsigned int t = __shfl_up_sync(0xffffffffu, winc, o); if (lane >= o) winc += t; }
-                s_warp[lane] = winc - w;
-                if (lane == 31) s_warp[32] = winc;
-            }
-            __syncthreads();
-            const unsigned long long ex = s_carry + s_warp[warp] + inc - v;
-            if (i < n_blocks) hist[(size_t)b * n_blocks + i] = (unsigned int)ex;   // offsets < 2^32 (checked by host)
-            __syncthreads();
-            if (threadIdx.x == 0) s_carry += s_warp[32];
-            __syncthreads();
-        }
-        if (threadIdx.x == 0) band_counts[b] = (long long)(s_carry - s_band_start);
-        __syncthreads();
+    unsigned long long carry = 0;
+    for (int b = 0; b < n_bands; ++b) {                        // offsets < 2^32 (checked by host)
+        const unsigned long long next = cta_scan_in_place<1>(hist + (size_t)b * n_blocks, n_blocks, carry);
+        if (threadIdx.x == 0) band_counts[b] = (long long)(next - carry);
+        carry = next;
     }
-    if (threadIdx.x == 0 && (long long)s_carry > capacity) atomicOr(status, 1);
+    if (threadIdx.x == 0 && (long long)carry > capacity) atomicOr(status, 1);
 }
 
 __global__ void __launch_bounds__(kRT)

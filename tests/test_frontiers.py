@@ -96,6 +96,23 @@ def test_gpu_frontiers_large_grid_vs_oracle(seed):
 
 
 @pytest.mark.gpu
+def test_gpu_frontiers_more_than_one_reserve_round():
+    """8208^2 cells = 16 449 blocks of 4 096: the single-CTA scan of the block counts (16 per thread
+    and round) takes a second round, whose offsets carry the first round's total."""
+    if not torch.cuda.is_available():
+        pytest.skip('no CUDA device')
+    n = 8208
+    assert (n * n + 4095) // 4096 > 1024 * 16
+    rng = np.random.default_rng(3)
+    arr = np.full((n, n), -1, np.int8)
+    arr[rng.integers(0, n, 40000), rng.integers(0, n, 40000)] = 0
+    g = gpu_grid(arr)
+    fr = g.get_frontiers()
+    want = O.get_frontiers_fast(arr)
+    assert fr == want and sum(y * n + x >= 1024 * 16 * 4096 for x, y in want) > 50
+
+
+@pytest.mark.gpu
 def test_gpu_frontiers_edge_cases():
     if not torch.cuda.is_available():
         pytest.skip('no CUDA device')

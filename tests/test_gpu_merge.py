@@ -241,6 +241,26 @@ def test_2048_grids(MM):
     run_pair(MM, 2048, 4, seed=7, span=50.0, origin=(-51.2, -51.2), check_every=False)
 
 
+def test_grid_of_more_than_1024_scan_blocks(MM):
+    """4160^2 cells = 1 057 blocks of 16 384: the single-CTA scans of the block counts (grid_to_pcd's
+    and the batched merge's) take a second round, whose offsets carry the first round's total."""
+    from oracle import merge_oracle as MO
+    n, res, origin = 4160, 0.05, (-104.0, -104.0)
+    assert (n * n + 16383) // 16384 > 1024
+    g = np.full((n, n), -1, np.int8)
+    g[np.random.default_rng(17).random((n, n)) < 0.003] = 100
+    pts = MM.MapMerger().grid_to_pcd(MM.make_grid_msg(g.ravel(), n, n, res, *origin))
+    ox, oy = MO.grid_to_points(g.ravel(), n, n, res, *origin)
+    assert np.array_equal(pts[:, 0], ox) and np.array_equal(pts[:, 1], oy)
+    o = MO.OracleMerger()
+    want = o.map_callback(g.ravel(), n, n, res, *origin)
+    m = MM.MapMerger()
+    out, org = m.merge(g[None], np.array([origin]), res)
+    assert np.array_equal(out, want[0]) and org == want[1]
+    pc = m.global_pcd
+    assert np.array_equal(pc[:, 0], o.gx) and np.array_equal(pc[:, 1], o.gy)
+
+
 def test_sharded_merger_single_rank_equals_merge(MM):
     """ShardedMapMerger (agent blocks per rank, batched extraction sharded, ordered voxel chain
     replicated) with world = 1 must equal MapMerger.merge and the oracle; an empty first grid

@@ -163,3 +163,31 @@ def test_gpu_registration_of_a_cloud_larger_than_the_resident_grid(MM):
     assert reg.correspondences == round(fw * lx.shape[0]) and reg.fitness == fw and reg.iterations == iw
     assert abs(reg.inlier_rmse - rw) < 1e-9
     assert np.allclose(reg.transformation, Tw, atol=1e-9)
+
+
+@pytest.mark.gpu
+def test_gpu_registration_with_a_cell_index_of_more_than_1024_scan_blocks(MM):
+    """A cluster 1 km below and left of the scene stretches the target's cell index past 1 024
+    blocks of 16 384 cells: the single-CTA scan of the block sums takes a second round, and the
+    scene's cells, all in that round, are found only if their offsets carry the first round's total."""
+    import torch
+    g, x, y = _cloud(256, 3)
+    gx, gy = MO.transform_points(x, y, MO.se2_matrix(0.12, -0.08, 0.03))
+    r = np.random.default_rng(4)
+    gx = np.concatenate([r.uniform(-1040.0, -1030.0, 64), gx])
+    gy = np.concatenate([r.uniform(-1040.0, -1030.0, 64), gy])
+    cell = 1.0 / 4.0                                       # MapMerger.register's index cell for a 1 m threshold
+    cw, ch = int((gx.max() - gx.min()) / cell) + 2, int((gy.max() - gy.min()) / cell) + 2
+    assert (cw * ch + 16383) // 16384 > 1024
+    m = MM.MapMerger(registration='icp')
+    m._ensure_capacity(gx.shape[0] + 16)
+    m._cloud.x[:gx.shape[0]].copy_(torch.from_numpy(gx))
+    m._cloud.y[:gx.shape[0]].copy_(torch.from_numpy(gy))
+    m._cloud.count.fill_(gx.shape[0])
+    m._n_global = gx.shape[0]
+    reg = m.register(MM.make_grid_msg(g.ravel(), 256, 256, 0.05, -6.4, -6.4))
+    Tw, fw, rw, iw = IO.registration_icp(x, y, gx, gy)
+    assert fw > 0.6
+    assert reg.correspondences == round(fw * x.shape[0]) and reg.fitness == fw and reg.iterations == iw
+    assert abs(reg.inlier_rmse - rw) < 1e-9
+    assert np.allclose(reg.transformation, Tw, atol=1e-9)
