@@ -623,7 +623,10 @@ class AgentGrids(OccupancyGrid):
     takes, without a copy.  All maps share one geometry.  ``agent_offsets`` must have n_agents + 1
     rows; the default is zero except row 2 = (separation, 0) (:851-852), so with separation = 0
     every agent maps in its own odometry frame.  Single-map operations (rays, pose records, counts,
-    frontiers, rendering) raise ``OccGridError``.
+    frontiers, rendering) raise ``OccGridError``.  For frontiers on the swarm's map,
+    ``MapMerger().fuse_occupancy(maps.grids_tensor, maps.origins, maps.res, transforms, target)``
+    fuses the stack into an ``OccupancyGrid`` that keeps free space; ``target.frontier_centroids()``
+    then runs there.
     """
 
     def __init__(self, n_agents=2, size=GRID_SIZE, resolution=GRID_RESOLUTION,

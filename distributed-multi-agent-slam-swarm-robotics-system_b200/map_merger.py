@@ -421,6 +421,59 @@ class MapMerger:
             return None, None
         return out.data, (out.info.origin.position.x, out.info.origin.position.y)
 
+    # ---- fused occupancy map (EXTENSION, no reference counterpart) ------------------------------
+    def fuse_occupancy(self, grids, origins, res, transforms, target):
+        """Resample every agent map into ``target`` under its agent->global transform and keep free
+        space: each target cell becomes max(-1, max of the covering agents' cells at its centre), so
+        occupied beats free beats unknown (``mapmerge_warp_fuse`` in include/occgrid_b200.h gives the
+        exact arithmetic).  Unlike ``merge``, the result can be explored: ``target.get_frontiers()``,
+        ``cluster_frontiers()`` and ``frontier_centroids()`` work on it.
+
+        grids       int8 [A, H, W]; a contiguous CUDA tensor on this merger's device (such as
+                    ``AgentGrids.grids_tensor``) is used without a copy, a host array is uploaded once
+        origins     float64 [A, 2], agent a's (origin_x, origin_y); ``res`` the agents' resolution
+        transforms  [A, 4, 4], [A, 3] (tx, ty, theta) or None (identity); every one applied as given
+        target      an ``OccupancyGrid`` holding its whole grid, on this merger's device, with its own
+                    size, resolution and origin; all of its cells are overwritten
+        Returns ``target``.  The merger's cloud and state are left alone."""
+        if target.window != (0, 0, target.size, target.size):
+            raise OccGridError('fuse_occupancy: the target must hold its whole grid (not a window of it)')
+        if target.device != self.device:
+            raise OccGridError(f'fuse_occupancy: the target is on {target.device}, the merger on {self.device}')
+        if isinstance(grids, torch.Tensor):
+            if grids.is_cuda and grids.device != self.device:
+                raise OccGridError(f'fuse_occupancy: the grids are on {grids.device}, the merger on {self.device}')
+            if grids.dtype != torch.int8:
+                raise ValueError('fuse_occupancy: grids must be int8')
+        else:
+            grids = np.ascontiguousarray(np.asarray(grids), dtype=np.int8)
+        if grids.ndim != 3 or min(grids.shape) < 1:
+            raise ValueError(f'fuse_occupancy: grids must be [A, H, W] with A, H, W >= 1, got {tuple(grids.shape)}')
+        A, h, w = (int(v) for v in grids.shape)
+        org = np.asarray(origins, np.float64)
+        if org.size != 2 * A:
+            raise ValueError(f'fuse_occupancy: origins must be [{A}, 2], got {org.shape}')
+        org = np.ascontiguousarray(org.reshape(A, 2))
+        if transforms is not None and len(transforms) != A:
+            raise ValueError(f'fuse_occupancy: {len(transforms)} transforms for {A} grids')
+        Tm = self._as_matrices(transforms, A)
+        lib = self._lib
+        with torch.cuda.device(self.device):
+            if isinstance(grids, np.ndarray):
+                grids = torch.from_numpy(grids).to(self.device)
+            elif not (grids.is_cuda and grids.is_contiguous()):
+                grids = grids.to(self.device).contiguous()
+            nbytes = lib.mapmerge_warp_fuse_workspace_bytes(A, target.size, target.size)
+            if nbytes == 0:
+                raise OccGridError('mapmerge_warp_fuse_workspace_bytes: ' + _native.last_error())
+            ws = self._workspace('fuse', nbytes)
+            rc = lib.mapmerge_warp_fuse(grids.data_ptr(), A, w, h, float(res), org.ctypes.data, Tm.ctypes.data,
+                                        target.ox, target.oy, target.res, target.size, target.size,
+                                        target.grid_tensor.data_ptr(), ws.data_ptr(), ws.numel(), self._stream())
+            _native.check(rc, 'mapmerge_warp_fuse')
+        target._host_cache = None
+        return target
+
     # ---- pieces of the batched merge (also driven by distributed.ShardedMapMerger) ---------------
     def _count_occupied(self, dev, same_shape):
         """Pass 1 over the grids: occupied cells per grid (device int64 [A]).  Equal-shaped grids go

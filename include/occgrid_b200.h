@@ -462,6 +462,37 @@ int mapmerge_rasterise(const double* d_px, const double* d_py, const int64_t* d_
  * of the multi-GPU fuse; the cross-GPU half is an NCCL max-reduction on int8. */
 int mapmerge_fuse_max(int8_t* d_dst, const int8_t* d_src, int64_t n, void* stream);
 
+/* EXTENSION (no reference counterpart): fused occupancy map.  Resamples every map of a stack
+ * d_maps int8 [n_agents][height][width] (row-major [gy][gx], agent a's origin origins_host[a] =
+ * (ox_a, oy_a), resolution res for all) into one target grid d_out int8 [out_h][out_w] with origin
+ * (out_ox, out_oy) and resolution out_res, and keeps free space: out = max(-1, max over the agents
+ * covering a cell of their cell value), so with -1/0/100 maps occupied beats free beats unknown and
+ * the result does not depend on agent order.  Every target cell is written (-1 where no agent
+ * covers it); the previous contents do not matter.
+ *   T_host [n_agents][16]: agent->global 4x4 row-major, R = T[0:2,0:2], t = (T[0][3], T[1][3]), each
+ *   applied as given (nothing is adopted).  Rejected unless every entry is finite and every entry of
+ *   R^T R - I is within 1e-9; the inverse used is R^T.
+ * Coefficients (host fp64, each operation rounded on its own, as bracketed):
+ *   bx = (out_ox + 0.5*g) - tx        by = (out_oy + 0.5*g) - ty        (g = out_res, r = res)
+ *   c0 = (R00*g)/r   c1 = (R10*g)/r   c2 = ((R00*bx + R10*by) - ox_a)/r
+ *   c3 = (R01*g)/r   c4 = (R11*g)/r   c5 = ((R01*bx + R11*by) - oy_a)/r
+ * Per target cell, column j and row i (device fp64, no contraction):
+ *   u = (c0*j) + ((c1*i) + c2)        v = (c3*j) + ((c4*i) + c5)
+ *   agent a covers the cell iff 0 <= u < width and 0 <= v < height (NaN never covers), and then
+ *   contributes map_a[(int)v][(int)u].
+ * An identity transform into a target of the maps' geometry returns the map bit for bit.
+ * n_agents 1..65535; the stack and the target may exceed 2^31 bytes.  OCCGRID_E_ARG for NULL
+ * pointers, n_agents or a size out of range, a resolution that is not finite and > 0, a stack whose
+ * size overflows size_t and a non-finite or non-rigid transform; OCCGRID_E_WORKSPACE for d_ws
+ * smaller than mapmerge_warp_fuse_workspace_bytes (64 bytes per agent, which returns 0 for
+ * n_agents or a target size out of range).  Stream-ordered: no atomics and no host
+ * synchronisation; the per-agent coefficients are copied into d_ws with cudaMemcpyAsync. */
+size_t mapmerge_warp_fuse_workspace_bytes(int n_agents, int32_t out_w, int32_t out_h);
+int mapmerge_warp_fuse(const int8_t* d_maps, int n_agents, int32_t width, int32_t height, double res,
+                       const double* origins_host /* [A][2] */, const double* T_host /* [A][16] */,
+                       double out_ox, double out_oy, double out_res, int32_t out_w, int32_t out_h,
+                       int8_t* d_out, void* d_ws, size_t ws_bytes, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  *  Frontier detection and clustering (SURVEY §8 row f1) — dual_bot_mapper.py:181-237, :948-956
  * ---------------------------------------------------------------------------------------- */
