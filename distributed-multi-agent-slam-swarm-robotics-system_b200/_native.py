@@ -13,7 +13,7 @@ import subprocess
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, 'csrc')
 LIB_PATH = os.path.join(PKG_DIR, 'liboccgrid_b200.so')
-SOURCES = ['occgrid_integrate.cu', 'occgrid_tiled.cu', 'occgrid_route.cu', 'occgrid_band.cu', 'mapmerge.cu', 'frontier.cu', 'icp.cu', 'render.cu', 'map_fuse.cu', 'slam_chain.cpp']
+SOURCES = ['occgrid_integrate.cu', 'occgrid_tiled.cu', 'occgrid_route.cu', 'occgrid_band.cu', 'mapmerge.cu', 'frontier.cu', 'icp.cu', 'render.cu', 'map_fuse.cu', 'frontier_assign.cu', 'slam_chain.cpp']
 HEADERS = ['common.cuh', 'beam_expand.cuh', 'block_ops.cuh', 'sincos_dd.cuh', os.path.join('..', '..', 'include', 'occgrid_b200.h')]
 
 STRATEGY = {'auto': -1, 'global_atomic': 0, 'tiled': 1}
@@ -214,12 +214,19 @@ def _bind_merge(L):
     L.mapmerge_warp_fuse_workspace_bytes.argtypes = [C.c_int, i32, i32]
     L.mapmerge_warp_fuse.restype = C.c_int
     L.mapmerge_warp_fuse.argtypes = [vp, C.c_int, i32, i32, dbl, vp, vp, dbl, dbl, dbl, i32, i32, vp, vp, sz, vp]
+    L.occgrid_frontier_assign_workspace_bytes.restype = sz
+    L.occgrid_frontier_assign_workspace_bytes.argtypes = [i32, i32, i32, i32, i64]
+    L.occgrid_frontier_assign.restype = C.c_int
+    L.occgrid_frontier_assign.argtypes = [vp, i32, i32, dbl, dbl, dbl, vp, i32, vp, vp, vp, vp, vp, vp, i32, i64,
+                                          vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
+    L.occgrid_geodesic_field.restype = C.c_int
+    L.occgrid_geodesic_field.argtypes = [vp, i32, i32, dbl, dbl, dbl, vp, i64, vp, vp, vp, vp, sz, vp]
 
 
 KERNEL_NAMES = ('integrate_global', 'resolve', 'update_rays', 'tile_count', 'tile_scan', 'tile_scatter',
                 'tile_raycast', 'tile_resolve', 'merge_extract', 'merge_bounds', 'merge_voxel', 'merge_raster',
                 'merge_fuse', 'probe', 'route', 'frontier', 'frontier_cluster', 'chain_probe', 'chain_incremental',
-                'chain_rebuild', 'icp', 'band_barrier', 'render', 'merge_scan', 'merge_warp_fuse')
+                'chain_rebuild', 'icp', 'band_barrier', 'render', 'merge_scan', 'merge_warp_fuse', 'frontier_assign')
 
 
 def profile_begin():

@@ -18,6 +18,7 @@ library or a CUDA device the compute entry points raise.
 from __future__ import annotations
 
 import ctypes
+import dataclasses
 import math
 import struct
 
@@ -127,6 +128,8 @@ class OccupancyGrid:
         self._copy_stream = None
         self._tab_cache = None
         self._fr = None
+        self._ws_assign = None
+        self._fa_sizes = {'pool': 4096, 'kmax': 1024}
         if not lazy_workspace:                  # (the multi-GPU band step brings its own workspace)
             self._ensure_workspace(int(max_batch))
 
@@ -514,6 +517,16 @@ class OccupancyGrid:
         xy = f['xy'][:n].cpu().numpy()
         return [(int(x), int(y)) for x, y in xy]
 
+    def _launch_clusters(self, f, min_cluster):
+        """Enqueues the stencil and the clustering into the buffers ``f``."""
+        self._launch_frontiers(f)
+        with torch.cuda.device(self.device):
+            rc = self._lib.occgrid_frontier_clusters(
+                f['xy'].data_ptr(), f['count'].data_ptr(), f['cap'], self.size, int(min_cluster), self.ox, self.oy, self.res,
+                f['label'].data_ptr(), f['root'].data_ptr(), f['size'].data_ptr(), f['cent'].data_ptr(), f['ncl'].data_ptr(),
+                f['ws'].data_ptr(), f['ws'].numel(), self._stream())
+            _native.check(rc, 'occgrid_frontier_clusters')
+
     def _cluster(self, min_cluster=FRONTIER_MIN_CLUSTER):
         """Stencil + clustering enqueued back to back (the cluster kernels take the frontier count
         from device memory), then ONE host read of (count, status, clusters)."""
@@ -522,13 +535,8 @@ class OccupancyGrid:
             cap = max(cap, self._fr['cap'])
         while True:
             f = self._frontier_buffers(cap)
-            self._launch_frontiers(f)
+            self._launch_clusters(f, min_cluster)
             with torch.cuda.device(self.device):
-                rc = self._lib.occgrid_frontier_clusters(
-                    f['xy'].data_ptr(), f['count'].data_ptr(), f['cap'], self.size, int(min_cluster), self.ox, self.oy, self.res,
-                    f['label'].data_ptr(), f['root'].data_ptr(), f['size'].data_ptr(), f['cent'].data_ptr(), f['ncl'].data_ptr(),
-                    f['ws'].data_ptr(), f['ws'].numel(), self._stream())
-                _native.check(rc, 'occgrid_frontier_clusters')
                 host = torch.cat([f['count'], f['status'].to(torch.int64), f['ncl']]).cpu().tolist()
             if host[1] & 1:                       # the list overflowed (count was forced to 0): grow and redo
                 f['status'].zero_()
@@ -567,6 +575,118 @@ class OccupancyGrid:
         f, n, k = self._cluster()
         return [(float(x), float(y)) for x, y in f['cent'][:k].cpu().numpy()]
 
+    # ---- frontier assignment (EXTENSION; the reference's is commented out, :958-996) ---------------
+    def _robot_positions(self, robot_xy, who):
+        xy = np.ascontiguousarray(np.asarray(robot_xy, dtype=np.float64))
+        if xy.ndim != 2 or xy.shape[1] != 2:
+            raise ValueError(f'{who}: robot_xy must be [A, 2] world positions, got shape {xy.shape}')
+        if not 1 <= xy.shape[0] <= MAX_ASSIGN_ROBOTS:
+            raise ValueError(f'{who}: {xy.shape[0]} robots, need 1..{MAX_ASSIGN_ROBOTS}')
+        if self.window != (0, 0, self.size, self.size):
+            raise OccGridError(f'{who} needs the whole grid (not a window of it)')
+        with torch.cuda.device(self.device):
+            return torch.from_numpy(xy).to(self.device)
+
+    def _assign_workspace(self, n_robots, max_clusters, tile_pool):
+        nb = self._lib.occgrid_frontier_assign_workspace_bytes(self.size, self.size, n_robots, max_clusters, tile_pool)
+        if nb == 0:
+            raise OccGridError('occgrid_frontier_assign_workspace_bytes: ' + _native.last_error())
+        if self._ws_assign is None or self._ws_assign.numel() < nb:
+            self._ws_assign = None
+            with torch.cuda.device(self.device):
+                self._ws_assign = torch.empty(nb, dtype=torch.uint8, device=self.device)
+        return self._ws_assign
+
+    def assign_frontiers(self, robot_xy, min_cluster=FRONTIER_MIN_CLUSTER):
+        """EXTENSION: one exploration target per robot by geodesic distance over the known free
+        space (``occgrid_frontier_assign`` in include/occgrid_b200.h gives the exact rules).
+
+        robot_xy  [A, 2] world positions, 1 <= A <= 65 535; a robot outside the grid or at a
+                  non-finite position has no source and gets no target.
+        Runs the frontier stencil, the clustering (``min_cluster`` as ``cluster_frontiers``) and the
+        assignment back to back on the device and reads the result once.  Returns a
+        ``FrontierAssignment``: robot a takes cluster ``cluster[a]`` (``frontier_centroids()``
+        order, -1 for none) at path length ``cost[a]`` cells, reaching it first at cell ``goal[a]``;
+        ``target_xy[a]`` is that cluster's centroid (NaN for none) and ``costs[a, k]`` robot a's
+        path length to cluster k (-1 when unreachable).  The tile pool grows until it holds every
+        field."""
+        d_xy = self._robot_positions(robot_xy, 'assign_frontiers')
+        A = d_xy.shape[0]
+        n_tiles = ((self.size + 63) // 64) ** 2
+        st = self._fa_sizes
+        cap = max(1 << 16, self.size * 8, self._fr['cap'] if self._fr is not None else 0)
+        dev = self.device
+        while True:
+            pool = min(max(st['pool'], 16 * A), A * n_tiles)       # A * n_tiles slots can never run out
+            kmax = st['kmax']
+            f = self._frontier_buffers(cap)
+            ws = self._assign_workspace(A, kmax, pool)
+            with torch.cuda.device(dev):
+                out = {'cluster': torch.empty(A, dtype=torch.int32, device=dev),
+                       'cost': torch.empty(A, dtype=torch.int32, device=dev),
+                       'goal': torch.empty((A, 2), dtype=torch.int32, device=dev),
+                       'target_xy': torch.empty((A, 2), dtype=torch.float64, device=dev),
+                       'costs': torch.empty((A, kmax), dtype=torch.int32, device=dev)}
+                hdr = torch.zeros(8, dtype=torch.int64, device=dev)     # count, frontier status, n_clusters, status, stats[3]
+                status = torch.zeros(1, dtype=torch.int32, device=dev)
+                self._launch_clusters(f, min_cluster)
+                rc = self._lib.occgrid_frontier_assign(
+                    self.grid_tensor.data_ptr(), self.size, self.size, self.ox, self.oy, self.res, d_xy.data_ptr(), A,
+                    f['xy'].data_ptr(), f['count'].data_ptr(), f['label'].data_ptr(), f['root'].data_ptr(), f['cent'].data_ptr(),
+                    f['ncl'].data_ptr(), kmax, pool, out['cluster'].data_ptr(), out['cost'].data_ptr(), out['goal'].data_ptr(),
+                    out['target_xy'].data_ptr(), out['costs'].data_ptr(), status.data_ptr(), hdr[4:7].data_ptr(),
+                    ws.data_ptr(), ws.numel(), self._stream())
+                _native.check(rc, 'occgrid_frontier_assign')
+                hdr[0:1].copy_(f['count'])
+                hdr[1:2].copy_(f['status'])
+                hdr[2:3].copy_(f['ncl'])
+                hdr[3:4].copy_(status)
+                host = {k: torch.empty(v.shape, dtype=v.dtype, pin_memory=True) for k, v in out.items()}
+                host['hdr'] = torch.empty(8, dtype=torch.int64, pin_memory=True)
+                host['hdr'].copy_(hdr, non_blocking=True)
+                for k, v in out.items():
+                    host[k].copy_(v, non_blocking=True)
+                torch.cuda.current_stream(dev).synchronize()          # the one host read
+            count, fstatus, ncl, astatus, rounds, items, slots = host['hdr'][:7].tolist()
+            if fstatus & 1:                       # the frontier list overflowed: grow and redo
+                f['status'].zero_()
+                cap *= 4
+                continue
+            if astatus & 2:
+                raise OccGridError('occgrid_frontier_assign: a grid barrier of the worklist kernel timed out')
+            if astatus & 1:                       # the tile pool ran out: grow and redo
+                st['pool'] = pool * 4
+                continue
+            if astatus & 4:                       # more clusters than columns: widen and redo
+                st['kmax'] = 1 << int(ncl - 1).bit_length()
+                continue
+            return FrontierAssignment(host['cluster'].numpy(), host['cost'].numpy(), host['goal'].numpy(),
+                                      host['target_xy'].numpy(), host['costs'].numpy()[:, :ncl].copy(),
+                                      {'frontier_cells': count, 'clusters': ncl, 'rounds': rounds, 'items': items,
+                                       'tile_slots': slots, 'tile_pool': pool})
+
+    def geodesic_distance(self, robot_xy, to_host=True):
+        """EXTENSION: the geodesic field of one robot at world position ``robot_xy`` = (x, y):
+        int32 [size, size] indexed [gy, gx], the 4-connected path length in cells over FREE cells
+        from the robot's cell (0 there whatever its value), -1 where unreachable or when the robot
+        is outside the grid.  For navigation: descend the field from a goal cell to the robot."""
+        xy = np.asarray(robot_xy, np.float64)
+        if xy.size != 2:
+            raise ValueError(f'geodesic_distance: robot_xy must be one (x, y) world position, got shape {xy.shape}')
+        d_xy = self._robot_positions(xy.reshape(1, 2), 'geodesic_distance')
+        pool = ((self.size + 63) // 64) ** 2                 # every tile: the pool cannot run out
+        ws = self._assign_workspace(1, 1, pool)
+        with torch.cuda.device(self.device):
+            field = torch.empty((self.size, self.size), dtype=torch.int32, device=self.device)
+            status = torch.zeros(1, dtype=torch.int32, device=self.device)
+            rc = self._lib.occgrid_geodesic_field(self.grid_tensor.data_ptr(), self.size, self.size, self.ox, self.oy, self.res,
+                                                  d_xy.data_ptr(), pool, field.data_ptr(), status.data_ptr(), None,
+                                                  ws.data_ptr(), ws.numel(), self._stream())
+            _native.check(rc, 'occgrid_geodesic_field')
+            if int(status.item()) != 0:
+                raise OccGridError(f'occgrid_geodesic_field: status {int(status.item())} (worklist failed)')
+        return field.cpu().numpy() if to_host else field
+
     # ---- overlay render (:492-527) — SURVEY §8 row f4 -----------------------------------------
     def render_overlay(self, width=1000, height=800, scale=100.0, offset_x=None, offset_y=None,
                        background=BG_COLOR, color=CELL_COLOR_FREE, to_host=True):
@@ -601,6 +721,27 @@ class OccupancyGrid:
         self._host_cache = None
 
 
+MAX_ASSIGN_ROBOTS = 65535
+
+
+@dataclasses.dataclass(frozen=True)
+class FrontierAssignment:
+    """Result of ``OccupancyGrid.assign_frontiers`` for A robots and K clusters (NumPy arrays)."""
+    cluster: np.ndarray      # int32 [A]: assigned cluster in frontier_centroids() order, -1 for none
+    cost: np.ndarray         # int32 [A]: path length in cells to the cluster's nearest cell, -1 for none
+    goal: np.ndarray         # int32 [A, 2]: (gx, gy) of that cell (lowest y * size + x on ties), -1 for none
+    target_xy: np.ndarray    # float64 [A, 2]: the cluster's centroid in world metres, NaN for none
+    costs: np.ndarray        # int32 [A, K]: path length from robot a to cluster k, -1 when unreachable
+    stats: dict              # frontier cells, clusters, worklist rounds, (robot, tile) items, tile slots used, pool
+
+
+def target_packets(result):
+    """``TARGET_FMT`` datagrams (b'TARG', x, y as float32) for the robots of ``result`` that have a
+    target, keyed by agent id: robot a of the ``assign_frontiers`` call is agent a + 1."""
+    return {a + 1: struct.pack(TARGET_FMT, b'TARG', float(x), float(y))
+            for a, (k, (x, y)) in enumerate(zip(result.cluster.tolist(), result.target_xy.tolist())) if k >= 0}
+
+
 def _single_map_only(name):
     def method(self, *args, **kwargs):
         raise OccGridError(f'AgentGrids.{name}: single-map operation; run it on an OccupancyGrid built from grid(agent_id)')
@@ -626,7 +767,7 @@ class AgentGrids(OccupancyGrid):
     frontiers, rendering) raise ``OccGridError``.  For frontiers on the swarm's map,
     ``MapMerger().fuse_occupancy(maps.grids_tensor, maps.origins, maps.res, transforms, target)``
     fuses the stack into an ``OccupancyGrid`` that keeps free space; ``target.frontier_centroids()``
-    then runs there.
+    and ``target.assign_frontiers(robot_xy)`` then run there.
     """
 
     def __init__(self, n_agents=2, size=GRID_SIZE, resolution=GRID_RESOLUTION,
@@ -703,6 +844,8 @@ class AgentGrids(OccupancyGrid):
     get_frontiers = _single_map_only('get_frontiers')
     cluster_frontiers = _single_map_only('cluster_frontiers')
     frontier_centroids = _single_map_only('frontier_centroids')
+    assign_frontiers = _single_map_only('assign_frontiers')
+    geodesic_distance = _single_map_only('geodesic_distance')
     render_overlay = _single_map_only('render_overlay')
 
 

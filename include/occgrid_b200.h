@@ -516,6 +516,71 @@ int occgrid_frontier_clusters(const int32_t* d_xy, const int64_t* d_count, int64
                               double* d_centroids, int64_t* d_n_clusters,
                               void* d_ws, size_t ws_bytes, void* stream);
 
+/* EXTENSION (no reference counterpart; the reference's assignment is commented out,
+ * dual_bot_mapper.py:958-996): frontier assignment by geodesic distance (DESIGN §6e).
+ * Inputs:
+ *   a grid int8 [H][W] (-1 / 0 / 100, [gy][gx]), origin (ox, oy) and resolution res;
+ *   robot positions in world metres, d_robot_xy double [A][2], 1 <= A <= 65 535;
+ *   the frontier clusters as occgrid_frontier_clusters leaves them on the device: the xy list,
+ *   d_count, d_label, d_cluster_root, d_centroids and d_n_clusters (cluster membership is read
+ *   from the labels and the ascending root list, so min_cluster is the one the clusters used).
+ * Rules:
+ *   Robot cell: the reference's world_to_grid, int((w - o) / res) with true fp64 division and
+ *     truncation.  A robot whose cell lies outside the grid, or whose position is not finite, has
+ *     no source: its row of costs is all -1 and it gets no target.
+ *   Geodesic distance: D_a(c) is the 4-connected, unit-cost BFS distance from robot a's cell.  The
+ *     source gets 0 whatever its value; the search moves only into FREE (0) cells.  Unreachable
+ *     cells are -1; values are int32.  D is the unique fixed point of
+ *     D(c) = min(seed(c), c FREE ? min over 4-neighbours n of D(n) + 1 : unreachable),
+ *     so any correct relaxation order gives the same field bit for bit.
+ *   Cost: cost[a][k] = min over the cells c of cluster k of D_a(c), or -1 when none is reachable;
+ *     the goal cell attains it, ties to the lowest linear index y*W + x.  Clusters are numbered in
+ *     frontier_centroids() order.
+ *   Assignment: a greedy pass in robot order.  For a = 0..A-1, robot a takes the unclaimed
+ *     cluster with the smallest non-negative cost[a][k], ties to the lowest k, and claims it.  A
+ *     robot left with no reachable unclaimed cluster gets -1.
+ * Outputs (device): d_cluster int32 [A], d_cost int32 [A], d_goal int32 [A][2] (x, y), d_target
+ * double [A][2] (the assigned cluster's centroid copied from d_centroids, NaN when none; cluster,
+ * cost and goal are -1 then) and d_costs int32 [A][max_clusters], of which columns
+ * 0..n_clusters-1 are written.  d_stats (optional, int64 [3]) receives the worklist rounds, the
+ * (robot, tile) items processed and the pool slots used.
+ * Fields are stored per (robot, 64 x 64 tile) in a pool of tile_pool slots of 16 KB inside d_ws.
+ * d_status bits are OR-ed in (zero it first):
+ *   OCCGRID_ASSIGN_POOL_FULL      the tile pool (or the worklist, which holds tile_pool items) ran
+ *                                 out; nothing is written outside the workspace and the outputs
+ *                                 are all "no target".  Grow tile_pool and call again.
+ *   OCCGRID_ASSIGN_TIMEOUT        a grid barrier of the worklist kernel timed out (an error).
+ *   OCCGRID_ASSIGN_CLUSTERS_FULL  n_clusters > max_clusters; the outputs are all "no target".
+ * OCCGRID_E_ARG (message key word in quotes) for a "NULL pointer", "n_robots" outside 1..65 535,
+ * "width x height" below 3 or a grid of 2^31 - 1 cells or more, a "resolution" that is not finite
+ * and > 0, a "capacity" (max_clusters, tile_pool) outside 1..2^31 - 1 and a workspace that
+ * "overflows size_t" (the [A][n_tiles] slot tables); OCCGRID_E_WORKSPACE for ws_bytes below
+ * occgrid_frontier_assign_workspace_bytes (which returns 0 for the same argument errors).
+ * Stream-ordered: the robots are read on the device, and the worklist runs as one cooperative
+ * launch with no host round trip. */
+#define OCCGRID_ASSIGN_POOL_FULL     1
+#define OCCGRID_ASSIGN_TIMEOUT       2
+#define OCCGRID_ASSIGN_CLUSTERS_FULL 4
+size_t occgrid_frontier_assign_workspace_bytes(int32_t width, int32_t height, int32_t n_robots,
+                                               int32_t max_clusters, int64_t tile_pool);
+int occgrid_frontier_assign(const int8_t* d_grid, int32_t width, int32_t height, double ox, double oy,
+                            double res, const double* d_robot_xy, int32_t n_robots,
+                            const int32_t* d_xy, const int64_t* d_count, const int32_t* d_label,
+                            const int32_t* d_cluster_root, const double* d_centroids,
+                            const int64_t* d_n_clusters, int32_t max_clusters, int64_t tile_pool,
+                            int32_t* d_cluster, int32_t* d_cost, int32_t* d_goal, double* d_target,
+                            int32_t* d_costs, int32_t* d_status, int64_t* d_stats,
+                            void* d_ws, size_t ws_bytes, void* stream);
+
+/* One robot's dense geodesic field d_field int32 [H][W] (the D_a above, -1 where unreachable),
+ * for navigation (descend the field to the goal).  The same worklist run for the one robot at
+ * d_robot_xy double [2], then its tiles expanded.  Workspace:
+ * occgrid_frontier_assign_workspace_bytes(width, height, 1, 1, tile_pool).  Status bits, stats and
+ * argument errors as occgrid_frontier_assign; d_field is not written when the pool ran out. */
+int occgrid_geodesic_field(const int8_t* d_grid, int32_t width, int32_t height, double ox, double oy,
+                           double res, const double* d_robot_xy, int64_t tile_pool, int32_t* d_field,
+                           int32_t* d_status, int64_t* d_stats, void* d_ws, size_t ws_bytes, void* stream);
+
 /* Tuning knob of the TILED strategy: cap the persistent raycast CTAs per SM (0 = as many as fit,
  * the default).  A pipelined multi-GPU ingest lowers it to 2 so that the routing kernel of the
  * next batch finds room on every SM and runs concurrently.  Process-wide. */
