@@ -13,8 +13,8 @@ import subprocess
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, 'csrc')
 LIB_PATH = os.path.join(PKG_DIR, 'liboccgrid_b200.so')
-SOURCES = ['occgrid_integrate.cu', 'occgrid_tiled.cu', 'occgrid_route.cu', 'occgrid_band.cu', 'mapmerge.cu', 'frontier.cu', 'icp.cu', 'render.cu', 'map_fuse.cu', 'frontier_assign.cu', 'slam_chain.cpp']
-HEADERS = ['common.cuh', 'beam_expand.cuh', 'block_ops.cuh', 'sincos_dd.cuh', os.path.join('..', '..', 'include', 'occgrid_b200.h')]
+SOURCES = ['occgrid_integrate.cu', 'occgrid_tiled.cu', 'occgrid_route.cu', 'occgrid_band.cu', 'mapmerge.cu', 'frontier.cu', 'icp.cu', 'icp_batch.cu', 'render.cu', 'map_fuse.cu', 'frontier_assign.cu', 'slam_chain.cpp']
+HEADERS = ['common.cuh', 'beam_expand.cuh', 'block_ops.cuh', 'icp_core.cuh', 'sincos_dd.cuh', os.path.join('..', '..', 'include', 'occgrid_b200.h')]
 
 STRATEGY = {'auto': -1, 'global_atomic': 0, 'tiled': 1}
 COUNTER_NAMES = ('packets', 'accepted', 'dropped', 'bad_pose', 'beams', 'hits', 'updates', 'slowpath',
@@ -190,6 +190,13 @@ def _bind_merge(L):
     L.mapmerge_icp_workspace_bytes.argtypes = [i64, i64, i32, i32]
     L.mapmerge_icp_register.restype = C.c_int
     L.mapmerge_icp_register.argtypes = [vp, vp, i64, vp, vp, i64, dbl, dbl, dbl, i32, i32, dbl, i32, dbl, dbl, vp, vp, sz, vp]
+    L.mapmerge_icp_register_batch_workspace_bytes.restype = sz
+    L.mapmerge_icp_register_batch_workspace_bytes.argtypes = [i64, i64, C.c_int, i32, i32]
+    L.mapmerge_icp_register_batch.restype = C.c_int
+    L.mapmerge_icp_register_batch.argtypes = [vp, vp, vp, C.c_int, vp, vp, i64, dbl, dbl, dbl, i32, i32, dbl, i32, dbl, dbl,
+                                              vp, vp, sz, vp]
+    L.mapmerge_icp_batch_set_max_ctas.restype = C.c_int
+    L.mapmerge_icp_batch_set_max_ctas.argtypes = [C.c_int]
     L.occgrid_slam_create.restype = vp
     L.occgrid_slam_create.argtypes = []
     L.occgrid_slam_destroy.restype = None
@@ -226,7 +233,8 @@ def _bind_merge(L):
 KERNEL_NAMES = ('integrate_global', 'resolve', 'update_rays', 'tile_count', 'tile_scan', 'tile_scatter',
                 'tile_raycast', 'tile_resolve', 'merge_extract', 'merge_bounds', 'merge_voxel', 'merge_raster',
                 'merge_fuse', 'probe', 'route', 'frontier', 'frontier_cluster', 'chain_probe', 'chain_incremental',
-                'chain_rebuild', 'icp', 'band_barrier', 'render', 'merge_scan', 'merge_warp_fuse', 'frontier_assign')
+                'chain_rebuild', 'icp', 'band_barrier', 'render', 'merge_scan', 'merge_warp_fuse', 'frontier_assign',
+                'icp_batch')
 
 
 def profile_begin():

@@ -50,7 +50,8 @@ static_assert(sizeof(PoseRec) == 48, "PoseRec must be 48 bytes");
 enum KernelId { K_INTEGRATE_GLOBAL = 0, K_RESOLVE, K_UPDATE_RAYS, K_TILE_COUNT, K_TILE_SCAN, K_TILE_SCATTER,
                 K_TILE_RAYCAST, K_TILE_RESOLVE, K_MERGE_EXTRACT, K_MERGE_BOUNDS, K_MERGE_VOXEL, K_MERGE_RASTER,
                 K_MERGE_FUSE, K_PROBE, K_ROUTE, K_FRONTIER, K_FRONTIER_CLUSTER, K_CHAIN_PROBE, K_CHAIN_INCR,
-                K_CHAIN_REBUILD, K_ICP, K_BAND_BARRIER, K_RENDER, K_MERGE_SCAN, K_MERGE_WARP_FUSE, K_FRONTIER_ASSIGN, K_N_KERNELS };
+                K_CHAIN_REBUILD, K_ICP, K_BAND_BARRIER, K_RENDER, K_MERGE_SCAN, K_MERGE_WARP_FUSE, K_FRONTIER_ASSIGN,
+                K_ICP_BATCH, K_N_KERNELS };
 bool profile_enabled();
 void profile_mark(int kernel_id, cudaStream_t st, bool begin, int n_kernels);
 

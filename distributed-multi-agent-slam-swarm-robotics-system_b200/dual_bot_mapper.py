@@ -767,7 +767,10 @@ class AgentGrids(OccupancyGrid):
     frontiers, rendering) raise ``OccGridError``.  For frontiers on the swarm's map,
     ``MapMerger().fuse_occupancy(maps.grids_tensor, maps.origins, maps.res, transforms, target)``
     fuses the stack into an ``OccupancyGrid`` that keeps free space; ``target.frontier_centroids()``
-    and ``target.assign_frontiers(robot_xy)`` then run there.
+    and ``target.assign_frontiers(robot_xy)`` then run there.  Transforms that drift are refined
+    first against the previous fused map, in one call for all agents: the loop is
+    ``maps -> register_maps(grids_tensor, origins, res, priors, reference=last_fused) ->
+    fuse_occupancy(..., result.transformation, target) -> assign_frontiers``.
     """
 
     def __init__(self, n_agents=2, size=GRID_SIZE, resolution=GRID_RESOLUTION,

@@ -474,6 +474,140 @@ class MapMerger:
         target._host_cache = None
         return target
 
+    # ---- batched map registration (EXTENSION, no reference counterpart) -------------------------
+    def register_maps(self, grids, origins, res, priors, reference=None, threshold=1.0, max_iteration=30,
+                      relative_fitness=1e-6, relative_rmse=1e-6):
+        """Refine every agent->global transform against ONE reference map in one device call: agent
+        a's occupied cells (> 50) at cell corners, moved by ``priors[a]``, are registered with
+        ``registration_icp(…, threshold, identity, point-to-point, max_iteration)`` (:45-52) against
+        the reference cloud (``mapmerge_icp_register_batch`` in include/occgrid_b200.h).  Each
+        agent's refinement equals a separate ``register``-style ICP call bit for bit; the cell list
+        of the reference is built once and the loops of all agents run in one cooperative launch.
+
+        grids       int8 [A, H, W] (``AgentGrids.grids_tensor`` is used without a copy); ``origins``
+                    float64 [A, 2]; ``res`` the agents' resolution
+        priors      [A, 4, 4], [A, 3] (tx, ty, theta) or None (identity): rigid agent->global
+                    transforms (every entry finite, |RᵀR − I| <= 1e-9, as ``fuse_occupancy``)
+        reference   None: the merger's global cloud (as ``register``); or an ``OccupancyGrid``
+                    holding its whole grid on this device, whose occupied cells at cell corners are
+                    the reference (typically the previous step's fused map)
+        The host reads twice: the occupied counts with the reference bounds, then the results.
+        Returns a namespace of NumPy arrays: ``refinement`` [A, 4, 4] (the ICP result U_a),
+        ``transformation`` [A, 4, 4] (U_a @ prior_a in fp64 where accepted, else the prior; it goes
+        straight into ``fuse_occupancy``), ``fitness``, ``inlier_rmse``, ``iterations``,
+        ``correspondences`` and ``accepted`` (fitness >= 0.6, the gate at :54-56).  An agent with no
+        occupied cells gets the identity refinement, fitness 0 and 0 iterations."""
+        if isinstance(grids, torch.Tensor):
+            if grids.is_cuda and grids.device != self.device:
+                raise OccGridError(f'register_maps: the grids are on {grids.device}, the merger on {self.device}')
+            if grids.dtype != torch.int8:
+                raise ValueError('register_maps: grids must be int8')
+        else:
+            grids = np.ascontiguousarray(np.asarray(grids), dtype=np.int8)
+        if grids.ndim != 3 or min(grids.shape) < 1:
+            raise ValueError(f'register_maps: grids must be [A, H, W] with A, H, W >= 1, got {tuple(grids.shape)}')
+        A = int(grids.shape[0])
+        org = np.asarray(origins, np.float64)
+        if org.size != 2 * A:
+            raise ValueError(f'register_maps: origins must be [{A}, 2], got {org.shape}')
+        org = np.ascontiguousarray(org.reshape(A, 2))
+        if priors is not None:
+            if len(priors) != A:
+                raise ValueError(f'register_maps: {len(priors)} priors for {A} grids')
+            for a in range(A):
+                if priors[a] is not None and np.asarray(priors[a]).size not in (3, 16):
+                    raise ValueError(f'register_maps: prior {a} must be 4x4 or (tx, ty, theta), got shape {np.asarray(priors[a]).shape}')
+        Tm = self._as_matrices(priors, A)
+        for a in range(A):                       # mapmerge_warp_fuse's rule, in the same fp64 arithmetic
+            T = Tm[a]
+            if not np.isfinite(T).all():
+                raise OccGridError(f'register_maps: prior {a} has a non-finite entry')
+            R = ((T[0, 0], T[0, 1]), (T[1, 0], T[1, 1]))
+            for p in range(2):
+                for q in range(2):
+                    rtr = float(R[0][p]) * float(R[0][q]) + float(R[1][p]) * float(R[1][q])
+                    if not abs(rtr - (1.0 if p == q else 0.0)) <= 1e-9:
+                        raise OccGridError(f'register_maps: prior {a} is not rigid (|R^T R - I| > 1e-9)')
+        if reference is not None:
+            if reference.window != (0, 0, reference.size, reference.size):
+                raise OccGridError('register_maps: the reference must hold its whole grid (not a window of it)')
+            if reference.device != self.device:
+                raise OccGridError(f'register_maps: the reference is on {reference.device}, the merger on {self.device}')
+        elif self._n_global == 0:
+            raise OccGridError('register_maps: the global cloud is empty')
+        lib = self._lib
+        with torch.cuda.device(self.device):
+            job = self._registration_inputs(grids, org, res, Tm, reference, threshold)
+            nbytes = lib.mapmerge_icp_register_batch_workspace_bytes(job.n_target, job.n_points, A, job.cells_w, job.cells_h)
+            if nbytes == 0:
+                raise OccGridError('mapmerge_icp_register_batch_workspace_bytes: ' + _native.last_error())
+            iws = self._workspace('icp', nbytes)
+            out = torch.empty((A, 20), dtype=torch.float64, device=self.device)
+            rc = lib.mapmerge_icp_register_batch(job.sx.data_ptr(), job.sy.data_ptr(), job.offsets.data_ptr(), A, job.tx.data_ptr(),
+                                                 job.ty.data_ptr(), job.n_target, job.min_x, job.min_y, job.cell, job.cells_w,
+                                                 job.cells_h, float(threshold), int(max_iteration), float(relative_fitness),
+                                                 float(relative_rmse), out.data_ptr(), iws.data_ptr(), iws.numel(), self._stream())
+            _native.check(rc, 'mapmerge_icp_register_batch')
+            r = out.cpu().numpy()                                               # host read 2
+        if (r[:, 18] < 0).any():
+            raise OccGridError('register_maps: the batched ICP loop kernel was aborted (grid barrier time-out)')
+        U = np.ascontiguousarray(r[:, :16].reshape(A, 4, 4))
+        fitness = r[:, 16].copy()
+        accepted = fitness >= 0.6                                               # :54-56
+        transformation = np.where(accepted[:, None, None], np.matmul(U, Tm), Tm)
+        return SimpleNamespace(refinement=U, transformation=transformation, fitness=fitness, inlier_rmse=r[:, 17].copy(),
+                               iterations=r[:, 18].astype(np.int64), correspondences=r[:, 19].astype(np.int64),
+                               accepted=accepted)
+
+    def _registration_inputs(self, grids, org, res, Tm, reference, threshold):
+        """The device inputs of mapmerge_icp_register_batch: every agent's occupied cells moved by its
+        prior (one batched extraction), the reference cloud and its cell list.  One host read: the
+        occupied counts with the reference's bounds, size and the status word."""
+        lib = self._lib
+        A = int(grids.shape[0])
+        if isinstance(grids, np.ndarray):
+            grids = torch.from_numpy(grids).to(self.device)
+        elif not (grids.is_cuda and grids.is_contiguous()):
+            grids = grids.to(self.device).contiguous()
+        dev = list(grids.unbind(0))
+        counts, ptrs, bws = self._count_occupied(dev, True)
+        if reference is None:
+            ref, n_ref = self._cloud, torch.full((1,), self._n_global, dtype=torch.int64, device=self.device)
+        else:                                    # the reference's occupied cells: at most one point per cell
+            cells = reference.size * reference.size
+            ref = self._reference_cloud(cells)
+            ref.count.zero_()
+            ws = self._workspace('extract', lib.mapmerge_extract_workspace_bytes(cells))
+            g = reference.grid_tensor
+            rc = lib.mapmerge_extract_transform(g.data_ptr(), reference.size, reference.size, reference.res, reference.ox,
+                                                reference.oy, None, ref.x.data_ptr(), ref.y.data_ptr(), ref.capacity,
+                                                ref.count.data_ptr(), self._last.data_ptr(), self._status.data_ptr(),
+                                                ws.data_ptr(), ws.numel(), self._stream())
+            _native.check(rc, 'mapmerge_extract_transform')
+            n_ref = ref.count
+        self._bounds_of(ref)
+        head = torch.cat([counts.double(), self._bounds, n_ref.double(), self._status.double()]).cpu().numpy()   # host read 1
+        n_occ = head[:A].astype(np.int64)
+        bb = head[A:A + 4].tolist()
+        n_target, status = int(head[A + 4]), int(head[A + 5])
+        if status:
+            self._check_status()
+        if n_target == 0:
+            raise OccGridError('register_maps: the reference has no occupied cells')
+        cell = float(threshold) / 4.0
+        cw, ch = int((bb[2] - bb[0]) / cell) + 2, int((bb[3] - bb[1]) / cell) + 2      # as register
+        n_new = int(n_occ.sum())
+        stage, offs = self._write_slices(dev, ptrs, bws, counts, np.ones(A, bool), Tm, org, res, n_new)
+        return SimpleNamespace(sx=stage.x, sy=stage.y, offsets=offs, n_points=n_new, n_occupied=n_occ, tx=ref.x, ty=ref.y,
+                               n_target=n_target, min_x=bb[0], min_y=bb[1], cell=cell, cells_w=cw, cells_h=ch)
+
+    def _reference_cloud(self, capacity):
+        """Scratch cloud for a reference map's points (grown, never shrunk)."""
+        c = getattr(self, '_ref_cloud', None)
+        if c is None or c.capacity < capacity:
+            c = self._ref_cloud = _Cloud(capacity, self.device)
+        return c
+
     # ---- pieces of the batched merge (also driven by distributed.ShardedMapMerger) ---------------
     def _count_occupied(self, dev, same_shape):
         """Pass 1 over the grids: occupied cells per grid (device int64 [A]).  Equal-shaped grids go

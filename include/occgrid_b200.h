@@ -451,6 +451,54 @@ int mapmerge_icp_register(const double* d_sx, const double* d_sy, int64_t n_sour
                           double relative_fitness, double relative_rmse, double* d_result,
                           void* d_ws, size_t ws_bytes, void* stream);
 
+/* EXTENSION (no reference counterpart): batched map registration (DESIGN §6f).  Refines A
+ * agent->global transforms against ONE reference cloud in one stream-ordered call.
+ * Inputs:
+ *   d_sx, d_sy: the A source clouds back to back, agent a's points at [d_offsets[a], d_offsets[a + 1]);
+ *     d_offsets int64 [n_agents + 1] on the device, d_offsets[0] = 0, non-decreasing.  The
+ *     Python layer passes every agent's occupied cells (> 50) at cell corners transformed by its
+ *     prior, in row-major order: what mapmerge_extract_batch_count / mapmerge_extract_batch_write
+ *     produce.
+ *   d_tx, d_ty: the reference cloud of n_target points (1 <= n_target < 2^32 - 1), binned into the
+ *     cell list of mapmerge_icp_register: cells of size `cell` from (min_x, min_y), cells_w x cells_h.
+ *   max_correspondence_distance (the threshold), max_iteration, relative_fitness, relative_rmse:
+ *     as mapmerge_icp_register.
+ * Per agent a, row d_results[a][0..19] has the layout of mapmerge_icp_register's d_result and
+ * equals, bit for bit, mapmerge_icp_register(source_a, reference, the same cell list and
+ * parameters): the 16 doubles of the refinement U_a, fitness, inlier_rmse, iterations and
+ * correspondences, with the same iteration count and convergence step.  An agent with no points
+ * gets an identity U_a, fitness 0, RMSE 0, iterations 0 and 0 correspondences and is never
+ * launched (the single call rejects n_source <= 0; this is the batched call's own rule).
+ * Iterations -1: a grid barrier of the loop kernel timed out before the agent finished.
+ * Iterations -2 in every row (identity, zeros otherwise): the offset table is not valid, or its
+ * d_offsets[n_agents] points do not fit the workspace.
+ * The cell list is built once; the loops of all agents run in one cooperative launch of
+ * k_icp_loop_batch (a converged agent is skipped in later rounds); the result does not depend on
+ * the grid size.  No host round trip, no atomics in the sums.
+ * Workspace: mapmerge_icp_register_batch_workspace_bytes(n_target, total_source_points, n_agents,
+ * cells_w, cells_h), regions aligned to 256 bytes: three cell tables of (cells + 1) * 4 bytes, the
+ * sorted target (n_target * (8 + 8 + 4)), the scan's block sums ((ceil(cells / 16384) + 1) * 4),
+ * 328 bytes of state per agent, (n_agents + 1) * 4 of block offsets and 256 of barrier words; then
+ * per point 8 + 8 + 4 bytes of working copy and per virtual block (ceil(points / 256) + n_agents of
+ * them) 48 + 16 + 4 bytes.  The call holds as many points as ws_bytes allows.
+ * OCCGRID_E_ARG (message key word in quotes) for a "NULL pointer", "n_agents" outside 1..65 535,
+ * "n_target" outside 1..2^32 - 2, a "cell" or "threshold" that is not finite and > 0,
+ * "max_iteration" below 0, "cells" below 1 and a cell list that "overflows size_t" (the workspace
+ * query also rejects "total_source_points" outside 0..2^39 and returns 0 for every argument
+ * error); OCCGRID_E_WORKSPACE for ws_bytes below the workspace of zero points. */
+size_t mapmerge_icp_register_batch_workspace_bytes(int64_t n_target, int64_t total_source_points,
+                                                   int n_agents, int32_t cells_w, int32_t cells_h);
+int mapmerge_icp_register_batch(const double* d_sx, const double* d_sy, const int64_t* d_offsets,
+                                int n_agents, const double* d_tx, const double* d_ty, int64_t n_target,
+                                double min_x, double min_y, double cell, int32_t cells_w,
+                                int32_t cells_h, double max_correspondence_distance,
+                                int32_t max_iteration, double relative_fitness, double relative_rmse,
+                                double* d_results /* [n_agents][20] */, void* d_ws, size_t ws_bytes,
+                                void* stream);
+/* Testing and tuning knob: cap the CTAs of k_icp_loop_batch (0 = every resident CTA, the default).
+ * Results do not depend on it.  Process-wide; OCCGRID_E_ARG for ctas < 0. */
+int mapmerge_icp_batch_set_max_ctas(int ctas);
+
 /* publish_global_map's rasterisation (:103-111): fill width x height with -1, then
  * grid[int((y-min_y)/res)][int((x-min_x)/res)] = 100 with index clipping (:108-109).
  * width/height follow :100-101 and are computed by the caller from the bounds. */
