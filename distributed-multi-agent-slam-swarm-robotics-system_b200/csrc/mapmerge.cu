@@ -1104,7 +1104,8 @@ using namespace occ;
 extern "C" {
 
 int mapmerge_count_occupied(const int8_t* d_grid, int64_t n_cells, int64_t* d_out, void* stream) {
-    if (!d_grid || !d_out || n_cells < 0) { set_last_error("mapmerge_count_occupied: bad arguments"); return OCCGRID_E_ARG; }
+    if (!d_grid || !d_out) { set_last_error("mapmerge_count_occupied: NULL pointer"); return OCCGRID_E_ARG; }
+    if (n_cells < 0) { set_last_error("mapmerge_count_occupied: n_cells %lld < 0", (long long)n_cells); return OCCGRID_E_ARG; }
     if (n_cells == 0) return OCCGRID_OK;
     cudaStream_t st = (cudaStream_t)stream;
     ProfileScope ps(K_MERGE_EXTRACT, st, 1);
@@ -1161,8 +1162,13 @@ size_t mapmerge_extract_batch_workspace_bytes(int64_t n_cells, int n_agents) {
 // Pass 1 of a batched extraction: per-block and per-agent occupied-cell counts.
 int mapmerge_extract_batch_count(const int8_t* const* d_grids, int n_agents, int32_t width, int32_t height,
                                  int64_t* d_agent_total, void* d_ws, size_t ws_bytes, int grids_bulk_ok, void* stream) {
-    if (!d_grids || n_agents <= 0 || n_agents > 65535 || width <= 0 || height <= 0 || !d_agent_total || !d_ws) {
-        set_last_error("mapmerge_extract_batch_count: bad arguments");
+    if (!d_grids || !d_agent_total || !d_ws) { set_last_error("mapmerge_extract_batch_count: NULL pointer"); return OCCGRID_E_ARG; }
+    if (n_agents <= 0 || n_agents > 65535) {
+        set_last_error("mapmerge_extract_batch_count: n_agents %d outside 1..65535", n_agents);
+        return OCCGRID_E_ARG;
+    }
+    if (width <= 0 || height <= 0) {
+        set_last_error("mapmerge_extract_batch_count: width x height %d x %d", (int)width, (int)height);
         return OCCGRID_E_ARG;
     }
     const long long n_cells = (long long)width * height;
@@ -1201,11 +1207,19 @@ int mapmerge_extract_batch_write(const int8_t* const* d_grids, int n_agents, int
                                  const uint8_t* use_host /* [A] or NULL */, void* d_xforms /* >= A * 96 bytes */,
                                  double* d_px, double* d_py, int64_t capacity, const int64_t* d_agent_total,
                                  int64_t* d_agent_offset, int32_t* d_status, void* d_ws, size_t ws_bytes, void* stream) {
-    if (!d_grids || n_agents <= 0 || n_agents > 65535 || width <= 0 || height <= 0 || !(res > 0.0) || !d_origins || !d_xforms ||
-        !d_px || !d_py || !d_agent_total || !d_agent_offset || !d_status || !d_ws) {
-        set_last_error("mapmerge_extract_batch_write: bad arguments");
+    if (!d_grids || !d_origins || !d_xforms || !d_px || !d_py || !d_agent_total || !d_agent_offset || !d_status || !d_ws) {
+        set_last_error("mapmerge_extract_batch_write: NULL pointer");
         return OCCGRID_E_ARG;
     }
+    if (n_agents <= 0 || n_agents > 65535) {
+        set_last_error("mapmerge_extract_batch_write: n_agents %d outside 1..65535", n_agents);
+        return OCCGRID_E_ARG;
+    }
+    if (width <= 0 || height <= 0) {
+        set_last_error("mapmerge_extract_batch_write: width x height %d x %d", (int)width, (int)height);
+        return OCCGRID_E_ARG;
+    }
+    if (!(res > 0.0)) { set_last_error("mapmerge_extract_batch_write: res %g must be > 0", res); return OCCGRID_E_ARG; }
     const long long n_cells = (long long)width * height;
     if (ws_bytes < mapmerge_extract_batch_workspace_bytes(n_cells, n_agents)) { set_last_error("mapmerge_extract_batch_write: workspace too small"); return OCCGRID_E_WORKSPACE; }
     static_assert(sizeof(BatchXform) <= 96, "BatchXform must fit the 96-byte slot");
@@ -1247,10 +1261,11 @@ int mapmerge_bounds_enc_reset(uint64_t* d_bounds_enc, void* stream) {
 int mapmerge_append_slice(const double* d_sx, const double* d_sy, const int64_t* d_agent_offset, int agent,
                           double* d_px, double* d_py, int64_t capacity, int64_t* d_count, int32_t* d_status,
                           uint64_t* d_bounds_enc, void* stream) {
-    if (!d_sx || !d_sy || !d_agent_offset || agent < 0 || !d_px || !d_py || !d_count || !d_status) {
-        set_last_error("mapmerge_append_slice: bad arguments");
+    if (!d_sx || !d_sy || !d_agent_offset || !d_px || !d_py || !d_count || !d_status) {
+        set_last_error("mapmerge_append_slice: NULL pointer");
         return OCCGRID_E_ARG;
     }
+    if (agent < 0) { set_last_error("mapmerge_append_slice: agent %d < 0", agent); return OCCGRID_E_ARG; }
     cudaStream_t st = (cudaStream_t)stream;
     ProfileScope ps(K_MERGE_EXTRACT, st, 2);
     k_append_slice<<<device_sm_count(), kMT, 0, st>>>(d_sx, d_sy, (const long long*)d_agent_offset, agent, d_px, d_py, capacity,
@@ -1264,10 +1279,8 @@ size_t mapmerge_bounds_workspace_bytes(void) { return (size_t)1024 * 8 * 4 * siz
 
 int mapmerge_bounds(const double* d_px, const double* d_py, const int64_t* d_count, double* d_bounds, void* d_ws,
                     size_t ws_bytes, void* stream) {
-    if (!d_px || !d_py || !d_count || !d_bounds || !d_ws || ws_bytes < mapmerge_bounds_workspace_bytes()) {
-        set_last_error("mapmerge_bounds: bad arguments");
-        return OCCGRID_E_ARG;
-    }
+    if (!d_px || !d_py || !d_count || !d_bounds || !d_ws) { set_last_error("mapmerge_bounds: NULL pointer"); return OCCGRID_E_ARG; }
+    if (ws_bytes < mapmerge_bounds_workspace_bytes()) { set_last_error("mapmerge_bounds: workspace too small"); return OCCGRID_E_WORKSPACE; }
     cudaStream_t st = (cudaStream_t)stream;
     const int blocks = device_sm_count() * 8;
     ProfileScope ps(K_MERGE_BOUNDS, st, 2);
@@ -1335,9 +1348,14 @@ int mapmerge_voxel_downsample(const double* d_px, const double* d_py, const int6
                               double voxel, const double* d_bounds, uint64_t* d_bounds_enc, int64_t lattice_capacity_cells,
                               double* d_out_px, double* d_out_py, int64_t* d_out_count, int32_t* d_status,
                               void* d_ws, size_t ws_bytes, void* stream) {
-    if (!d_px || !d_py || !d_count || (!d_bounds && !d_bounds_enc) || !d_out_px || !d_out_py || !d_out_count || !d_status || !d_ws ||
-        !(voxel > 0.0) || lattice_capacity_cells <= 0 || point_capacity <= 0) {
-        set_last_error("mapmerge_voxel_downsample: bad arguments");
+    if (!d_px || !d_py || !d_count || (!d_bounds && !d_bounds_enc) || !d_out_px || !d_out_py || !d_out_count || !d_status || !d_ws) {
+        set_last_error("mapmerge_voxel_downsample: NULL pointer");
+        return OCCGRID_E_ARG;
+    }
+    if (!(voxel > 0.0)) { set_last_error("mapmerge_voxel_downsample: voxel %g must be > 0", voxel); return OCCGRID_E_ARG; }
+    if (lattice_capacity_cells <= 0 || point_capacity <= 0) {
+        set_last_error("mapmerge_voxel_downsample: capacity < 1 (lattice %lld cells, %lld points)", (long long)lattice_capacity_cells,
+                       (long long)point_capacity);
         return OCCGRID_E_ARG;
     }
     size_t off[9];
@@ -1401,6 +1419,18 @@ static bool chain_dims_ok(const int64_t* dims, int n_agents) {
            dims[0] * dims[1] < 0x7fffffffll && dims[2] < 0x7ffffff0ll && dims[3] < 0x7ffffff0ll;
 }
 
+// chain_dims_ok with a message naming what failed; false -> OCCGRID_E_ARG.
+static bool chain_dims_check(const char* fn, const int64_t* dims, int n_agents) {
+    if (!dims) { set_last_error("%s: NULL pointer (dims)", fn); return false; }
+    if (n_agents <= 0 || n_agents > 65535) { set_last_error("%s: n_agents %d outside 1..65535", fn, n_agents); return false; }
+    if (!chain_dims_ok(dims, n_agents)) {
+        set_last_error("%s: dims {%lld, %lld, %lld, %lld} out of range", fn, (long long)dims[0], (long long)dims[1],
+                       (long long)dims[2], (long long)dims[3]);
+        return false;
+    }
+    return true;
+}
+
 size_t mapmerge_chain_workspace_bytes(const int64_t* dims, int n_agents) {
     if (!chain_dims_ok(dims, n_agents)) return 0;
     return chain_layout(dims, n_agents, nullptr, nullptr);
@@ -1409,9 +1439,13 @@ size_t mapmerge_chain_workspace_bytes(const int64_t* dims, int n_agents) {
 int mapmerge_chain_init(void* d_chain, size_t chain_bytes, const int64_t* dims, int n_agents, const double* d_sx,
                         const double* d_sy, const int64_t* d_agent_offset, const int32_t* order_host, int n_order,
                         const double* d_px, const double* d_py, const int64_t* d_count, void* stream) {
-    if (!d_chain || !chain_dims_ok(dims, n_agents) || !d_sx || !d_sy || !d_agent_offset || !order_host || n_order < 0 ||
-        n_order > n_agents || !d_px || !d_py || !d_count) {
-        set_last_error("mapmerge_chain_init: bad arguments");
+    if (!d_chain || !d_sx || !d_sy || !d_agent_offset || !order_host || !d_px || !d_py || !d_count) {
+        set_last_error("mapmerge_chain_init: NULL pointer");
+        return OCCGRID_E_ARG;
+    }
+    if (!chain_dims_check("mapmerge_chain_init", dims, n_agents)) return OCCGRID_E_ARG;
+    if (n_order < 0 || n_order > n_agents) {
+        set_last_error("mapmerge_chain_init: n_order %d outside 0..n_agents", n_order);
         return OCCGRID_E_ARG;
     }
     if (chain_bytes < chain_layout(dims, n_agents, nullptr, nullptr)) { set_last_error("mapmerge_chain_init: workspace too small"); return OCCGRID_E_WORKSPACE; }
@@ -1439,11 +1473,15 @@ int mapmerge_chain_init(void* d_chain, size_t chain_bytes, const int64_t* dims, 
 int mapmerge_chain_run(void* d_chain, const int64_t* dims, int n_agents, int n_order, int n_callbacks, const double* d_sx,
                        const double* d_sy, const int64_t* d_agent_offset, double voxel, double* d_px, double* d_py,
                        int64_t capacity, int64_t* d_count, int32_t* d_status, void* stream) {
-    if (!d_chain || !chain_dims_ok(dims, n_agents) || n_order < 0 || n_order > n_agents || n_callbacks < 0 || !d_sx || !d_sy ||
-        !d_agent_offset || !(voxel > 0.0) || !d_px || !d_py || capacity > dims[2] || !d_count || !d_status) {
-        set_last_error("mapmerge_chain_run: bad arguments");
+    if (!d_chain || !d_sx || !d_sy || !d_agent_offset || !d_px || !d_py || !d_count || !d_status) {
+        set_last_error("mapmerge_chain_run: NULL pointer");
         return OCCGRID_E_ARG;
     }
+    if (!chain_dims_check("mapmerge_chain_run", dims, n_agents)) return OCCGRID_E_ARG;
+    if (n_order < 0 || n_order > n_agents) { set_last_error("mapmerge_chain_run: n_order %d outside 0..n_agents", n_order); return OCCGRID_E_ARG; }
+    if (n_callbacks < 0) { set_last_error("mapmerge_chain_run: n_callbacks %d < 0", n_callbacks); return OCCGRID_E_ARG; }
+    if (!(voxel > 0.0)) { set_last_error("mapmerge_chain_run: voxel %g must be > 0", voxel); return OCCGRID_E_ARG; }
+    if (capacity > dims[2]) { set_last_error("mapmerge_chain_run: capacity above dims[2]"); return OCCGRID_E_ARG; }
     if (n_callbacks == 0) return OCCGRID_OK;
     ChainArrays c;
     chain_layout(dims, n_agents, &c, d_chain);
@@ -1477,7 +1515,8 @@ int mapmerge_chain_run(void* d_chain, const int64_t* dims, int n_agents, int n_o
 
 // Synchronises the stream; state_out = {cursor, stalled}.
 int mapmerge_chain_poll(void* d_chain, const int64_t* dims, int n_agents, int32_t* state_out, void* stream) {
-    if (!d_chain || !chain_dims_ok(dims, n_agents) || !state_out) { set_last_error("mapmerge_chain_poll: bad arguments"); return OCCGRID_E_ARG; }
+    if (!d_chain || !state_out) { set_last_error("mapmerge_chain_poll: NULL pointer"); return OCCGRID_E_ARG; }
+    if (!chain_dims_check("mapmerge_chain_poll", dims, n_agents)) return OCCGRID_E_ARG;
     ChainArrays c;
     chain_layout(dims, n_agents, &c, d_chain);
     cudaStream_t st = (cudaStream_t)stream;
@@ -1492,7 +1531,8 @@ int mapmerge_chain_poll(void* d_chain, const int64_t* dims, int n_agents, int32_
 
 int mapmerge_chain_rebounds(void* d_chain, const int64_t* dims, int n_agents, const double* d_px, const double* d_py,
                             const int64_t* d_count, void* stream) {
-    if (!d_chain || !chain_dims_ok(dims, n_agents) || !d_px || !d_py || !d_count) { set_last_error("mapmerge_chain_rebounds: bad arguments"); return OCCGRID_E_ARG; }
+    if (!d_chain || !d_px || !d_py || !d_count) { set_last_error("mapmerge_chain_rebounds: NULL pointer"); return OCCGRID_E_ARG; }
+    if (!chain_dims_check("mapmerge_chain_rebounds", dims, n_agents)) return OCCGRID_E_ARG;
     ChainArrays c;
     chain_layout(dims, n_agents, &c, d_chain);
     cudaStream_t st = (cudaStream_t)stream;
@@ -1507,11 +1547,15 @@ int mapmerge_chain_rebuild(void* d_chain, const int64_t* dims, int n_agents, con
                            const int64_t* d_agent_offset, int agent, double voxel, double* d_px, double* d_py, int64_t capacity,
                            int64_t* d_count, double* d_out_px, double* d_out_py, int64_t* d_out_count, int32_t* d_status,
                            void* d_voxel_ws, size_t voxel_ws_bytes, int64_t lattice_capacity_cells, void* stream) {
-    if (!d_chain || !chain_dims_ok(dims, n_agents) || !d_sx || !d_sy || !d_agent_offset || agent < 0 || agent >= n_agents ||
-        !(voxel > 0.0) || !d_px || !d_py || capacity > dims[2] || !d_count || !d_out_px || !d_out_py || !d_out_count || !d_status) {
-        set_last_error("mapmerge_chain_rebuild: bad arguments");
+    if (!d_chain || !d_sx || !d_sy || !d_agent_offset || !d_px || !d_py || !d_count || !d_out_px || !d_out_py || !d_out_count ||
+        !d_status) {
+        set_last_error("mapmerge_chain_rebuild: NULL pointer");
         return OCCGRID_E_ARG;
     }
+    if (!chain_dims_check("mapmerge_chain_rebuild", dims, n_agents)) return OCCGRID_E_ARG;
+    if (agent < 0 || agent >= n_agents) { set_last_error("mapmerge_chain_rebuild: agent %d outside 0..n_agents-1", agent); return OCCGRID_E_ARG; }
+    if (!(voxel > 0.0)) { set_last_error("mapmerge_chain_rebuild: voxel %g must be > 0", voxel); return OCCGRID_E_ARG; }
+    if (capacity > dims[2]) { set_last_error("mapmerge_chain_rebuild: capacity above dims[2]"); return OCCGRID_E_ARG; }
     size_t off[9];
     if (!d_voxel_ws || lattice_capacity_cells < dims[0] * dims[1] || voxel_ws_bytes < voxel_layout(lattice_capacity_cells, dims[2], off)) {
         set_last_error("mapmerge_chain_rebuild: voxel workspace too small");
@@ -1537,10 +1581,12 @@ int mapmerge_chain_rebuild(void* d_chain, const int64_t* dims, int n_agents, con
 
 int mapmerge_rasterise(const double* d_px, const double* d_py, const int64_t* d_count, double res, const double* d_bounds,
                        int32_t width, int32_t height, int8_t* d_grid_out, void* stream) {
-    if (!d_px || !d_py || !d_count || !d_bounds || !d_grid_out || width <= 0 || height <= 0 || !(res > 0.0)) {
-        set_last_error("mapmerge_rasterise: bad arguments");
+    if (!d_px || !d_py || !d_count || !d_bounds || !d_grid_out) { set_last_error("mapmerge_rasterise: NULL pointer"); return OCCGRID_E_ARG; }
+    if (width <= 0 || height <= 0) {
+        set_last_error("mapmerge_rasterise: width x height %d x %d", (int)width, (int)height);
         return OCCGRID_E_ARG;
     }
+    if (!(res > 0.0)) { set_last_error("mapmerge_rasterise: res %g must be > 0", res); return OCCGRID_E_ARG; }
     cudaStream_t st = (cudaStream_t)stream;
     const long long n = (long long)width * height;
     ProfileScope ps(K_MERGE_RASTER, st, 2);
@@ -1551,7 +1597,8 @@ int mapmerge_rasterise(const double* d_px, const double* d_py, const int64_t* d_
 }
 
 int mapmerge_fuse_max(int8_t* d_dst, const int8_t* d_src, int64_t n, void* stream) {
-    if (!d_dst || !d_src || n < 0) { set_last_error("mapmerge_fuse_max: bad arguments"); return OCCGRID_E_ARG; }
+    if (!d_dst || !d_src) { set_last_error("mapmerge_fuse_max: NULL pointer"); return OCCGRID_E_ARG; }
+    if (n < 0) { set_last_error("mapmerge_fuse_max: n %lld < 0", (long long)n); return OCCGRID_E_ARG; }
     if (n == 0) return OCCGRID_OK;
     cudaStream_t st = (cudaStream_t)stream;
     ProfileScope ps(K_MERGE_FUSE, st);

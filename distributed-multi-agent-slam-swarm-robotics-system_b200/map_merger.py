@@ -341,7 +341,9 @@ class MapMerger:
 
     @staticmethod
     def _as_matrices(transforms, A):
-        """[A, 4, 4] float64 from None / [A, 4, 4] / [A, 3] (tx, ty, theta) / a list mixing both."""
+        """[A, 4, 4] float64 from None / [A, 4, 4] / [A, 3] (tx, ty, theta) / a list mixing both.
+        Always a new array: merge() writes the identity into the adopted agent's row, and the
+        caller passes the same transforms on to fuse_occupancy / register_maps."""
         if transforms is None:
             return np.tile(np.eye(4), (A, 1, 1))
         try:
@@ -349,7 +351,7 @@ class MapMerger:
         except ValueError:
             t = None
         if t is not None and t.shape == (A, 4, 4):
-            return np.ascontiguousarray(t)
+            return np.array(t, np.float64, order='C')
         out = np.tile(np.eye(4), (A, 1, 1))
         for a in range(A):
             T = transforms[a]

@@ -343,7 +343,15 @@ int mapmerge_extract_transform(const int8_t* d_grid, int32_t width, int32_t heig
  * d_agent_offset[a] = start of agent a's slice (d_agent_offset[A] = total).  d_xforms is scratch
  * (A * 96 bytes); the workspace must be the one _count filled, untouched: it carries the block
  * counts and one occupancy bit per cell, so _write does not read the grids again.  The sequential chain appends
- * slice a with mapmerge_append_slice when callback a's turn comes (:59). */
+ * slice a with mapmerge_append_slice when callback a's turn comes (:59).
+ * Argument errors of the older merge entry points (this one, mapmerge_count_occupied,
+ * mapmerge_append_slice, mapmerge_bounds, mapmerge_voxel_downsample, mapmerge_chain_*,
+ * mapmerge_rasterise, mapmerge_fuse_max) return OCCGRID_E_ARG before anything is launched, with the
+ * message key word in quotes: a "NULL pointer", "n_agents" outside 1..65 535, "width x height"
+ * below 1, a "res" or "voxel" that is not > 0 (NaN included), a negative "n_cells" / "n", an
+ * "agent" out of range, "dims" out of range, "n_order" outside 0..n_agents, "n_callbacks" < 0, a
+ * "capacity" below 1 (voxel filter) or above dims[2] (chain), an "order entry" out of range.  A
+ * workspace below its *_workspace_bytes returns OCCGRID_E_WORKSPACE ("workspace"). */
 size_t mapmerge_extract_batch_workspace_bytes(int64_t n_cells, int n_agents);
 int mapmerge_extract_batch_count(const int8_t* const* d_grids, int n_agents, int32_t width, int32_t height,
                                  int64_t* d_agent_total, void* d_ws, size_t ws_bytes,
