@@ -129,6 +129,8 @@ class OccupancyGrid:
         self._tab_cache = None
         self._fr = None
         self._ws_assign = None
+        self._ws_edt = None
+        self._nav = None
         self._fa_sizes = {'pool': 4096, 'kmax': 1024}
         if not lazy_workspace:                  # (the multi-GPU band step brings its own workspace)
             self._ensure_workspace(int(max_batch))
@@ -597,7 +599,7 @@ class OccupancyGrid:
                 self._ws_assign = torch.empty(nb, dtype=torch.uint8, device=self.device)
         return self._ws_assign
 
-    def assign_frontiers(self, robot_xy, min_cluster=FRONTIER_MIN_CLUSTER):
+    def assign_frontiers(self, robot_xy, min_cluster=FRONTIER_MIN_CLUSTER, robot_radius=None):
         """EXTENSION: one exploration target per robot by geodesic distance over the known free
         space (``occgrid_frontier_assign`` in include/occgrid_b200.h gives the exact rules).
 
@@ -609,7 +611,13 @@ class OccupancyGrid:
         order, -1 for none) at path length ``cost[a]`` cells, reaching it first at cell ``goal[a]``;
         ``target_xy[a]`` is that cluster's centroid (NaN for none) and ``costs[a, k]`` robot a's
         path length to cluster k (-1 when unreachable).  The tile pool grows until it holds every
-        field."""
+        field.
+
+        robot_radius  None (a robot is a point) or metres >= 0: the stencil and the clustering still
+                  run on ``grid_tensor``, and the paths run over ``navigation_grid(robot_radius,
+                  robot_xy)``, so they keep that clearance from every obstacle except inside the
+                  robots' own footprints."""
+        max_d2 = None if robot_radius is None else self._max_d2(robot_radius, 'assign_frontiers')
         d_xy = self._robot_positions(robot_xy, 'assign_frontiers')
         A = d_xy.shape[0]
         n_tiles = ((self.size + 63) // 64) ** 2
@@ -630,8 +638,9 @@ class OccupancyGrid:
                 hdr = torch.zeros(8, dtype=torch.int64, device=dev)     # count, frontier status, n_clusters, status, stats[3]
                 status = torch.zeros(1, dtype=torch.int32, device=dev)
                 self._launch_clusters(f, min_cluster)
+                paths = self.grid_tensor if max_d2 is None else self._launch_inflate(max_d2, d_xy)
                 rc = self._lib.occgrid_frontier_assign(
-                    self.grid_tensor.data_ptr(), self.size, self.size, self.ox, self.oy, self.res, d_xy.data_ptr(), A,
+                    paths.data_ptr(), self.size, self.size, self.ox, self.oy, self.res, d_xy.data_ptr(), A,
                     f['xy'].data_ptr(), f['count'].data_ptr(), f['label'].data_ptr(), f['root'].data_ptr(), f['cent'].data_ptr(),
                     f['ncl'].data_ptr(), kmax, pool, out['cluster'].data_ptr(), out['cost'].data_ptr(), out['goal'].data_ptr(),
                     out['target_xy'].data_ptr(), out['costs'].data_ptr(), status.data_ptr(), hdr[4:7].data_ptr(),
@@ -665,11 +674,14 @@ class OccupancyGrid:
                                       {'frontier_cells': count, 'clusters': ncl, 'rounds': rounds, 'items': items,
                                        'tile_slots': slots, 'tile_pool': pool})
 
-    def geodesic_distance(self, robot_xy, to_host=True):
+    def geodesic_distance(self, robot_xy, to_host=True, robot_radius=None):
         """EXTENSION: the geodesic field of one robot at world position ``robot_xy`` = (x, y):
         int32 [size, size] indexed [gy, gx], the 4-connected path length in cells over FREE cells
         from the robot's cell (0 there whatever its value), -1 where unreachable or when the robot
-        is outside the grid.  For navigation: descend the field from a goal cell to the robot."""
+        is outside the grid.  For navigation: descend the field from a goal cell to the robot.
+        With ``robot_radius`` (metres >= 0) the field runs over ``navigation_grid(robot_radius,
+        robot_xy)``: a robot of that radius can follow it."""
+        max_d2 = None if robot_radius is None else self._max_d2(robot_radius, 'geodesic_distance')
         xy = np.asarray(robot_xy, np.float64)
         if xy.size != 2:
             raise ValueError(f'geodesic_distance: robot_xy must be one (x, y) world position, got shape {xy.shape}')
@@ -679,13 +691,87 @@ class OccupancyGrid:
         with torch.cuda.device(self.device):
             field = torch.empty((self.size, self.size), dtype=torch.int32, device=self.device)
             status = torch.zeros(1, dtype=torch.int32, device=self.device)
-            rc = self._lib.occgrid_geodesic_field(self.grid_tensor.data_ptr(), self.size, self.size, self.ox, self.oy, self.res,
+            paths = self.grid_tensor if max_d2 is None else self._launch_inflate(max_d2, d_xy)
+            rc = self._lib.occgrid_geodesic_field(paths.data_ptr(), self.size, self.size, self.ox, self.oy, self.res,
                                                   d_xy.data_ptr(), pool, field.data_ptr(), status.data_ptr(), None,
                                                   ws.data_ptr(), ws.numel(), self._stream())
             _native.check(rc, 'occgrid_geodesic_field')
             if int(status.item()) != 0:
                 raise OccGridError(f'occgrid_geodesic_field: status {int(status.item())} (worklist failed)')
         return field.cpu().numpy() if to_host else field
+
+    # ---- obstacle clearance (EXTENSION) -------------------------------------------------------
+    def _max_d2(self, robot_radius, who):
+        """The one conversion of a robot radius: max_d2 = floor((robot_radius / res) ** 2) in fp64,
+        so a cell is blocked when an obstacle's centre lies within robot_radius of its centre."""
+        r = float(robot_radius)
+        if not (math.isfinite(r) and r >= 0.0):
+            raise ValueError(f'{who}: robot_radius must be finite and >= 0, got {robot_radius!r}')
+        q = r / self.res
+        q = q * q                                              # (r / res) ** 2, inf rather than OverflowError
+        return (1 << 62) if q >= 2.0 ** 62 else math.floor(q)   # past 2 * 32767^2 every value blocks the same
+
+    def _edt_workspace(self):
+        if self.window != (0, 0, self.size, self.size):
+            raise OccGridError('the distance field needs the whole grid (not a window of it)')
+        nb = self._lib.occgrid_distance_field_workspace_bytes(self.size, self.size)
+        if nb == 0:
+            raise OccGridError('occgrid_distance_field_workspace_bytes: ' + _native.last_error())
+        if self._ws_edt is None or self._ws_edt.numel() < nb:
+            self._ws_edt = None
+            with torch.cuda.device(self.device):
+                self._ws_edt = torch.empty(nb, dtype=torch.uint8, device=self.device)
+        return self._ws_edt
+
+    def _launch_inflate(self, max_d2, d_xy, out=None):
+        """Enqueues occgrid_inflate of grid_tensor with the robots d_xy ([A, 2] on the device or None)
+        into ``out``, by default the cached navigation buffer; returns it."""
+        ws = self._edt_workspace()
+        with torch.cuda.device(self.device):
+            if out is None:
+                if self._nav is None:
+                    self._nav = torch.empty((self.size, self.size), dtype=torch.int8, device=self.device)
+                out = self._nav
+            A = 0 if d_xy is None else int(d_xy.shape[0])
+            rc = self._lib.occgrid_inflate(self.grid_tensor.data_ptr(), self.size, self.size, self.ox, self.oy, self.res,
+                                           int(max_d2), d_xy.data_ptr() if A else None, A, out.data_ptr(),
+                                           ws.data_ptr(), ws.numel(), self._stream())
+            _native.check(rc, 'occgrid_inflate')
+        return out
+
+    def distance_field(self, to_host=True):
+        """EXTENSION: the exact squared Euclidean distance from every cell to the nearest obstacle
+        (a cell > 50), int32 [size, size] indexed [gy, gx], in cells between cell centres: 0 on
+        obstacles, and -1 everywhere when the grid has no obstacle.  The clearance in metres is
+        ``sqrt(d2) * res``."""
+        ws = self._edt_workspace()
+        with torch.cuda.device(self.device):
+            d2 = torch.empty((self.size, self.size), dtype=torch.int32, device=self.device)
+            rc = self._lib.occgrid_distance_field(self.grid_tensor.data_ptr(), self.size, self.size, d2.data_ptr(),
+                                                  ws.data_ptr(), ws.numel(), self._stream())
+            _native.check(rc, 'occgrid_distance_field')
+        return d2.cpu().numpy() if to_host else d2
+
+    def navigation_grid(self, robot_radius, robot_xy=None, to_host=True):
+        """EXTENSION: the grid a robot of ``robot_radius`` metres can plan on, int8 [size, size]:
+        every FREE cell whose centre lies within robot_radius of an obstacle's centre becomes
+        OCCUPIED (max_d2 = floor((robot_radius / res) ** 2) cells^2), except in the footprints of the
+        robots at ``robot_xy`` ([A, 2] world metres, 0 <= A <= 65 535, or None), so that a robot
+        standing closer than its radius to a wall can still leave.  Other cells keep their value."""
+        max_d2 = self._max_d2(robot_radius, 'navigation_grid')
+        d_xy = None
+        if robot_xy is not None:
+            xy = np.ascontiguousarray(np.asarray(robot_xy, dtype=np.float64))
+            if xy.ndim != 2 or xy.shape[1] != 2 or xy.shape[0] > MAX_ASSIGN_ROBOTS:
+                raise ValueError(f'navigation_grid: robot_xy must be [A, 2] world positions with A <= {MAX_ASSIGN_ROBOTS}, '
+                                 f'got shape {xy.shape}')
+            if xy.shape[0]:
+                with torch.cuda.device(self.device):
+                    d_xy = torch.from_numpy(xy).to(self.device)
+        with torch.cuda.device(self.device):
+            out = torch.empty((self.size, self.size), dtype=torch.int8, device=self.device)
+        self._launch_inflate(max_d2, d_xy, out)
+        return out.cpu().numpy() if to_host else out
 
     # ---- overlay render (:492-527) — SURVEY §8 row f4 -----------------------------------------
     def render_overlay(self, width=1000, height=800, scale=100.0, offset_x=None, offset_y=None,
@@ -849,6 +935,8 @@ class AgentGrids(OccupancyGrid):
     frontier_centroids = _single_map_only('frontier_centroids')
     assign_frontiers = _single_map_only('assign_frontiers')
     geodesic_distance = _single_map_only('geodesic_distance')
+    distance_field = _single_map_only('distance_field')
+    navigation_grid = _single_map_only('navigation_grid')
     render_overlay = _single_map_only('render_overlay')
 
 

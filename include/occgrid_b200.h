@@ -613,7 +613,9 @@ int occgrid_frontier_clusters(const int32_t* d_xy, const int64_t* d_count, int64
  * "overflows size_t" (the [A][n_tiles] slot tables); OCCGRID_E_WORKSPACE for ws_bytes below
  * occgrid_frontier_assign_workspace_bytes (which returns 0 for the same argument errors).
  * Stream-ordered: the robots are read on the device, and the worklist runs as one cooperative
- * launch with no host round trip. */
+ * launch with no host round trip.
+ * d_grid may be a navigation grid from occgrid_inflate of the grid the clusters came from; the costs
+ * are then path lengths over its FREE cells. */
 #define OCCGRID_ASSIGN_POOL_FULL     1
 #define OCCGRID_ASSIGN_TIMEOUT       2
 #define OCCGRID_ASSIGN_CLUSTERS_FULL 4
@@ -636,6 +638,36 @@ int occgrid_frontier_assign(const int8_t* d_grid, int32_t width, int32_t height,
 int occgrid_geodesic_field(const int8_t* d_grid, int32_t width, int32_t height, double ox, double oy,
                            double res, const double* d_robot_xy, int64_t tile_pool, int32_t* d_field,
                            int32_t* d_status, int64_t* d_stats, void* d_ws, size_t ws_bytes, void* stream);
+
+/* EXTENSION (no reference counterpart): obstacle clearance (DESIGN §6g).
+ * occgrid_distance_field: the exact squared Euclidean distance transform of a grid int8 [H][W]
+ * ([gy][gx]), 1 <= W, H <= 32 768.  Obstacles are the cells > 50 (the occupied rule of grid_to_pcd).
+ * d_d2 int32 [H][W] receives d2[y][x] = min over obstacles (x', y') of (x - x')^2 + (y - y')^2, the
+ * squared distance between cell centres in cells (0 on obstacles, at most 2 * 32 767^2, which fits
+ * int32), or -1 in every cell when the grid has no obstacle.  Integer arithmetic, no atomics: the
+ * result depends on the input alone.
+ * occgrid_inflate: the navigation grid of a robot radius.  d_out int8 [H][W] (must not overlap
+ * d_grid) is OCCUPIED (100) where grid[c] == 0 (FREE), 0 <= d2[c] <= max_d2 and c lies in no robot's
+ * footprint, else grid[c].  Robot a's footprint is the cells (x, y) with (x - rx)^2 + (y - ry)^2 <=
+ * max_d2 around its cell (rx, ry) = (int((x_a - ox) / res), int((y_a - oy) / res)) (fp64 division,
+ * truncation, as occgrid_frontier_assign); a robot outside the grid or at a non-finite position has no
+ * footprint.  d_robot_xy double [A][2] world metres, 0 <= A <= 65 535 (NULL allowed when A == 0).  The
+ * footprint lets a robot that stands closer than its radius to a wall leave it.  The EDT is computed
+ * in the workspace.
+ * Both take one workspace of occgrid_distance_field_workspace_bytes(W, H) bytes; with
+ * n_bands = ceil(H / 32) and a(v) = v rounded up to a multiple of 256 it is exactly
+ *   a(4 W n_bands) + a(8 W n_bands) + a(4 W H) + a(8 W H)
+ * (band masks, band links, the inflation's d2, the envelope stacks).
+ * OCCGRID_E_ARG (message key word in quotes) for a "NULL pointer" (d_robot_xy too when A > 0), a
+ * "width x height" side outside 1..32 768, "max_d2" < 0, "n_robots" outside 0..65 535 and a
+ * "resolution" that is not finite and > 0; OCCGRID_E_WORKSPACE for a short workspace (the query
+ * returns 0 for a bad side).  Stream-ordered, no host synchronisation. */
+size_t occgrid_distance_field_workspace_bytes(int32_t width, int32_t height);
+int occgrid_distance_field(const int8_t* d_grid, int32_t width, int32_t height,
+                           int32_t* d_d2, void* d_ws, size_t ws_bytes, void* stream);
+int occgrid_inflate(const int8_t* d_grid, int32_t width, int32_t height, double ox, double oy, double res,
+                    int64_t max_d2, const double* d_robot_xy /* [A][2] or NULL when A == 0 */, int32_t n_robots,
+                    int8_t* d_out, void* d_ws, size_t ws_bytes, void* stream);
 
 /* Tuning knob of the TILED strategy: cap the persistent raycast CTAs per SM (0 = as many as fit,
  * the default).  A pipelined multi-GPU ingest lowers it to 2 so that the routing kernel of the
