@@ -1,5 +1,6 @@
 // Device building blocks of the merge, ICP, frontier and route kernels: a block-wide scan, a
-// single-CTA scan of per-block counts and a grid barrier for cooperative launches.
+// single-CTA scan of per-block counts, a grid barrier for cooperative launches, and the 1-D bulk
+// copy (TMA) into shared memory with its mbarrier.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -115,6 +116,31 @@ __device__ __forceinline__ bool grid_barrier(unsigned int* bar, unsigned int& ta
 
 __device__ __forceinline__ bool grid_barrier(unsigned int* bar, unsigned int& target, int* abort_flag) {
     return grid_barrier(bar, target, abort_flag, nullptr, [] { return 0; });
+}
+
+// 1-D bulk copy (cp.async.bulk, the TMA unit) of `bytes` (a multiple of 16, both addresses 16-byte
+// aligned) into shared memory, completing on an mbarrier: one elected thread arms the barrier with
+// the byte count and issues the copy; the consumers wait on the barrier's phase parity.
+__device__ __forceinline__ unsigned int smem_u32(const void* p) { return (unsigned int)__cvta_generic_to_shared(p); }
+
+__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned int count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
+}
+__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned int bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned int parity) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "WAIT_%=:\n\t"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
+        "@p bra DONE_%=;\n\t"
+        "bra WAIT_%=;\n\t"
+        "DONE_%=:\n\t}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
+}
+__device__ __forceinline__ void bulk_load(void* smem_dst, const void* gmem_src, unsigned int bytes, unsigned long long* bar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 ::"r"(smem_u32(smem_dst)), "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
 
 }  // namespace occ

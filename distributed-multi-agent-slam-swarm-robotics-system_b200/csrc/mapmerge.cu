@@ -221,28 +221,6 @@ constexpr int kScanStages = 4;
 constexpr int kScanCtasPerSm = 3;            // 3 x 4 x 16 KiB = 192 KiB of bulk loads in flight per SM
 constexpr int kScanStageBytes = kChunk;                    // 16 KiB = one chunk of the existing mask layout
 
-__device__ __forceinline__ unsigned int smem_u32(const void* p) { return (unsigned int)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned int bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned int parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "WAIT_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra DONE_%=;\n\t"
-        "bra WAIT_%=;\n\t"
-        "DONE_%=:\n\t}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_load(void* smem_dst, const void* gmem_src, unsigned int bytes, unsigned long long* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(smem_dst)), "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-
 // 16 int8 cells (one uint4 from shared memory) -> 16 occupancy bits.
 __device__ __forceinline__ unsigned int occupied_bits16(uint4 v) {
     const unsigned int w[4] = {v.x, v.y, v.z, v.w};

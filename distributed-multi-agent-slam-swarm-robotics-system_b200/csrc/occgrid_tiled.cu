@@ -12,9 +12,10 @@
 // home tile grown by R on every side.  Binning therefore needs only the robot cell — no
 // trigonometry, one record per packet, no duplicates:
 //
-//   k_home_bin      thread/packet: decode (:828-843), pose correction (:851-857), robot cell
-//                   (:142) -> 48-byte pose record (packet order) + packets per home tile, and each
-//                   CTA's packet indices grouped by tile with its rank inside every tile's bin
+//   k_home_bin      persistent CTAs streaming 2048-packet segments through a bulk-copy ring, thread
+//                   per packet: decode (:828-843), pose correction (:851-857), robot cell (:142) ->
+//                   48-byte pose record (packet order) + packets per home tile, and each segment's
+//                   packet indices grouped by tile with its rank inside every tile's bin
 //   k_tile_plan     one CTA over the active tiles (listed by the bin pass): exclusive scan of
 //                   their counts -> bin offsets, (tile, chunk) work items of <= kChunkPk packets
 //   k_place_runs    thread/packet: copy the grouped indices to their tile's bin
@@ -44,7 +45,7 @@ constexpr int kMaxWindowBytes = 100 * 1024;   // smem window budget (two CTAs pe
 struct TilePlanHeader {
     unsigned int n_items, n_active, total_records, work_counter, resolve_counter, overflow;
     unsigned int active_count;   // tiles appended to the active list by the count pass of the current call
-    unsigned int pad;
+    unsigned int bin_counter;    // segments claimed by the packet bin pass of the current call
 };
 
 // Home tile of a corrected pose, or -1 when no beam of the packet can reach the window.
@@ -115,11 +116,11 @@ __device__ __forceinline__ void reserve_tile_ranges(const unsigned int* s_keys, 
         if (key[j] != kEmpty) s_vals[j * kTT + threadIdx.x] = off[j] + base[j];
 }
 
-// Packet path: the bin pass does the whole binning but the final placement.  Binning CTA b owns
-// the segment [b * kPkPerCta, (b + 1) * kPkPerCta) of the batch and of the arrays below:
+// Packet path: the bin pass does the whole binning but the final placement.  Segment s of the
+// batch is [s * kPkPerCta, (s + 1) * kPkPerCta), and so are its slices of the arrays below:
 //   local_bins  its accepted packets grouped by home tile: (run << 16) | packet index in the segment
 //   runs        one per distinct tile of the segment, in local_bins order: (tile, tile_rank - local
-//               begin), where tile_rank is the CTA's position inside the tile's bin (the return
+//               begin), where tile_rank is the segment's position inside the tile's bin (the return
 //               value of its one atomic on tile_count) and local begin the run's first position
 //   seg_count   number of local_bins entries
 // Once k_tile_plan has the bin offsets, k_place_runs moves entry j of run r to
@@ -127,157 +128,208 @@ __device__ __forceinline__ void reserve_tile_ranges(const unsigned int* s_keys, 
 // every binned packet is stored in packet order for the raycast: decoding the 42-byte wire record
 // again in the raycast instead was measured slower (DESIGN §3).
 //
+// The pass is a stream: persistent CTAs take segment blockIdx.x, then claim one segment after the
+// other from hdr->bin_counter, and one thread keeps a ring of kBinStages sub-batches (kTT wire
+// records each) in flight with bulk copies, across segment boundaries, so the loads of the next
+// sub-batches (and of the next segment while the current one's per-tile atomics, scan and runs are
+// done) overlap the decode.
+//
 // kMaps (occgrid_integrate_packets_agent_maps): the map is folded into the tile KEY, (agent - 1) *
 // n_tiles + home tile.  Everything below and the plan and placement passes work on keys unchanged.
-constexpr size_t kBinSmem = (size_t)kTT * kMaxRecStride + 2 * kHash * sizeof(unsigned int) + kPkPerCta * sizeof(unsigned short);
+constexpr int kBinStages = 3;           // 3 x 10.5 KB of 42-byte records: with the hash, 3 CTAs/SM
+constexpr int kSmemAgents = 256;        // agent-offset rows staged in shared memory (the wire id is one byte)
 constexpr unsigned int kNoSlot = 0xffffu;
 
+static size_t bin_smem_bytes(int stride) {
+    return (size_t)kBinStages * kTT * stride + 2 * kHash * sizeof(unsigned int) + kPkPerCta * sizeof(unsigned short);
+}
+
 template <bool kMaps = false>
-__global__ void __launch_bounds__(kTT)
+__global__ void __launch_bounds__(kTT, 3)
 k_home_bin(Geom g, TileGeom tg, const uint8_t* __restrict__ pkts, long long n, int stride,
            const int32_t* __restrict__ agent_idx, const double* __restrict__ drift,
            const double* __restrict__ agent_off, int n_agents,
            unsigned int* __restrict__ tile_count, PoseRec* __restrict__ recs, unsigned int* __restrict__ local_bins, uint2* __restrict__ runs,
            unsigned int* __restrict__ seg_count, unsigned int* __restrict__ active, TilePlanHeader* __restrict__ hdr,
            uint64_t* counters) {
-    extern __shared__ __align__(16) uint8_t s_bin[];                                  // kBinSmem
-    uint8_t* const s_rec = s_bin;                                                     // staged records, later the local bin list
-    unsigned int* const s_keys = reinterpret_cast<unsigned int*>(s_bin + kTT * kMaxRecStride);
+    extern __shared__ __align__(128) uint8_t s_bin[];                                 // bin_smem_bytes(stride)
+    const int stage_bytes = kTT * stride;                                             // a multiple of 16
+    uint8_t* const s_stage = s_bin;                                                   // kBinStages sub-batches of wire records
+    unsigned int* const s_keys = reinterpret_cast<unsigned int*>(s_bin + (size_t)kBinStages * stage_bytes);
     unsigned int* const s_vals = s_keys + kHash;
     unsigned short* const s_slot = reinterpret_cast<unsigned short*>(s_vals + kHash);   // hash slot of every packet, or kNoSlot
+    __shared__ __align__(8) unsigned long long s_full[kBinStages];
+    __shared__ double s_off[2 * kSmemAgents];
     __shared__ unsigned int s_wsum[kTT / 32];
-    for (int i = threadIdx.x; i < kHash; i += kTT) { s_keys[i] = kEmpty; s_vals[i] = 0u; }
-    unsigned long long c[OCCGRID_C_HITS + 1] = {};
-    const long long cta_first = (long long)blockIdx.x * kPkPerCta;
-    // Software-pipelined staging: the 16-byte loads of sub-batch s+1 are in flight while
-    // sub-batch s is decoded out of shared memory.
-    constexpr int kVec = (kTT * kMaxRecStride / 16 + kTT - 1) / kTT;      // uint4 per thread per sub-batch (<= 4)
-    uint4 pre[kVec];
-    auto prefetch = [&](int sub) {
-        const long long first = cta_first + (long long)sub * kTT;
-        const long long left = n - first;
-        const size_t bytes = left <= 0 ? 0 : (size_t)min((long long)kTT, left) * stride;
-        const uint4* s4 = reinterpret_cast<const uint4*>(pkts + (size_t)first * stride);
-#pragma unroll
-        for (int j = 0; j < kVec; ++j) {
-            const size_t i = (size_t)j * kTT + threadIdx.x;
-            pre[j] = (i * 16 + 16 <= bytes) ? __ldg(s4 + i) : make_uint4(0u, 0u, 0u, 0u);
+    const long long n_segs = (n + kPkPerCta - 1) / kPkPerCta;
+    // The agent-offset table from shared memory keeps a dependent global load off every packet's
+    // decode; the values and the arithmetic of decode_packet are the same.
+    const double* off_tab = agent_off;
+    if (n_agents < kSmemAgents) {
+        for (int i = threadIdx.x; i < 2 * (n_agents + 1); i += kTT) s_off[i] = agent_off[i];
+        off_tab = s_off;
+    }
+    // Sub-batch i of this CTA: sub-batch i % kSub of its segment number q = i / kSub.  Thread 0
+    // claims segment q + 1 when it first needs it (for the ring, or at the end of segment q) and
+    // publishes it in s_seg[(q + 1) & 1].  Claims only grow, so only the batch's last segment can be
+    // short, and it is the last one of its CTA.
+    // (n < 2^29: segment and sub-batch numbers fit in 32 bits)
+    __shared__ int s_seg[2];
+    int claimed = blockIdx.x;                                                         // thread 0: segment number claimed_q
+    int claimed_q = 0;
+    auto seg_of = [&](int q) {                                                        // thread 0 only; q <= claimed_q + 1
+        if (q > claimed_q) {
+            claimed = (int)(gridDim.x + atomicAdd(&hdr->bin_counter, 1u));
+            claimed_q = q;
+            s_seg[q & 1] = claimed;
         }
+        return claimed;
     };
-    const bool vec_ok = (reinterpret_cast<uintptr_t>(pkts) & 15) == 0 && ((kTT * stride) & 15) == 0;
-    if (vec_ok) prefetch(0);
-    for (int sub = 0; sub < kSub; ++sub) {
-        const long long first = cta_first + (long long)sub * kTT;
-        if (first >= n) break;
-        const int count = (int)min((long long)kTT, n - first);
-        __syncthreads();
-        if (vec_ok) {
-            const size_t bytes = (size_t)count * stride;
-            uint4* d4 = reinterpret_cast<uint4*>(s_rec);
-#pragma unroll
-            for (int j = 0; j < kVec; ++j) {
-                const size_t i = (size_t)j * kTT + threadIdx.x;
-                if (i * 16 + 16 <= bytes) d4[i] = pre[j];
-            }
-            for (size_t i = (bytes / 16) * 16 + threadIdx.x; i < bytes; i += kTT) s_rec[i] = __ldg(pkts + (size_t)first * stride + i);
-            if (sub + 1 < kSub) prefetch(sub + 1);
-        } else {
-            stage_records(pkts + (size_t)first * stride, (size_t)count * stride, s_rec);
-        }
-        __syncthreads();
-        if ((int)threadIdx.x < count) {
-            const long long k = first + threadIdx.x;
-            double rx, ry, ryaw;
-            float dist[4];
-            c[OCCGRID_C_PACKETS] += 1;
-            unsigned int slot = kNoSlot;
-            int agent = 1;
-            const int st = decode_packet(s_rec + threadIdx.x * stride, k, agent_idx, drift, agent_off, n_agents, &rx, &ry, &ryaw, dist,
-                                         kMaps ? &agent : nullptr);
-            if (st == PKT_DROPPED) c[OCCGRID_C_DROPPED] += 1;
-            else if (st == PKT_BAD_POSE) c[OCCGRID_C_BAD_POSE] += 1;
-            else {
-                c[OCCGRID_C_ACCEPTED] += 1;
-                c[OCCGRID_C_BEAMS] += 4;
-#pragma unroll
-                for (int s = 0; s < 4; ++s) {
-                    const double d = (double)dist[s];
-                    c[OCCGRID_C_HITS] += (OCC_MIN_DIST_M < d && d <= OCC_MAX_DIST_M) ? 1 : 0;     // :888
-                }
-                int tile = home_tile(g, tg, rx, ry);
-                if (kMaps && tile >= 0) tile += (agent - 1) * tg.n_tiles;
-                if (tile >= 0) {
-                    slot = (unsigned int)hash_insert(s_keys, (unsigned int)tile);
-                    atomicAdd(&s_vals[slot], 1u);
-                    PoseRec r;
-                    r.rx = rx; r.ry = ry; r.yaw = (float)ryaw;      // ryaw came from an fp32 field: exact
-                    r.d[0] = dist[0]; r.d[1] = dist[1]; r.d[2] = dist[2]; r.d[3] = dist[3];
-                    r.k = (unsigned int)k;
-                    r.tile = tile; r.pad = 0;
-                    recs[k] = r;                                    // packet order: coalesced 48-byte stores
-                }
-            }
-            s_slot[sub * kTT + threadIdx.x] = (unsigned short)slot;
-        }
+    const bool bulk_ok = (reinterpret_cast<uintptr_t>(pkts) & 15) == 0;
+    auto issue = [&](int i) {                                                         // thread 0 only
+        const long long seg = seg_of(i / kSub);
+        const long long first = seg * kPkPerCta + (i % kSub) * kTT;
+        if (seg >= n_segs || first >= n) return;
+        const unsigned int bytes = (unsigned int)(min((long long)kTT, n - first) * stride) & ~15u;   // >= 16: stride >= 41
+        const int st = (int)(i % kBinStages);
+        mbar_expect_tx(&s_full[st], bytes);
+        bulk_load(s_stage + (size_t)st * stage_bytes, pkts + (size_t)first * stride, bytes, &s_full[st]);
+    };
+    if (threadIdx.x == 0) {
+        s_seg[0] = blockIdx.x;
+        for (int s = 0; s < kBinStages; ++s) mbar_init(&s_full[s], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     }
     __syncthreads();
-    // One global atomic per distinct tile, as in flush_tile_counts; its return value is this CTA's
-    // rank inside the tile's bin.
-    unsigned int key[kHashPerThread], rank[kHashPerThread];
-#pragma unroll
-    for (int j = 0; j < kHashPerThread; ++j) {
-        const int i = j * kTT + threadIdx.x;
-        key[j] = s_keys[i];
-        rank[j] = 0u;
-        if (key[j] != kEmpty) rank[j] = atomicAdd(&tile_count[key[j]], s_vals[i]);
-    }
-    // Exclusive scan of (count | 1 << 16) over the occupied slots in (thread, j) order: the low half
-    // is the slot's first local position, the high half its run index (both < kPkPerCta).  An empty
-    // slot has count 0.
+    if (threadIdx.x == 0 && bulk_ok)
+        for (int s = 0; s < kBinStages; ++s) issue(s);
+    unsigned int c[OCCGRID_C_HITS + 1] = {};      // per thread: <= 4 * 2^29 / kTT beams, 32 bits suffice
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    unsigned int mine = 0u;
+    int i = 0;                                                                        // this CTA's sub-batch sequence
+    for (int q = 0;; ++q) {
+        const long long seg = s_seg[q & 1];
+        if (seg >= n_segs) break;                                                     // uniform: read after a barrier
+        const size_t seg0 = (size_t)seg * kPkPerCta;
+        for (int h = threadIdx.x; h < kHash; h += kTT) { s_keys[h] = kEmpty; s_vals[h] = 0u; }
+        __syncthreads();
+        for (int sub = 0; sub < kSub; ++sub, ++i) {
+            const long long first = (long long)seg0 + (long long)sub * kTT;
+            if (first >= n) break;
+            const int count = (int)min((long long)kTT, n - first);
+            const int st = (int)(i % kBinStages);
+            uint8_t* const s_rec = s_stage + (size_t)st * stage_bytes;
+            const size_t bytes = (size_t)count * stride;
+            if (bulk_ok) {
+                mbar_wait(&s_full[st], (unsigned int)((i / kBinStages) & 1));
+                const size_t done = bytes & ~(size_t)15;                              // a short last sub-batch: < 16 bytes left
+                if (done < bytes) {
+                    if (threadIdx.x < bytes - done) s_rec[done + threadIdx.x] = __ldg(pkts + (size_t)first * stride + done + threadIdx.x);
+                    __syncthreads();
+                }
+            } else {
+                stage_records(pkts + (size_t)first * stride, bytes, s_rec);
+                __syncthreads();
+            }
+            if ((int)threadIdx.x < count) {
+                const long long k = first + threadIdx.x;
+                double rx, ry, ryaw;
+                float dist[4];
+                c[OCCGRID_C_PACKETS] += 1;
+                unsigned int slot = kNoSlot;
+                int agent = 1;
+                const int st_pk = decode_packet(s_rec + threadIdx.x * stride, k, agent_idx, drift, off_tab, n_agents, &rx, &ry, &ryaw, dist,
+                                                kMaps ? &agent : nullptr);
+                if (st_pk == PKT_DROPPED) c[OCCGRID_C_DROPPED] += 1;
+                else if (st_pk == PKT_BAD_POSE) c[OCCGRID_C_BAD_POSE] += 1;
+                else {
+                    c[OCCGRID_C_ACCEPTED] += 1;
+                    c[OCCGRID_C_BEAMS] += 4;
 #pragma unroll
-    for (int j = 0; j < kHashPerThread; ++j) mine += key[j] != kEmpty ? s_vals[j * kTT + threadIdx.x] + 0x10000u : 0u;
-    unsigned int inc = mine;
+                    for (int s = 0; s < 4; ++s) {
+                        const double d = (double)dist[s];
+                        c[OCCGRID_C_HITS] += (OCC_MIN_DIST_M < d && d <= OCC_MAX_DIST_M) ? 1 : 0;     // :888
+                    }
+                    int tile = home_tile(g, tg, rx, ry);
+                    if (kMaps && tile >= 0) tile += (agent - 1) * tg.n_tiles;
+                    if (tile >= 0) {
+                        slot = (unsigned int)hash_insert(s_keys, (unsigned int)tile);
+                        atomicAdd(&s_vals[slot], 1u);
+                        PoseRec r;
+                        r.rx = rx; r.ry = ry; r.yaw = (float)ryaw;      // ryaw came from an fp32 field: exact
+                        r.d[0] = dist[0]; r.d[1] = dist[1]; r.d[2] = dist[2]; r.d[3] = dist[3];
+                        r.k = (unsigned int)k;
+                        r.tile = tile; r.pad = 0;
+                        recs[k] = r;                                    // packet order: coalesced 48-byte stores
+                    }
+                }
+                s_slot[sub * kTT + threadIdx.x] = (unsigned short)slot;
+            }
+            __syncthreads();                                                          // stage st is consumed
+            if (threadIdx.x == 0 && bulk_ok) issue(i + kBinStages);
+        }
+        // One global atomic per distinct tile, as in flush_tile_counts; its return value is this
+        // segment's rank inside the tile's bin.
+        unsigned int key[kHashPerThread], rank[kHashPerThread];
 #pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { const unsigned int u = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += u; }
-    if (lane == 31) s_wsum[warp] = inc;
-    __syncthreads();
-    unsigned int pos = inc - mine, n_local = 0u;
+        for (int j = 0; j < kHashPerThread; ++j) {
+            const int h = j * kTT + threadIdx.x;
+            key[j] = s_keys[h];
+            rank[j] = 0u;
+            if (key[j] != kEmpty) rank[j] = atomicAdd(&tile_count[key[j]], s_vals[h]);
+        }
+        // Exclusive scan of (count | 1 << 16) over the occupied slots in (thread, j) order: the low
+        // half is the slot's first local position, the high half its run index (both < kPkPerCta).
+        // An empty slot has count 0.
+        unsigned int mine = 0u;
 #pragma unroll
-    for (int w = 0; w < kTT / 32; ++w) {
-        pos += w < warp ? s_wsum[w] : 0u;
-        n_local += s_wsum[w];
+        for (int j = 0; j < kHashPerThread; ++j) mine += key[j] != kEmpty ? s_vals[j * kTT + threadIdx.x] + 0x10000u : 0u;
+        unsigned int inc = mine;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) { const unsigned int u = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += u; }
+        if (lane == 31) s_wsum[warp] = inc;
+        __syncthreads();
+        unsigned int pos = inc - mine, n_local = 0u;
+#pragma unroll
+        for (int w = 0; w < kTT / 32; ++w) {
+            pos += w < warp ? s_wsum[w] : 0u;
+            n_local += s_wsum[w];
+        }
+        n_local &= 0xffffu;
+        if (threadIdx.x == 0) seg_count[seg] = n_local;
+        // run descriptors; each slot (owned by this thread alone) now holds (run << 16) | its next
+        // free local position
+#pragma unroll
+        for (int j = 0; j < kHashPerThread; ++j) {
+            if (key[j] == kEmpty) continue;
+            const int h = j * kTT + threadIdx.x;
+            const unsigned int run = pos >> 16, begin = pos & 0xffffu;
+            runs[seg0 + run] = make_uint2(key[j], rank[j] - begin);
+            pos += s_vals[h] + 0x10000u;
+            s_vals[h] = (run << 16) | begin;
+            if (rank[j] == 0u) active[atomicAdd(&hdr->active_count, 1u)] = key[j];     // first toucher lists the tile
+        }
+        __syncthreads();
+        // the packet indices grouped by tile, assembled in the (now free) hash keys, then stored
+        // coalesced
+        unsigned int* const s_local = s_keys;
+        const int n_seg = (int)min((long long)kPkPerCta, n - (long long)seg0);
+        for (int j = threadIdx.x; j < n_seg; j += kTT) {
+            const unsigned int slot = s_slot[j];
+            if (slot != kNoSlot) {
+                const unsigned int at = atomicAdd(&s_vals[slot], 1u);
+                s_local[at & 0xffffu] = (at & 0xffff0000u) | (unsigned int)j;
+            }
+        }
+        __syncthreads();
+        for (unsigned int j = threadIdx.x; j < n_local; j += kTT) local_bins[seg0 + j] = s_local[j];
+        if (threadIdx.x == 0) seg_of(q + 1);
+        __syncthreads();
     }
-    n_local &= 0xffffu;
-    if (threadIdx.x == 0) seg_count[blockIdx.x] = n_local;
-    const size_t seg0 = (size_t)blockIdx.x * kPkPerCta;
-    // run descriptors; each slot (owned by this thread alone) now holds its run index and its next
-    // free local position
+    unsigned long long c64[OCCGRID_C_HITS + 1];
 #pragma unroll
-    for (int j = 0; j < kHashPerThread; ++j) {
-        if (key[j] == kEmpty) continue;
-        const int i = j * kTT + threadIdx.x;
-        const unsigned int run = pos >> 16, begin = pos & 0xffffu;
-        runs[seg0 + run] = make_uint2(key[j], rank[j] - begin);
-        pos += s_vals[i] + 0x10000u;
-        s_keys[i] = run;
-        s_vals[i] = begin;
-        if (rank[j] == 0u) active[atomicAdd(&hdr->active_count, 1u)] = key[j];     // first toucher lists the tile
-    }
-    __syncthreads();
-    // the packet indices grouped by tile, assembled in the (now free) staging buffer, then stored
-    // coalesced
-    unsigned int* const s_local = reinterpret_cast<unsigned int*>(s_rec);
-    const int n_seg = (int)min((long long)kPkPerCta, n - (long long)seg0);
-    for (int j = threadIdx.x; j < n_seg; j += kTT) {
-        const unsigned int slot = s_slot[j];
-        if (slot != kNoSlot) s_local[atomicAdd(&s_vals[slot], 1u)] = (s_keys[slot] << 16) | (unsigned int)j;
-    }
-    __syncthreads();
-    for (unsigned int j = threadIdx.x; j < n_local; j += kTT) local_bins[seg0 + j] = s_local[j];
-    __syncthreads();
-    block_add_counters(c, reinterpret_cast<unsigned long long*>(s_rec), counters);
+    for (int j = 0; j <= OCCGRID_C_HITS; ++j) c64[j] = c[j];
+    block_add_counters(c64, reinterpret_cast<unsigned long long*>(s_keys), counters);
 }
 
 // Thread per local_bins entry of one binning CTA's segment (see k_home_bin): no hash and no atomics,
@@ -501,7 +553,7 @@ k_tile_plan(unsigned int* __restrict__ tile_count, unsigned int* __restrict__ ti
         h.active_count = 0;                  // ready for the next call's count pass
         h.overflow = (s_carry[0] > max_records || s_carry[1] > max_items) ? 1u : 0u;
         if (h.overflow) { h.n_items = 0; h.n_active = 0; }
-        h.pad = 0;
+        h.bin_counter = 0;
         *hdr = h;
         if (counters) atomicAdd(reinterpret_cast<unsigned long long*>(counters) + OCCGRID_C_RECORDS, (unsigned long long)s_carry[0]);
     }
@@ -1297,10 +1349,15 @@ int integrate_tiled(const occgrid_geom* geom, const PacketBatch& batch, const Po
             k_home_count_poses<<<grid_chunks(n_chunks), kTT, 0, st>>>(g, tg, d_poses, nullptr, seg, n_chunks, 0, P.tile_count, P.tile_ids, P.active,
                                                                       P.hdr, d_counters);
         } else {
+            // persistent: one CTA per resident slot, never more than there are segments
             const auto bin = maps ? k_home_bin<true> : k_home_bin<false>;
-            OCC_CUDA_TRY(cudaFuncSetAttribute(bin, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBinSmem));
-            bin<<<blocks, kTT, kBinSmem, st>>>(g, tg, batch.pkts, n, batch.stride, batch.agent_idx, batch.drift, batch.agent_off, batch.n_agents,
-                                               P.tile_count, P.recs, P.local_bins, P.runs, P.seg_count, P.active, P.hdr, d_counters);
+            const size_t smem = bin_smem_bytes(batch.stride);
+            OCC_CUDA_TRY(cudaFuncSetAttribute(bin, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            int per_sm = 1;
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, bin, kTT, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
+            const unsigned int ctas = min(blocks, (unsigned int)(device_sm_count() * per_sm));
+            bin<<<ctas, kTT, smem, st>>>(g, tg, batch.pkts, n, batch.stride, batch.agent_idx, batch.drift, batch.agent_off, batch.n_agents,
+                                         P.tile_count, P.recs, P.local_bins, P.runs, P.seg_count, P.active, P.hdr, d_counters);
         }
     }
     {
