@@ -13,7 +13,7 @@ import subprocess
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, 'csrc')
 LIB_PATH = os.path.join(PKG_DIR, 'liboccgrid_b200.so')
-SOURCES = ['occgrid_integrate.cu', 'occgrid_tiled.cu', 'occgrid_route.cu', 'occgrid_band.cu', 'mapmerge.cu', 'frontier.cu', 'icp.cu', 'icp_batch.cu', 'render.cu', 'map_fuse.cu', 'frontier_assign.cu', 'distance_field.cu', 'slam_chain.cpp']
+SOURCES = ['occgrid_integrate.cu', 'occgrid_tiled.cu', 'occgrid_route.cu', 'occgrid_band.cu', 'mapmerge.cu', 'frontier.cu', 'icp.cu', 'icp_batch.cu', 'render.cu', 'map_fuse.cu', 'frontier_assign.cu', 'distance_field.cu', 'map_align.cu', 'slam_chain.cpp']
 HEADERS = ['common.cuh', 'beam_expand.cuh', 'block_ops.cuh', 'icp_core.cuh', 'sincos_dd.cuh', os.path.join('..', '..', 'include', 'occgrid_b200.h')]
 
 STRATEGY = {'auto': -1, 'global_atomic': 0, 'tiled': 1}
@@ -234,13 +234,20 @@ def _bind_merge(L):
     L.occgrid_distance_field.argtypes = [vp, i32, i32, vp, vp, sz, vp]
     L.occgrid_inflate.restype = C.c_int
     L.occgrid_inflate.argtypes = [vp, i32, i32, dbl, dbl, dbl, i64, vp, i32, vp, vp, sz, vp]
+    L.mapmerge_align_workspace_bytes.restype = sz
+    L.mapmerge_align_workspace_bytes.argtypes = [C.c_int, i32, i32, i32, i32, i32, i32, i32, i64]
+    L.mapmerge_align.restype = C.c_int
+    L.mapmerge_align.argtypes = [vp, C.c_int, i32, i32, dbl, vp, vp, vp, i32, i32, dbl, dbl, dbl, vp, i32, i32, i32,
+                                 vp, vp, vp, sz, vp]
+    L.mapmerge_align_set_block.restype = C.c_int
+    L.mapmerge_align_set_block.argtypes = [C.c_int]
 
 
 KERNEL_NAMES = ('integrate_global', 'resolve', 'update_rays', 'tile_count', 'tile_scan', 'tile_scatter',
                 'tile_raycast', 'tile_resolve', 'merge_extract', 'merge_bounds', 'merge_voxel', 'merge_raster',
                 'merge_fuse', 'probe', 'route', 'frontier', 'frontier_cluster', 'chain_probe', 'chain_incremental',
                 'chain_rebuild', 'icp', 'band_barrier', 'render', 'merge_scan', 'merge_warp_fuse', 'frontier_assign',
-                'icp_batch', 'distance_field')
+                'icp_batch', 'distance_field', 'map_align')
 
 
 def profile_begin():

@@ -46,6 +46,24 @@ def se2_matrix(tx, ty, theta):
     return T
 
 
+def align_transform(prior, origin, res, width, height, cs, sn, dx, dy, ref_res):
+    """The agent->global transform of alignment candidate (rotation (cs, sn), offset (dx, dy) reference
+    cells) for a width x height map at ``origin``: the prior rotated about the map's centre as the prior
+    places it, then shifted, in fp64 with every operation rounded as ``mapmerge_align`` states."""
+    p = np.asarray(prior, np.float64)
+    p00, p01, p03, p10, p11, p13 = (float(p[0, 0]), float(p[0, 1]), float(p[0, 3]), float(p[1, 0]), float(p[1, 1]),
+                                    float(p[1, 3]))
+    ox, oy, r, g, cs, sn = float(origin[0]), float(origin[1]), float(res), float(ref_res), float(cs), float(sn)
+    mx, my = ox + ((0.5 * width) * r), oy + ((0.5 * height) * r)
+    ex, ey = -((p00 * mx) + (p01 * my)), -((p10 * mx) + (p11 * my))
+    T = np.eye(4)
+    T[0, 0], T[0, 1] = (cs * p00) - (sn * p10), (cs * p01) - (sn * p11)
+    T[1, 0], T[1, 1] = (sn * p00) + (cs * p10), (sn * p01) + (cs * p11)
+    T[0, 3] = (p03 + (((cs - 1.0) * ex) - (sn * ey))) + dx * g
+    T[1, 3] = (p13 + ((sn * ex) + ((cs - 1.0) * ey))) + dy * g
+    return T
+
+
 class _Cloud:
     """fp64 x[], y[] + device-resident count."""
 
@@ -499,37 +517,7 @@ class MapMerger:
         straight into ``fuse_occupancy``), ``fitness``, ``inlier_rmse``, ``iterations``,
         ``correspondences`` and ``accepted`` (fitness >= 0.6, the gate at :54-56).  An agent with no
         occupied cells gets the identity refinement, fitness 0 and 0 iterations."""
-        if isinstance(grids, torch.Tensor):
-            if grids.is_cuda and grids.device != self.device:
-                raise OccGridError(f'register_maps: the grids are on {grids.device}, the merger on {self.device}')
-            if grids.dtype != torch.int8:
-                raise ValueError('register_maps: grids must be int8')
-        else:
-            grids = np.ascontiguousarray(np.asarray(grids), dtype=np.int8)
-        if grids.ndim != 3 or min(grids.shape) < 1:
-            raise ValueError(f'register_maps: grids must be [A, H, W] with A, H, W >= 1, got {tuple(grids.shape)}')
-        A = int(grids.shape[0])
-        org = np.asarray(origins, np.float64)
-        if org.size != 2 * A:
-            raise ValueError(f'register_maps: origins must be [{A}, 2], got {org.shape}')
-        org = np.ascontiguousarray(org.reshape(A, 2))
-        if priors is not None:
-            if len(priors) != A:
-                raise ValueError(f'register_maps: {len(priors)} priors for {A} grids')
-            for a in range(A):
-                if priors[a] is not None and np.asarray(priors[a]).size not in (3, 16):
-                    raise ValueError(f'register_maps: prior {a} must be 4x4 or (tx, ty, theta), got shape {np.asarray(priors[a]).shape}')
-        Tm = self._as_matrices(priors, A)
-        for a in range(A):                       # mapmerge_warp_fuse's rule, in the same fp64 arithmetic
-            T = Tm[a]
-            if not np.isfinite(T).all():
-                raise OccGridError(f'register_maps: prior {a} has a non-finite entry')
-            R = ((T[0, 0], T[0, 1]), (T[1, 0], T[1, 1]))
-            for p in range(2):
-                for q in range(2):
-                    rtr = float(R[0][p]) * float(R[0][q]) + float(R[1][p]) * float(R[1][q])
-                    if not abs(rtr - (1.0 if p == q else 0.0)) <= 1e-9:
-                        raise OccGridError(f'register_maps: prior {a} is not rigid (|R^T R - I| > 1e-9)')
+        grids, A, org, Tm = self._agent_inputs('register_maps', grids, origins, priors)
         if reference is not None:
             if reference.window != (0, 0, reference.size, reference.size):
                 raise OccGridError('register_maps: the reference must hold its whole grid (not a window of it)')
@@ -560,6 +548,121 @@ class MapMerger:
         return SimpleNamespace(refinement=U, transformation=transformation, fitness=fitness, inlier_rmse=r[:, 17].copy(),
                                iterations=r[:, 18].astype(np.int64), correspondences=r[:, 19].astype(np.int64),
                                accepted=accepted)
+
+    # ---- correlative map alignment (EXTENSION, no reference counterpart) -------------------------
+    def align_maps(self, grids, origins, res, priors, reference, max_offset=1.0, max_angle=math.radians(30),
+                   angle_step=math.radians(1), clearance=0.1):
+        """Find, for every agent map, the rotation and translation in a window around its prior that
+        best overlays the reference map's obstacles (``mapmerge_align`` in include/occgrid_b200.h): a
+        correlative search, exact, in one device call.  Use it when a prior is too far off for
+        ``register_maps``, then pass ``transformation`` to ``register_maps(priors=...)``.
+
+        grids       int8 [A, H, W] (``AgentGrids.grids_tensor`` is used without a copy); ``origins``
+                    float64 [A, 2]; ``res`` the agents' resolution; ``priors`` as ``register_maps``
+        reference   an ``OccupancyGrid`` holding its whole grid on this device; its distance field
+                    (``reference.distance_field``) weights the candidates
+        max_offset  translation half-width in metres: Rc = round(max_offset / reference.res) cells
+        max_angle, angle_step   rotations θ = m * angle_step about each map's centre for
+                    m = 0, 1, -1, 2, -2, ... ±K0, K0 = round(max_angle / angle_step)
+        clearance   a point scores max_d2 + 1 - d2 within max_d2 = floor((clearance / reference.res)²)
+                    cells² of a reference obstacle (the rule of ``navigation_grid``)
+        The host reads twice: the occupied counts, then the results.
+        Returns a namespace of NumPy arrays: ``transformation`` [A, 4, 4] (the winner's transform, or
+        the prior for an agent without occupied cells), ``score``, ``prior_score``, ``points``,
+        ``angle`` (the winner's θ), ``offset`` [A, 2] (dx, dy in reference cells), ``improved``
+        (score > prior_score), and ``candidates`` / ``scored`` (how many candidates were searched and
+        how many were scored exactly; these depend on the pruning block size)."""
+        grids, A, org, Tm = self._agent_inputs('align_maps', grids, origins, priors)
+        if reference.window != (0, 0, reference.size, reference.size):
+            raise OccGridError('align_maps: the reference must hold its whole grid (not a window of it)')
+        if reference.device != self.device:
+            raise OccGridError(f'align_maps: the reference is on {reference.device}, the merger on {self.device}')
+        for name, v in (('max_offset', max_offset), ('max_angle', max_angle), ('clearance', clearance)):
+            if not (math.isfinite(float(v)) and float(v) >= 0.0):
+                raise ValueError(f'align_maps: {name} must be finite and >= 0, got {v!r}')
+        if not (math.isfinite(float(angle_step)) and float(angle_step) > 0.0):
+            raise ValueError(f'align_maps: angle_step must be finite and > 0, got {angle_step!r}')
+        g = float(reference.res)
+        rc = round(float(max_offset) / g)
+        k0 = round(float(max_angle) / float(angle_step))
+        q = float(clearance) / g
+        max_d2 = math.floor(q * q)
+        if rc > 2048:
+            raise ValueError(f'align_maps: max_offset {max_offset} m is {rc} reference cells, more than 2048')
+        if 2 * k0 + 1 > 65535:
+            raise ValueError(f'align_maps: {2 * k0 + 1} rotations, more than 65 535')
+        if max_d2 > 254:
+            raise ValueError(f'align_maps: clearance {clearance} m gives max_d2 = {max_d2} cells², more than 254')
+        steps = [0] + [m for i in range(1, k0 + 1) for m in (i, -i)]
+        theta = np.array([m * float(angle_step) for m in steps])
+        rot = np.ascontiguousarray([[math.cos(t), math.sin(t)] for t in theta], np.float64)
+        h, w = int(grids.shape[1]), int(grids.shape[2])
+        lib = self._lib
+        with torch.cuda.device(self.device):
+            if isinstance(grids, np.ndarray):
+                grids = torch.from_numpy(grids).to(self.device)
+            elif not (grids.is_cuda and grids.is_contiguous()):
+                grids = grids.to(self.device).contiguous()
+            d2 = reference.distance_field(to_host=False)
+            counts, _, _ = self._count_occupied(list(grids.unbind(0)), True)
+            n_points = int(counts.sum().item())                                 # host read 1
+            nbytes = lib.mapmerge_align_workspace_bytes(A, w, h, reference.size, reference.size, max_d2, rc, len(steps), n_points)
+            if nbytes == 0:
+                raise OccGridError('mapmerge_align_workspace_bytes: ' + _native.last_error())
+            ws = self._workspace('align', nbytes)
+            out = torch.empty(6 * A + 2, dtype=torch.int64, device=self.device)
+            rc_call = lib.mapmerge_align(grids.data_ptr(), A, w, h, float(res), org.ctypes.data, Tm.ctypes.data, d2.data_ptr(),
+                                         reference.size, reference.size, reference.ox, reference.oy, g, rot.ctypes.data,
+                                         len(steps), rc, max_d2, out.data_ptr(), out[6 * A:].data_ptr(), ws.data_ptr(),
+                                         ws.numel(), self._stream())
+            _native.check(rc_call, 'mapmerge_align')
+            r = out.cpu().numpy()                                               # host read 2
+        rows, diag = r[:6 * A].reshape(A, 6), r[6 * A:]
+        if (rows[:, 0] < 0).any():
+            raise OccGridError('align_maps: the occupied cells did not fit the workspace')
+        transformation = Tm.copy()
+        for a in np.flatnonzero(rows[:, 5] > 0):
+            transformation[a] = align_transform(Tm[a], org[a], float(res), w, h, *rot[rows[a, 1]], int(rows[a, 2]),
+                                                int(rows[a, 3]), g)
+        return SimpleNamespace(transformation=transformation, score=rows[:, 0].copy(), prior_score=rows[:, 4].copy(),
+                               points=rows[:, 5].copy(), angle=theta[rows[:, 1]], offset=rows[:, 2:4].copy(),
+                               improved=rows[:, 0] > rows[:, 4], candidates=int(diag[0]), scored=int(diag[1]))
+
+    def _agent_inputs(self, who, grids, origins, priors):
+        """The checks register_maps and align_maps share: grids int8 [A, H, W] (a tensor must be on this
+        device), origins [A, 2] and rigid priors -> (grids, A, origins [A, 2], priors [A, 4, 4])."""
+        if isinstance(grids, torch.Tensor):
+            if grids.is_cuda and grids.device != self.device:
+                raise OccGridError(f'{who}: the grids are on {grids.device}, the merger on {self.device}')
+            if grids.dtype != torch.int8:
+                raise ValueError(f'{who}: grids must be int8')
+        else:
+            grids = np.ascontiguousarray(np.asarray(grids), dtype=np.int8)
+        if grids.ndim != 3 or min(grids.shape) < 1:
+            raise ValueError(f'{who}: grids must be [A, H, W] with A, H, W >= 1, got {tuple(grids.shape)}')
+        A = int(grids.shape[0])
+        org = np.asarray(origins, np.float64)
+        if org.size != 2 * A:
+            raise ValueError(f'{who}: origins must be [{A}, 2], got {org.shape}')
+        org = np.ascontiguousarray(org.reshape(A, 2))
+        if priors is not None:
+            if len(priors) != A:
+                raise ValueError(f'{who}: {len(priors)} priors for {A} grids')
+            for a in range(A):
+                if priors[a] is not None and np.asarray(priors[a]).size not in (3, 16):
+                    raise ValueError(f'{who}: prior {a} must be 4x4 or (tx, ty, theta), got shape {np.asarray(priors[a]).shape}')
+        Tm = self._as_matrices(priors, A)
+        for a in range(A):                       # mapmerge_warp_fuse's rule, in the same fp64 arithmetic
+            T = Tm[a]
+            if not np.isfinite(T).all():
+                raise OccGridError(f'{who}: prior {a} has a non-finite entry')
+            R = ((T[0, 0], T[0, 1]), (T[1, 0], T[1, 1]))
+            for p in range(2):
+                for q in range(2):
+                    rtr = float(R[0][p]) * float(R[0][q]) + float(R[1][p]) * float(R[1][q])
+                    if not abs(rtr - (1.0 if p == q else 0.0)) <= 1e-9:
+                        raise OccGridError(f'{who}: prior {a} is not rigid (|R^T R - I| > 1e-9)')
+        return grids, A, org, Tm
 
     def _registration_inputs(self, grids, org, res, Tm, reference, threshold):
         """The device inputs of mapmerge_icp_register_batch: every agent's occupied cells moved by its

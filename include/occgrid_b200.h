@@ -669,6 +669,87 @@ int occgrid_inflate(const int8_t* d_grid, int32_t width, int32_t height, double 
                     int64_t max_d2, const double* d_robot_xy /* [A][2] or NULL when A == 0 */, int32_t n_robots,
                     int8_t* d_out, void* d_ws, size_t ws_bytes, void* stream);
 
+/* EXTENSION (no reference counterpart): correlative map alignment (DESIGN §6h).  For every agent map,
+ * the rotation x translation in a window around its prior that best overlays the reference's
+ * obstacles, exactly the winner of the exhaustive search, in one stream-ordered call.  Its transform
+ * is the prior for mapmerge_icp_register_batch when the prior is too far off for ICP.
+ * Inputs:
+ *   d_grids int8 [A][H][W] on the device (W = width, H = height); origins_host [A][2] = (ox_a, oy_a)
+ *     and one resolution r = res for all.
+ *   priors_host [A][16]: agent->global, 4x4 row-major.  Rejected unless every entry is finite and
+ *     |R^T R - I| <= 1e-9, the rule of mapmerge_warp_fuse.
+ *   The reference as its squared distance field d_d2 int32 [Hr][Wr] on the device (Wr = ref_w, Hr =
+ *     ref_h), exactly what occgrid_distance_field writes (-1 everywhere when the grid has no
+ *     obstacle), its origin (gox, goy) = (ref_ox, ref_oy) and resolution g = ref_res (g need not
+ *     equal r).
+ *   rot_host [n_angles][2]: the rotation table (cs_k, sn_k), each |cs^2 + sn^2 - 1| <= 1e-9.  The
+ *     caller orders it by preference, entry 0 normally the identity (1, 0).
+ *   max_offset = Rc, the translation half-width in reference cells, and max_d2.
+ * Occupied cells: agent a's cells > 50 (the rule of grid_to_pcd, the extraction and ICP).  Cell (u, v)
+ * is column u, row v.
+ * Coefficients per (agent, rotation), host fp64, each operation rounded on its own as bracketed (the
+ * library is built with -ffp-contract=off); p = the prior:
+ *   mx = ox_a + ((0.5*W)*r)          my = oy_a + ((0.5*H)*r)            (map centre, agent frame)
+ *   ex = -((p00*mx) + (p01*my))      ey = -((p10*mx) + (p11*my))        (t_p - c, where c is the centre placed by the prior)
+ *   m00 = (cs*p00) - (sn*p10)        m01 = (cs*p01) - (sn*p11)
+ *   m10 = (sn*p00) + (cs*p10)        m11 = (sn*p01) + (cs*p11)
+ *   tx = p03 + (((cs - 1)*ex) - (sn*ey))      ty = p13 + ((sn*ex) + ((cs - 1)*ey))
+ *   bx = ox_a + 0.5*r                by = oy_a + 0.5*r                  (centre of agent cell (0, 0))
+ *   e0 = (m00*r)/g   e1 = (m01*r)/g   e2 = ((((m00*bx) + (m01*by)) + tx) - gox)/g
+ *   e3 = (m10*r)/g   e4 = (m11*r)/g   e5 = ((((m10*bx) + (m11*by)) + ty) - goy)/g
+ * Together these rotate the map about its own centre, as placed by the prior.  With (cs, sn) = (1, 0),
+ * m and t are the prior's own entries, bit for bit up to the sign of a zero.
+ * Per occupied cell, on the device (fp64, no contraction, __dmul_rn / __dadd_rn as in §4):
+ *   X = (e0*u) + ((e1*v) + e2)       Y = (e3*u) + ((e4*v) + e5)         j = floor(X), i = floor(Y)
+ *   A point with |X| or |Y| >= 2^30, or NaN, contributes 0 to every candidate.
+ * Candidates: (k, dx, dy) with -Rc <= dx, dy <= Rc moves every point of rotation k to cell
+ *   (j + dx, i + dy).  A point contributes w = max_d2 + 1 - d2[i+dy][j+dx] when that cell lies inside
+ *   the reference and 0 <= d2 <= max_d2, and 0 otherwise.  score = the integer sum of these; with
+ *   max_d2 = 0 it is the number of points that land on reference obstacles.
+ * Winner: the largest score, ties to the lowest rank, where
+ *   o(v) = 2v - 1 if v > 0, else -2v          rank = (k*(2Rc+1) + o(dy))*(2Rc+1) + o(dx)
+ *   so candidate (0, 0, 0), the prior, wins every tie and an agent that matches nothing keeps its
+ *   prior.  The key (uint64)score << 32 | (2^32 - 1 - rank) makes this a plain 64-bit integer max,
+ *   independent of order.
+ * Output d_out int64 [A][6]: score, k, dx, dy, prior_score (the score of (0, 0, 0)), n_points.  An agent
+ *   with no occupied cells gets all zeros.  If the occupied cells do not fit the workspace, every row
+ *   is -2, 0, 0, 0, 0, 0 (as mapmerge_icp_register_batch).  d_diag int64 [2] (may be NULL): the
+ *   candidates searched (A' * n_angles * (2Rc+1)^2 over the A' agents with points) and the
+ *   candidates scored exactly; these depend on the block size and are not part of the contract.
+ * Transform of candidate (k, dx, dy): [[m00, m01, 0, tx + dx*g], [m10, m11, 0, ty + dy*g], [0, 0, 1, 0],
+ *   [0, 0, 0, 1]], computed in host fp64.
+ * Limits: OCCGRID_E_ARG (message key word in quotes) for a "NULL pointer" (d_diag may be NULL),
+ * "n_agents" outside 1..65 535, "width x height" with a side < 1 or W*H*(max_d2+1) > 2^31 - 1 (so a
+ * score fits 31 bits), a "reference size" side outside 1..32 768 (the range of
+ * occgrid_distance_field), "max_d2" outside 0..254, "max_offset" (Rc) outside 0..2048, "n_angles"
+ * outside 1..65 535, more than 2^32 - 1 "candidates" (n_angles*(2Rc+1)^2), a "resolution" that is not
+ * finite and > 0, a "prior" that is not finite or not rigid and a "rotation" that is not a unit
+ * (cs, sn) pair.  OCCGRID_E_WORKSPACE for ws_bytes below the workspace of zero points.
+ * Workspace: mapmerge_align_workspace_bytes(n_agents, W, H, Wr, Hr, max_d2, Rc, n_angles,
+ * total_points) returns 0 for any of the size errors above and for total_points outside
+ * 0..A*W*H; otherwise, with a(v) = v rounded up to a multiple of 256, s the block size in effect
+ * (mapmerge_align_set_block), cpa = ceil(W*H / 4096), nb = ceil((2Rc+1) / s)^2, pad = 2Rc + 64 and
+ * np = (Wr + 2 pad)(Hr + 2 pad), it is exactly
+ *   a(48 A n_angles) + a(4 A cpa) + a(8 (A + 1)) + a(4 A n_angles nb) + 3 a(8 A) + a(65 536) + 256
+ *   + a(np) + a(np) + a(np) + a(8 total_points)
+ * (coefficients, compaction counts, agent offsets, block bounds, best keys / prior scores / picked
+ * blocks, per-CTA counts, status, the weight table Lw, its s x s maximum Ls and the row maxima, the
+ * (u, v) points).  Every size is below 2^51, so nothing overflows.  The call holds as many points as
+ * ws_bytes allows.
+ * Stream-ordered: no host synchronisation and no atomics except the 64-bit key max; the per-(agent,
+ * rotation) coefficients reach the device by cudaMemcpyAsync into the workspace. */
+size_t mapmerge_align_workspace_bytes(int n_agents, int32_t width, int32_t height, int32_t ref_w, int32_t ref_h,
+                                      int32_t max_d2, int32_t max_offset, int32_t n_angles, int64_t total_points);
+int mapmerge_align(const int8_t* d_grids, int n_agents, int32_t width, int32_t height, double res,
+                   const double* origins_host /* [A][2] */, const double* priors_host /* [A][16] */,
+                   const int32_t* d_d2, int32_t ref_w, int32_t ref_h, double ref_ox, double ref_oy, double ref_res,
+                   const double* rot_host /* [n_angles][2] */, int32_t n_angles, int32_t max_offset, int32_t max_d2,
+                   int64_t* d_out /* [A][6] */, int64_t* d_diag /* [2] or NULL */, void* d_ws, size_t ws_bytes,
+                   void* stream);
+/* Testing knob: the pruning block size s (0 = the default, 8; 1..64 allowed).  Results do not depend
+ * on it; the workspace does (nb above).  Process-wide; OCCGRID_E_ARG ("block") outside 0..64. */
+int mapmerge_align_set_block(int s);
+
 /* Tuning knob of the TILED strategy: cap the persistent raycast CTAs per SM (0 = as many as fit,
  * the default).  A pipelined multi-GPU ingest lowers it to 2 so that the routing kernel of the
  * next batch finds room on every SM and runs concurrently.  Process-wide. */
